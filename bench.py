@@ -2,7 +2,7 @@
 """Benchmark of the hot path: images/s for ViT-B/32 LoRA encode_image over the MTA crop batch
 (N=64 crops + 1 centre view per image) -> MTA x3 -> LP++ head -> top-5, image-sharded over N GPUs.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -65,7 +65,15 @@ def parse():
                          "the north star's 1e-2 logit tolerance end to end, bf16 is its literal wording (0.02-0.07 off)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the top-5 class ids the last timed step returned for the whole global "
+                         "batch (--impl reference: its one image) as DIR/topk.npy (float64 [images, 5]); the inputs are seeded, "
+                         "so runs with the same arguments can be compared output for output (N > 1: needs --no-balance, the "
+                         "balanced split depends on timings)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def workload_config(args, world, views_mib=None):
@@ -178,9 +186,12 @@ def run_reference(args):
         cpu_oracle_image(torch, sd_t, lora, texts, lp_t, imgs)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        cpu_oracle_image(torch, sd_t, lora, texts, lp_t, imgs)
+        top5 = cpu_oracle_image(torch, sd_t, lora, texts, lp_t, imgs)
     dt = time.perf_counter() - t0
     val = args.steps / dt
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "topk.npy"), top5.reshape(1, -1).numpy().astype(np.float64))
     sample = f"{args.steps} steps x 1 image x {V} views (224x224 fp32), full pipeline, oracle port on host cores"
     line = {
         "impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -218,6 +229,9 @@ def main():
         print(f"[bench rank {rank} +{time.perf_counter() - t_start:6.1f}s] {name}", file=sys.stderr, flush=True)
     if world != args.gpus and rank == 0:
         print(f"warning: --gpus {args.gpus} but WORLD_SIZE={world}; using WORLD_SIZE", file=sys.stderr)
+    if args.dump_outputs and world > 1 and not args.no_balance:
+        raise SystemExit("--dump-outputs on more than one GPU needs --no-balance: the balanced shards, and with them the "
+                         "images of a step, depend on measured speeds")
     peaks = measured_peaks()
     V = args.crops + 1
     I = args.images_per_gpu
@@ -294,9 +308,11 @@ def main():
     gather_all = jb.dist.AsyncTopkGather(world * K * I_max, 5, dev, sizes=[K * I_max] * world, depth=1) if G != 1 else None
     kept = torch.zeros((K, I_max, 5), dtype=torch.int32, device=dev)
     step_no = [0]
+    last_topk = [None]                       # this rank's predictions of the latest step (--dump-outputs)
 
     def step_device():
         topk = hp.evaluate_base(images, topk_to_host=False)
+        last_topk[0] = topk
         if G == 1:
             return gather.submit(topk)
         kept[step_no[0] % K, :topk.shape[0]].copy_(topk, non_blocking=True)
@@ -384,6 +400,13 @@ def main():
     torch.cuda.synchronize()
     jb.dist.barrier()
     prof = ctx.profile_stop()
+    if args.dump_outputs:
+        # the global batch's predictions of the last timed step, shards in rank order (40 bytes per image: far below
+        # 64 MB for any batch whose views fit in device memory)
+        topk_last = jb.dist.all_gather_topk(last_topk[0], n_total, sizes)
+        if rank == 0:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "topk.npy"), topk_last.cpu().numpy().astype(np.float64))
     if R and all_kept is not None:
         # the gathered block of rank r, step k holds that step's shard of rank r in rows [0, split[k][r]): every step's
         # predictions cover the whole global batch exactly once

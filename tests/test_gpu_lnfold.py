@@ -55,7 +55,7 @@ for trained_like in (False, "offset", "outliers", "both"):
 
 
 @pytest.mark.parametrize("mode", ["0", "1", "2"])
-def test_layernorm_schedules(mode):
+def test_layernorm_schedules(mode, cuda_dev):
     env = dict(os.environ, JCB_LN_FOLD=mode)
     r = subprocess.run([sys.executable, "-c", SNIPPET], env=env, capture_output=True, text=True, timeout=900)
     print(r.stdout[-3000:])

@@ -244,7 +244,7 @@ def test_cls_only_last_block_matches_full_schedule(jb, cuda_dev, vpt):
 def _shipped_lora_pickle(tmp_path):
     """The reference's trained adapters (lora_weights1/lora_weights.pkl) rebuilt in the reference's pickle layout
     (save_lora, test.py:642-684) from the numeric fixture tests/golden/lora_weights1_arrays.npz
-    (oracle/make_golden_lora.py)."""
+    (oracle/make_golden_lora.py; stored as float16, widened back to the checkpoint's float32 here)."""
     import json
     import os
     import pickle
@@ -255,7 +255,7 @@ def _shipped_lora_pickle(tmp_path):
         if key == "metadata_json":
             continue
         layer, proj, name = key.split("/")
-        weights.setdefault(layer, {}).setdefault(proj, {})[name] = z[key]
+        weights.setdefault(layer, {}).setdefault(proj, {})[name] = z[key].astype(np.float32)
     path = tmp_path / "lora_weights.pkl"
     with open(path, "wb") as f:
         pickle.dump({"weights": weights, "metadata": meta}, f)
