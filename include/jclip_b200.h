@@ -284,10 +284,22 @@ void jcb_mta_default_params(jcb_mta_params* p);
  *   text_dev     [dim, n_classes] float32  (the orientation the reference passes: `text_features.t()`)
  *   out_mode_dev [n_images, dim]            the mode, unit norm            (test.py:1461)
  *   out_logits_dev [n_images, n_classes] or NULL: 100 * mode @ text         (ood.py:819)
- *   params NULL = reference constants */
+ *   params NULL = reference constants
+ * JCB_E_INVALID, before anything is allocated or launched, for n_views outside [1, 2048], n_classes < 1, dim not a
+ * multiple of 32 in [32, 1024], a non-finite parameter, lambda_y <= 0, temperature <= 0, th < 0, max_iter < 1 or
+ * k_frac outside [0, 1] (the reference averages at most n_views - 1 neighbours).  n_views = 1 is accepted and gives
+ * what the reference gives: its bandwidth is the mean of no distances, so the mode is all NaN. */
 int jcb_mta(jcb_ctx* ctx, const float* feats_dev, const float* text_dev, int64_t n_images, int32_t n_views,
             int32_t n_classes, int32_t dim, const jcb_mta_params* params, float* out_mode_dev,
             float* out_logits_dev);
+/* jcb_mta plus the solver's state per image, for tests and debugging; each output may be NULL (skipped):
+ *   out_bw_dev       [n_images, n_views]           the bandwidths                                (test.py:1403-1408)
+ *   out_y_dev        [n_images, n_views]           the inlierness weights the last mode loop used (test.py:1434)
+ *   out_affinity_dev [n_images, n_views, n_views]  A = P P^T, P = softmax(100 X T / temperature)  (test.py:1411)
+ * The mode and logits are the ones jcb_mta returns for the same arguments. */
+int jcb_mta_debug(jcb_ctx* ctx, const float* feats_dev, const float* text_dev, int64_t n_images, int32_t n_views,
+                  int32_t n_classes, int32_t dim, const jcb_mta_params* params, float* out_mode_dev,
+                  float* out_logits_dev, float* out_bw_dev, float* out_y_dev, float* out_affinity_dev);
 
 /* ---------------------------------------------------------------- head ----------------------- */
 typedef struct jcb_head_weights {   /* Channel_LP parameters, test.py:1223-1228, all device fp32 */

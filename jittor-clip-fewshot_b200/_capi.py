@@ -136,6 +136,8 @@ PROTOTYPES = {
     "jcb_mta_default_params": (None, [POINTER(MtaParams)]),
     "jcb_mta": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32, POINTER(MtaParams),
                         c_void_p, c_void_p]),
+    "jcb_mta_debug": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32, POINTER(MtaParams),
+                              c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "jcb_head": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                          POINTER(HeadWeights), c_int64, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p,
                          c_void_p]),

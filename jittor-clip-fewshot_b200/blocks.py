@@ -85,6 +85,25 @@ def attention(qkv, n_views, tokens, heads, out, causal=False, sync=True):
         ctx.sync()
 
 
+def mta_debug(feats, text, params=None):
+    """jcb_mta_debug on feats [I, V, D] fp32 and text [D, C] fp32 (CUDA): the modes [I, D] and logits [I, C] of jcb_mta
+    with the solver's state -- bandwidths [I, V], final inlierness weights y [I, V], affinity [I, V, V].  `params`: dict
+    of jcb_mta_params fields to override (others keep the reference's constants)."""
+    ctx = _ctx(feats)
+    I, V, D = feats.shape
+    C = text.shape[1]
+    p = _capi.MtaParams()
+    ctx.lib.jcb_mta_default_params(byref(p))
+    for k, v in (params or {}).items():
+        setattr(p, k, v)
+    new = lambda *shape: torch.empty(shape, dtype=torch.float32, device=feats.device)
+    out = {"mode": new(I, D), "logits": new(I, C), "bw": new(I, V), "y": new(I, V), "affinity": new(I, V, V)}
+    check(ctx.lib.jcb_mta_debug(ctx.handle, ptr(feats), ptr(text), I, V, C, D, byref(p),
+                                *(ptr(out[k]) for k in ("mode", "logits", "bw", "y", "affinity"))), ctx.handle)
+    ctx.sync()
+    return out
+
+
 def im2col(images, resolution, patch, apply_clip_norm, out):
     from .runtime import img_dtype_code
     ctx = _ctx(images)

@@ -1,6 +1,7 @@
 // C-ABI of libjclip_b200.so (include/jclip_b200.h): contexts, weight packing, the image-tower schedule
 // and the MTA / head entry points.  Everything here is host orchestration; the arithmetic lives in
 // gemm.cu, attention.cu, rowwise.cu, mta.cu and head.cu.
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -1423,25 +1424,63 @@ MtaParams to_params(const jcb_mta_params* p) {
   }
   return m;
 }
+
+// Arguments of jcb_mta / jcb_mta_debug, checked before the workspace is sized from them.  Parameters are rejected where
+// the solver would stop meaning what the reference computes: temperature and lambda_y divide (test.py:1411, :1434); the
+// reference's loops run at least once (`while True`), the kernels' would run max_iter < 1 times and return view 0; the
+// reference averages sorted_dist[:, 1:k+1], at most V - 1 neighbours, where the kernels divide by k -- k_frac <= 1 keeps
+// k = int(k_frac (V - 1)) <= V - 1.
+int check_mta_args(jcb_ctx* ctx, const char* fn, const float* feats, const float* text, const float* out_mode,
+                   int64_t n_images, int32_t V, int32_t C, int32_t D, const jcb_mta_params* p) {
+  if (n_images < 0 || !feats || !text || !out_mode) return fail(ctx, JCB_E_INVALID, "%s: bad arguments", fn);
+  if (!mta_shape_supported(V, C, D))
+    return fail(ctx, JCB_E_INVALID, "%s: unsupported n_views=%d n_classes=%d dim=%d (need 1 <= n_views <= 2048, n_classes >= 1, "
+                "dim a multiple of 32 in [32, 1024])", fn, V, C, D);
+  if (!p) return JCB_OK;
+  if (!std::isfinite(p->lambda_y) || !std::isfinite(p->lambda_q) || !std::isfinite(p->th) || !std::isfinite(p->temperature) ||
+      !std::isfinite(p->k_frac))
+    return fail(ctx, JCB_E_INVALID, "%s: non-finite parameter", fn);
+  if (p->lambda_y <= 0.f) return fail(ctx, JCB_E_INVALID, "%s: lambda_y=%g must be > 0", fn, p->lambda_y);
+  if (p->temperature <= 0.f) return fail(ctx, JCB_E_INVALID, "%s: temperature=%g must be > 0", fn, p->temperature);
+  if (p->th < 0.f) return fail(ctx, JCB_E_INVALID, "%s: th=%g must be >= 0", fn, p->th);
+  if (p->max_iter < 1) return fail(ctx, JCB_E_INVALID, "%s: max_iter=%d must be >= 1", fn, p->max_iter);
+  if (!(p->k_frac >= 0.0 && p->k_frac <= 1.0)) return fail(ctx, JCB_E_INVALID, "%s: k_frac=%g must be in [0, 1]", fn, p->k_frac);
+  return JCB_OK;
+}
 }  // namespace
 
 // fp32 work of one solve_mta: P = softmax(100 X T) (2 V C D), the two V x V Gram matrices over the upper triangle
 // (V^2 (C + D)) and <= 50 density / mode passes over X (4 V D each): the figure the MTA profile class reports
 static double mta_flops(double I, double V, double C, double D) { return I * (2 * V * C * D + V * V * (C + D) + 50 * 4 * V * D); }
 
-int jcb_mta(jcb_ctx* ctx, const float* feats_dev, const float* text_dev, int64_t n_images, int32_t n_views,
-            int32_t n_classes, int32_t dim, const jcb_mta_params* params, float* out_mode_dev, float* out_logits_dev) {
+static int mta_run(jcb_ctx* ctx, const char* fn, const float* feats_dev, const float* text_dev, int64_t n_images,
+                   int32_t n_views, int32_t n_classes, int32_t dim, const jcb_mta_params* params, float* out_mode_dev,
+                   float* out_logits_dev, const MtaDebug* debug) {
   if (!ctx) return JCB_E_INVALID;
-  if (n_images < 0 || !feats_dev || !text_dev || !out_mode_dev) return fail(ctx, JCB_E_INVALID, "jcb_mta: bad arguments");
+  int rc = check_mta_args(ctx, fn, feats_dev, text_dev, out_mode_dev, n_images, n_views, n_classes, dim, params);
+  if (rc) return rc;
   DeviceGuard g(ctx->device);
   const size_t scratch = mta_scratch_bytes(n_images, n_views, n_classes, dim);
-  int rc = ws_reserve(ctx, scratch);
-  if (rc) return rc;
+  if ((rc = ws_reserve(ctx, scratch))) return rc;
   MtaSet set{feats_dev, text_dev, out_mode_dev, out_logits_dev};
   LAUNCH_P(ctx, JCB_KC_MTA, mta_flops(n_images, n_views, n_classes, dim), static_cast<double>(n_images) * (n_views + 1) * dim * 4,
            launch_mta(&set, 1, n_images, n_views, n_classes, dim, to_params(params),
-                      scratch ? static_cast<float*>(ctx->ws) : nullptr, ctx->stream, ctx->dev_status, ctx->num_sms));
+                      scratch ? static_cast<float*>(ctx->ws) : nullptr, ctx->stream, ctx->dev_status, ctx->num_sms, debug));
   return JCB_OK;
+}
+
+int jcb_mta(jcb_ctx* ctx, const float* feats_dev, const float* text_dev, int64_t n_images, int32_t n_views,
+            int32_t n_classes, int32_t dim, const jcb_mta_params* params, float* out_mode_dev, float* out_logits_dev) {
+  return mta_run(ctx, "jcb_mta", feats_dev, text_dev, n_images, n_views, n_classes, dim, params, out_mode_dev, out_logits_dev,
+                 nullptr);
+}
+
+int jcb_mta_debug(jcb_ctx* ctx, const float* feats_dev, const float* text_dev, int64_t n_images, int32_t n_views,
+                  int32_t n_classes, int32_t dim, const jcb_mta_params* params, float* out_mode_dev, float* out_logits_dev,
+                  float* out_bw_dev, float* out_y_dev, float* out_affinity_dev) {
+  const MtaDebug debug{out_bw_dev, out_y_dev, out_affinity_dev};
+  return mta_run(ctx, "jcb_mta_debug", feats_dev, text_dev, n_images, n_views, n_classes, dim, params, out_mode_dev,
+                 out_logits_dev, &debug);
 }
 
 int jcb_head(jcb_ctx* ctx, const float* m_pt, const float* m_hand, const float* m_zs, const float* T_pt,

@@ -137,13 +137,22 @@ struct MtaSet {
   float* out_mode;      // [I, D]
   float* out_logits;    // [I, C] = 100 * mode @ text, or nullptr
 };
+// solver state of set 0 written at the end of the solve (jcb_mta_debug); each pointer may be nullptr
+struct MtaDebug {
+  float* bw;         // [I, V] bandwidths
+  float* y;          // [I, V] inlierness weights of the last mode loop
+  float* affinity;   // [I, V, V] softmax(100 X T / temperature) softmax(...)^T
+};
+// the (V, C, D) launch_mta accepts
+bool mta_shape_supported(int V, int C, int D);
 // bytes of global scratch launch_mta needs (0 when a problem fits in shared memory)
 size_t mta_scratch_bytes(int64_t n_problems, int V, int C, int D);
 // n_sets independent (feats, text) problems per image in one launch: grid = (I, n_sets)
 // dev_status + num_sms given: softmax(100 X T) runs as a bf16 x 3-limb GEMM on the tensor cores (launch_gemm) for
 // C <= 512; otherwise (or JCB_MTA_PROBS=simt) the fp32 SIMT kernel
 cudaError_t launch_mta(const MtaSet* sets, int n_sets, int64_t I, int V, int C, int D, const MtaParams& p,
-                       float* scratch, cudaStream_t stream, int* dev_status = nullptr, int num_sms = 0);
+                       float* scratch, cudaStream_t stream, int* dev_status = nullptr, int num_sms = 0,
+                       const MtaDebug* debug = nullptr);
 
 enum HeadScore : int { SCORE_LOGITS = 0, SCORE_CS = 1, SCORE_CS1 = 2, SCORE_CS2 = 3, SCORE_CS3 = 4, SCORE_CS4 = 5, SCORE_CS5 = 6, SCORE_COUNT = 7 };
 // Opt a kernel in to `bytes` of dynamic shared memory on the CURRENT device.  cudaFuncSetAttribute acts on the current

@@ -46,6 +46,7 @@ struct MtaDev {
   int n_groups, max_group;   // max_group = the largest group_count: affinity slots in shared memory
   int group_count[MTA_MAX_SETS];
   int group_sets[MTA_MAX_SETS][MTA_MAX_SETS];
+  MtaDebug dbg;              // set 0's bandwidths, final y and affinity (jcb_mta_debug); all nullptr otherwise
 };
 
 template <int NW>
@@ -88,6 +89,19 @@ __device__ __forceinline__ void density_step(const float* __restrict__ X, const 
     }
   }
   __syncthreads();
+}
+// the solver state of image `img` for jcb_mta_debug, written by threads t0, t0 + nt, ...
+__device__ __forceinline__ void mta_write_debug(const MtaDebug& g, long long img, int V, const float* s_bw, const float* s_y,
+                                                const float* A, int ldA, int t0, int nt) {
+  if (g.bw)
+    for (int i = t0; i < V; i += nt) g.bw[img * V + i] = s_bw[i];
+  if (g.y)
+    for (int i = t0; i < V; i += nt) g.y[img * V + i] = s_y[i];
+  if (g.affinity)
+    for (int idx = t0; idx < V * V; idx += nt) {
+      const int i = idx / V, j = idx - i * V;
+      g.affinity[img * V * V + idx] = A[static_cast<long long>(i) * ldA + j];
+    }
 }
 
 
@@ -212,8 +226,11 @@ __global__ void __launch_bounds__(256, 1) mta_probs_kernel(const ProbsDev a) {
 // text bank that must keep fp32 accuracy (bf16 logits move the modes by 1e-3).  Every fp32 value is split into three
 // bf16 limbs, x = x1 + x2 + x3 (24 significand bits, fp32's exponent range -- no underflow of the small limbs, which is
 // what rules fp16 limbs out), and the six limb products of weight >= 2^-16,
-//     x.t ~= x1 t1 + x1 t2 + x1 t3 + x2 t1 + x2 t2 + x3 t1        (dropped: <= 2^-24 relative),
-// are ONE bf16 GEMM with the limbs concatenated along K:  A' = [X1 X1 X1 X2 X2 X3],  B' = [T1 T2 T3 T1 T2 T1],
+//     x.t ~= x3 t1 + x2 t2 + x1 t3 + x2 t1 + x1 t2 + x1 t1        (dropped: <= 2^-24 relative),
+// are ONE bf16 GEMM with the limbs concatenated along K:  A' = [X3 X2 X1 X2 X1 X1],  B' = [T1 T2 T3 T1 T2 T1].  The
+// smallest products come first: every MMA step adds to the accumulator at the accumulator's precision, and adding the
+// small limbs onto the finished x1 t1 sum (the order [X1 X1 X1 X2 X2 X3]) rounded six times as many steps at full
+// magnitude -- affinities ~2e-5 from the float64 reference, against ~5e-6 on the fp32 SIMT path (B200, 1000 W);
 // K' = 6 D = 3072 -- the tower's own tcgen05 kernel (gemm.cu, fp32 accumulation in TMEM, fp32 output), 26 GFLOP per bank
 // instead of 8.6 GFLOP of fp32 SIMT FMAs at a third of the SIMT peak.  A row softmax kernel finishes.
 __device__ __forceinline__ void split3(float x, uint16_t (&l)[3]) {
@@ -224,7 +241,7 @@ __device__ __forceinline__ void split3(float x, uint16_t (&l)[3]) {
   const __nv_bfloat16 c = __float2bfloat16_rn(r2);
   l[0] = __bfloat16_as_ushort(a); l[1] = __bfloat16_as_ushort(b); l[2] = __bfloat16_as_ushort(c);
 }
-// X [rows, D] fp32 -> A' [rows, 6 D] bf16, blocks (1, 1, 1, 2, 2, 3)
+// X [rows, D] fp32 -> A' [rows, 6 D] bf16, blocks (3, 2, 1, 2, 1, 1)
 __global__ void __launch_bounds__(256) mta_split_x_kernel(const float* __restrict__ X, long long rows, int D,
                                                           uint16_t* __restrict__ out) {
   griddep_wait();               // programmatic dependent launch (ptx.cuh): nothing global is touched above
@@ -236,7 +253,7 @@ __global__ void __launch_bounds__(256) mta_split_x_kernel(const float* __restric
   uint16_t l[3];
   split3(X[i], l);
   uint16_t* o = out + r * 6 * D + d;
-  o[0] = l[0]; o[D] = l[0]; o[2 * D] = l[0]; o[3 * D] = l[1]; o[4 * D] = l[1]; o[5 * D] = l[2];
+  o[0] = l[2]; o[D] = l[1]; o[2 * D] = l[0]; o[3 * D] = l[1]; o[4 * D] = l[0]; o[5 * D] = l[0];
 }
 // T^T [D, C] fp32 (the orientation solve_mta receives) -> B' [CP, 6 D] bf16, blocks (1, 2, 3, 1, 2, 1); rows >= C zero
 __global__ void __launch_bounds__(256) mta_split_t_kernel(const float* __restrict__ Tt, int C, int CP, int D,
@@ -665,6 +682,7 @@ __global__ void __launch_bounds__(NT, 1) mta_kernel(const MtaDev a) {
       set.out_logits[img * C + c] = s * 100.0f;
     }
   }
+  if (blockIdx.y == 0) mta_write_debug(a.dbg, img, V, s_bw, s_y, A, ldA, tid, NT);
 }
 
 constexpr size_t MTA_SMEM_LIMIT = 220 * 1024;
@@ -808,8 +826,9 @@ __device__ __forceinline__ void mf_density(const float* __restrict__ X, int ldx,
   else mf_density_q<WITH_Y, 0>(X, ldx, s_mode, s_bw, s_y, s_out, V, D, gw, GW);
 }
 
-__device__ __forceinline__ void mf_solve_bank(const MtaDev& a, const MtaSet& set, long long img, const float* __restrict__ X,
+__device__ __forceinline__ void mf_solve_bank(const MtaDev& a, int si, long long img, const float* __restrict__ X,
                               const float* __restrict__ A, const float* s_bw, float* st, int gw, int GW, int bar_id) {
+  const MtaSet& set = a.sets[si];
   const int V = a.V, C = a.C, D = a.D, ldA = a.ldA, ldx = a.ldx;
   const int lane = threadIdx.x & 31, gt = gw * 32 + lane, GT = GW * 32;
   const int vp = (V + 3) & ~3, iq_n = mf_iq(V), nds = D >> 7;
@@ -945,6 +964,7 @@ __device__ __forceinline__ void mf_solve_bank(const MtaDev& a, const MtaSet& set
       set.out_logits[img * C + c] = s2 * 100.0f;
     }
   }
+  if (si == 0) mta_write_debug(a.dbg, img, V, s_bw, s_y, A, ldA, gt, GT);
 }
 
 // NT = 512 threads and one CTA per SM for the headline view counts (V = 65: 215 KB of shared memory with three banks);
@@ -1040,7 +1060,7 @@ __global__ void __launch_bounds__(NT, NT == 512 ? 1 : (NT == 128 ? 4 : (NT == 64
     st = U + b0 * mf_state_floats(V, D);
   }
   for (int b = b0; b < b1; ++b)
-    mf_solve_bank(a, a.sets[a.group_sets[group][b]], img, X, A_all + b * a_elems, s_bw, st, gw, GW, bar);
+    mf_solve_bank(a, a.group_sets[group][b], img, X, A_all + b * a_elems, s_bw, st, gw, GW, bar);
 }
 
 // banks whose iteration state is live at the same time: the 512-thread kernel (V > 32) iterates its banks side by side
@@ -1107,13 +1127,18 @@ size_t mta_scratch_bytes(int64_t n_problems, int V, int C, int D) {
   return b;
 }
 
+bool mta_shape_supported(int V, int C, int D) {
+  return V >= 1 && V <= 2048                    // small state must stay well inside shared memory
+         && C >= 1 && D >= 32 && D % 32 == 0 && D <= 1024;
+}
+
 cudaError_t launch_mta(const MtaSet* sets, int n_sets, int64_t I, int V, int C, int D, const MtaParams& p,
-                       float* scratch, cudaStream_t stream, int* dev_status, int num_sms) {
-  if (V < 1 || C < 1 || D < 32 || D % 32 != 0 || D > 1024) return cudaErrorInvalidValue;
-  if (V > 2048) return cudaErrorInvalidValue;  // small state must stay well inside shared memory
+                       float* scratch, cudaStream_t stream, int* dev_status, int num_sms, const MtaDebug* debug) {
+  if (!mta_shape_supported(V, C, D)) return cudaErrorInvalidValue;
   if (n_sets < 1 || n_sets > MTA_MAX_SETS) return cudaErrorInvalidValue;
   if (I == 0) return cudaSuccess;
   MtaDev a;
+  a.dbg = debug ? *debug : MtaDebug{nullptr, nullptr, nullptr};
   for (int s = 0; s < n_sets; ++s) a.sets[s] = sets[s];
   for (int s = n_sets; s < MTA_MAX_SETS; ++s) a.sets[s] = sets[0];
   a.I = I; a.V = V; a.C = C; a.D = D;

@@ -37,24 +37,28 @@ def cdist(x1, x2):
 
 
 @torch.no_grad()
-def solve_mta(image_features, text_features, return_state=False):
+def solve_mta(image_features, text_features, return_state=False, *, dtype=torch.float32, lambda_y=LAMBDA_Y,
+              lambda_q=LAMBDA_Q, th=TH, temperature=TEMPERATURE, k_frac=K_FRAC, max_iter=MAX_ITER):
     """image_features [V,512] unit rows (row 0 = un-augmented view), text_features [512,C].
-    Returns the unit mode [1,512] (test.py:1461)."""
-    x = image_features.to(torch.float32)
-    t = text_features.to(torch.float32)
+    Returns the unit mode [1,512] (test.py:1461).
+
+    `dtype` is the arithmetic precision (float64 gives the reference the kernels' fp32 rounding is measured against);
+    the keywords are the solver's constants (jcb_mta_params), defaulting to the reference's."""
+    x = image_features.to(dtype)
+    t = text_features.to(dtype)
     logits = x @ t * 100                                           # :1393
     V = x.shape[0]
 
     dist = cdist(x, x)                                             # :1403
     sorted_dist, _ = torch.sort(dist, dim=1)                       # :1404 jt.argsort -> (idx, values), ascending
-    k = max(int(K_FRAC * (V - 1)), 1)                              # :1405 (+ max, see docstring)
+    k = max(int(k_frac * (V - 1)), 1)                              # :1405 (+ max, see docstring)
     selected = sorted_dist[:, 1:k + 1] ** 2                        # :1406
     bandwidth = torch.sqrt(0.5 * selected.mean(dim=1))             # :1407-1408
 
-    p = torch.softmax(logits / TEMPERATURE, dim=1)
+    p = torch.softmax(logits / temperature, dim=1)
     affinity = p @ p.t()                                           # :1411
 
-    y = torch.ones(V, dtype=torch.float32) / V                     # :1414
+    y = torch.ones(V, dtype=dtype) / V                             # :1414
     mode = x[0]                                                    # :1417-1418
     it = 0
     while True:                                                    # :1424
@@ -64,8 +68,8 @@ def solve_mta(image_features, text_features, return_state=False):
             i += 1
             old_y = y
             weighted_affinity = affinity * y.unsqueeze(0)          # :1433
-            y = torch.softmax(1 / LAMBDA_Y * (density + LAMBDA_Q * weighted_affinity.sum(dim=1)), dim=-1)  # :1434
-            if torch.norm(old_y - y) < TH or i >= MAX_ITER:        # :1436
+            y = torch.softmax(1 / lambda_y * (density + lambda_q * weighted_affinity.sum(dim=1)), dim=-1)  # :1434
+            if torch.norm(old_y - y) < th or i >= max_iter:        # :1436
                 break
         i = 0
         while True:                                                # :1443
@@ -75,10 +79,10 @@ def solve_mta(image_features, text_features, return_state=False):
             w = density * y                                        # :1447
             mode = (w.unsqueeze(1) * x).sum(dim=0) / w.sum()       # :1448
             mode = mode / mode.norm(p=2, dim=-1)                   # :1449
-            if torch.norm(old_mode - mode) < TH or i >= MAX_ITER:  # :1452
+            if torch.norm(old_mode - mode) < th or i >= max_iter:  # :1452
                 break
         it += 1                                                    # :1455
-        if it >= MAX_ITER:
+        if it >= max_iter:
             break
     if return_state:
         return mode.unsqueeze(0), {"bandwidth": bandwidth, "affinity": affinity, "y": y, "logits": logits}
