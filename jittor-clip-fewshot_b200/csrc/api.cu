@@ -18,13 +18,13 @@
 using namespace jcb;
 
 namespace jcb {
-// Programmatic dependent launch is OPT-IN (JCB_PDL=1).  Measured with it on AND the explicit early trigger
-// (griddepcontrol.launch_dependents right after the wait, now only with -DJCB_PDL_EARLY_TRIGGER): one image x 65 views per
+// Programmatic dependent launch is OPT-IN (JCB_PDL=1).  Measured with it on AND an explicit early trigger
+// (griddepcontrol.launch_dependents right after the wait, since removed): one image x 65 views per
 // call 1.43 -> 1.39 ms (CUDA graphs) / 1.59 -> 1.43 (no graphs), the batched step +0.5 %, all GPU tests green -- but two
 // FULL-SIZE pipeline calls adjacent in the stream (call k's head kernel directly followed by call k + 1's im2col while
 // call k is still running) never finish: tools/pdl_first_calls_probe.py, profiles/r02_pdl_hang_probes.log (one GPU, no
-// NCCL).  Without the early trigger (the shipped build: dependents are released by the exit of the primary's CTAs) the same
-// probe finishes; that form was checked by the probe and a test subset only, hence still not the default.
+// NCCL).  Without the early trigger (dependents are released by the exit of the primary's CTAs) the same probe
+// finishes; that form was checked by the probe and a test subset only, hence still not the default.
 bool pdl_enabled() {
   static const bool on = [] { const char* e = getenv("JCB_PDL"); return e && e[0] == '1'; }();
   return on;
@@ -82,8 +82,6 @@ struct jcb_ctx {
   int cls_only_last = 0;             // opt-in: last block of the image tower on the class-token rows only (see tower_blocks)
   bool overlapped = false;           // this submission was enqueued behind an un-waited one: its first upload is hidden
   int64_t launches = 0;
-  int ln_fold = 2;                   // LayerNorm folded into the GEMMs (EPI_LNFOLD_* / EPI_RESID_LNPREP_*):
-                                     // 0 none, 1 ln_1 only (c_proj -> QKV), 2 ln_1 and ln_2
   int operand_f16 = 1;               // 16-bit operand type towers are packed with: 1 = fp16 (default), 0 = bf16
   int lora_applied = 0;              // how towers packed from now on carry their LoRA adapters: 0 = merged into the
                                      // weights (default), 1 = applied as low-rank GEMMs (jcb_ctx_set_lora_mode)
@@ -401,20 +399,19 @@ int tower_blocks(TowerBase* t, int64_t n, const TowerWs& w, int causal, bool cls
   const int M = static_cast<int>(n * T);
   const double MW = static_cast<double>(M) * W;
   int rc;
-  if (ctx->ln_fold && t->layers[0].in_wf != nullptr) {
-    // LayerNorm folded into the GEMMs: for a folded LayerNorm, w.ln_out holds the CENTRED 16-bit copy of the residual
-    // stream (x - shift[row]), w.stats[cur] its per-row partial sums and w.shift[cur] the shift (written by the embed
-    // kernel for block 0, then by the residual epilogue of the producing GEMM), and no stand-alone pass reads the
-    // fp32 residual stream.
-    //   ln_fold >= 1: ln_1 (c_proj of block l-1 -> QKV of block l).  c_proj's 48 k-blocks per tile hide the heavier
-    //                 epilogue; measured net gain (-1.5 ms / step).
-    //   ln_fold == 2: ln_2 as well (out_proj -> c_fc); the default.  out_proj is HBM-bound and pays 12 instead of 10
-    //                 bytes per element (6.9 -> 9.3 ms), c_fc's epilogue gets one FMA heavier (+0.3 ms); the 4.0 ms ln_2
-    //                 pass disappears.  A net loss while c_fc ran a 4-stage operand ring (its heavier epilogue then
-    //                 stalled an already starved main loop); with 5 stages a net gain of 1.5-3 ms / step.
-    const bool fold2 = ctx->ln_fold >= 2;
+  if (t->layers[0].in_wf != nullptr) {
+    // Both LayerNorms folded into the GEMMs (towers packed with merged or no LoRA): w.ln_out holds the CENTRED 16-bit
+    // copy of the residual stream (x - shift[row]), w.stats[cur] its per-row partial sums and w.shift[cur] the shift
+    // (written by the embed kernel for block 0, then by the residual epilogue of the producing GEMM), and no
+    // stand-alone pass reads the fp32 residual stream.
+    //   ln_1 (c_proj of block l-1 -> QKV of block l): c_proj's 48 k-blocks per tile hide the heavier epilogue;
+    //       measured net gain (-1.5 ms / step).
+    //   ln_2 (out_proj -> c_fc): out_proj is HBM-bound and pays 12 instead of 10 bytes per element (6.9 -> 9.3 ms),
+    //       c_fc's epilogue gets one FMA heavier (+0.3 ms); the 4.0 ms ln_2 pass disappears.  A net loss while c_fc
+    //       ran a 4-stage operand ring (its heavier epilogue then stalled an already starved main loop); with 5 stages
+    //       a net gain: 75.7-76.0 vs 77.2-78.7 ms / step with ln_1 folded alone (same B200).
     const int slots = (W + 255) / 256;
-    const bool cls_only = cls_row0 && ctx->cls_only_last && fold2 && !causal && T <= 64;
+    const bool cls_only = cls_row0 && ctx->cls_only_last && !causal && T <= 64;
     int cur = 0;   // which of w.stats / w.shift describes the copy in w.ln_out
     auto consumer = [&]() { LnArgs a; a.stats = w.stats[cur]; a.slots = slots; return a; };
     auto producer = [&](int64_t in_stride) {
@@ -458,19 +455,14 @@ int tower_blocks(TowerBase* t, int64_t n, const TowerWs& w, int causal, bool cls
       }
       LAUNCH_P(ctx, JCB_KC_ATTENTION, 4.0 * n * t->heads * T * T * 64, MW * (6 + 2),
                launch_attention(w.qkv, n, T, t->heads, w.attn, s, causal, ctx->dev_status, ctx->num_sms, f16));
-      if (fold2) {
-        {
-          LnArgs a = producer(1);
-          if ((rc = run_gemm(ctx, JCB_KC_GEMM_OUT, f16, w.attn, L.out_w, M, W, W, L.out_b, EPI_RESID_LNPREP_SHORT, w.tokens, W, a))) return rc;
-        }
+      {
+        LnArgs a = producer(1);
+        if ((rc = run_gemm(ctx, JCB_KC_GEMM_OUT, f16, w.attn, L.out_w, M, W, W, L.out_b, EPI_RESID_LNPREP_SHORT, w.tokens, W, a))) return rc;
+      }
+      {
         LnArgs a = consumer();
         a.colsum = L.fc_S;
         if ((rc = run_gemm(ctx, JCB_KC_GEMM_FC1, f16, w.ln_out, L.fc_wf, M, 4 * W, W, L.fc_c, EPI_LNFOLD_GELU_BF16, w.big, 4 * W, a))) return rc;
-      } else {
-        if ((rc = run_gemm(ctx, JCB_KC_GEMM_OUT, f16, w.attn, L.out_w, M, W, W, L.out_b, EPI_BIAS_RESID_F32, w.tokens, W))) return rc;
-        // ln_1's centred copy in w.ln_out was consumed by the QKV GEMM above; ln_2's stand-alone output replaces it
-        LAUNCH_P(ctx, JCB_KC_LAYERNORM, 0, MW * (4 + 2), launch_layernorm(w.tokens, M, W, L.ln2_g, L.ln2_b, w.ln_out, s, f16));
-        if ((rc = run_gemm(ctx, JCB_KC_GEMM_FC1, f16, w.ln_out, L.fc_w, M, 4 * W, W, L.fc_b, EPI_BIAS_GELU_BF16, w.big, 4 * W))) return rc;
       }
       if (l + 1 < t->L) {
         LnArgs a = producer(1);
@@ -539,7 +531,7 @@ int tower_forward(jcb_vit* v, const void* images, int dt, int64_t n, int apply_n
   if (rc) return rc;
   // class token + positional embedding + ln_pre (residual stream) + layer 0's ln_1
   LAUNCH_P(ctx, JCB_KC_EMBED_LN, 0, MW * (4 + 4 + 2), launch_embed_ln(w.tokens, n, T, W, v->cls, v->pos, v->vpt, v->cfg.vpt_tokens, v->ln_pre_g, v->ln_pre_b, v->layers[0].ln1_g,
-                              v->layers[0].ln1_b, w.ln_out, s, (ctx->ln_fold && v->layers[0].in_wf) ? w.stats[0] : nullptr, (W + 255) / 256,
+                              v->layers[0].ln1_b, w.ln_out, s, v->layers[0].in_wf ? w.stats[0] : nullptr, (W + 255) / 256,
                               patch_out, w.shift[0], v->f16));
   return tower_blocks(v, n, w, 0, /*cls_row0=*/true);   // the tail reads token row 0 only
 }
@@ -660,9 +652,6 @@ int jcb_ctx_create(int device, jcb_ctx** out) {
     ctx->lora_applied = (env_lm && (env_lm[0] == 'a' || env_lm[0] == 'A')) ? 1 : 0;
     const char* env_g = getenv("JCB_GRAPHS");
     ctx->graphs_on = (env_g && env_g[0] == '0') ? 0 : 1;
-    const char* env = getenv("JCB_LN_FOLD");
-    ctx->ln_fold = env ? atoi(env) : 2;   // default: both LayerNorms folded (measured, same box: 75.7-76.0 vs
-                                          // 77.2-78.7 ms / step for ln_1 only); see tower_blocks
   }
   ctx->cc_major = prop.major;
   ctx->cc_minor = prop.minor;
@@ -1072,7 +1061,7 @@ struct Packer {
       if ((rc = up_f32(blk(t, li, "ln_1.bias"), &Ld.ln1_b))) return rc;
       if ((rc = up_f32(blk(t, li, "ln_2.weight"), &Ld.ln2_g))) return rc;
       if ((rc = up_f32(blk(t, li, "ln_2.bias"), &Ld.ln2_b))) return rc;
-      if (ctx->ln_fold && !applied) {   // LoRA applied runs the stand-alone LayerNorm schedule (tower_blocks)
+      if (!applied) {   // LoRA applied runs the stand-alone LayerNorm schedule (tower_blocks)
         if ((rc = up_folded(blk(t, li, "attn.in_proj_weight"), 3 * W, W, in_ad, Ld.ln1_g, Ld.ln1_b, Ld.in_b, &Ld.in_wf,
                             &Ld.in_S, &Ld.in_c))) return rc;
         if ((rc = up_folded(blk(t, li, "mlp.c_fc.weight"), 4 * W, W, {}, Ld.ln2_g, Ld.ln2_b, Ld.fc_b, &Ld.fc_wf, &Ld.fc_S,
@@ -1254,7 +1243,7 @@ int jcb_encode_text(jcb_text* t, const int64_t* tokens_dev, int64_t n_seq, int n
     LAUNCH_P(ctx, JCB_KC_EMBED_LN, 0, MW * (4 + 4 + 2),
              launch_text_embed_ln(reinterpret_cast<const long long*>(tokens_dev) + off * T, m, T, W, t->cfg.vocab_size,
                                   t->tok_emb, t->pos, t->layers[0].ln1_g, t->layers[0].ln1_b, w.tokens, w.ln_out, eot,
-                                  ctx->stream, (ctx->ln_fold && t->layers[0].in_wf) ? w.stats[0] : nullptr, (W + 255) / 256,
+                                  ctx->stream, t->layers[0].in_wf ? w.stats[0] : nullptr, (W + 255) / 256,
                                   w.shift[0], t->f16));
     if ((rc = tower_blocks(t, m, w, 1))) return rc;
     LAUNCH_P(ctx, JCB_KC_TAIL, 2.0 * m * W * E, static_cast<double>(m) * (W + E) * 4,
@@ -1614,7 +1603,7 @@ struct PipelineGraph {
   const jcb_vit *vit = nullptr, *vit_zs = nullptr;
   uint64_t vit_gen = 0, zs_gen = 0, ws_gen = 0;
   int64_t I = 0;
-  int V = 0, dt = 0, apply_norm = 0, C = 0, rank_by = 0, k = 0, ln_fold = 0, cls_only = 0;
+  int V = 0, dt = 0, apply_norm = 0, C = 0, rank_by = 0, k = 0, cls_only = 0;
   const void* ptrs[10] = {nullptr};   // text banks (6) + head weights (4)
   cudaStream_t stream = nullptr;
   // state
@@ -1642,7 +1631,7 @@ bool graph_key_equal(const PipelineGraph& g, const jcb_ctx* ctx, const jcb_vit* 
   if (g.vit != vit || g.vit_zs != vit_zs || g.vit_gen != vit->gen || g.zs_gen != (vit_zs ? vit_zs->gen : 0) ||
       g.I != a->n_images || g.V != a->n_views || g.dt != a->img_dtype ||
       g.apply_norm != a->apply_clip_norm || g.C != a->n_classes || g.rank_by != a->rank_by || g.k != a->k ||
-      g.ln_fold != ctx->ln_fold || g.cls_only != ctx->cls_only_last || g.stream != ctx->stream)
+      g.cls_only != ctx->cls_only_last || g.stream != ctx->stream)
     return false;
   const void* p[10] = {a->text_pt_dev, a->text_hand_dev, a->text_zs_dev, a->text_pt_t_dev, a->text_hand_t_dev, a->text_zs_t_dev,
                        a->lp.scale1, a->lp.bias1, a->lp.fc_w, a->lp.fc_b};
@@ -1684,7 +1673,7 @@ int pipeline_try_graph(jcb_vit* vit, jcb_vit* vit_zs, const jcb_pipeline_args* a
     g = new PipelineGraph();
     g->vit = vit; g->vit_zs = vit_zs; g->vit_gen = vit->gen; g->zs_gen = vit_zs ? vit_zs->gen : 0;
     g->I = a->n_images; g->V = a->n_views; g->dt = a->img_dtype; g->apply_norm = a->apply_clip_norm; g->C = a->n_classes;
-    g->rank_by = a->rank_by; g->k = a->k; g->ln_fold = ctx->ln_fold; g->cls_only = ctx->cls_only_last; g->stream = ctx->stream;
+    g->rank_by = a->rank_by; g->k = a->k; g->cls_only = ctx->cls_only_last; g->stream = ctx->stream;
     const void* p[10] = {a->text_pt_dev, a->text_hand_dev, a->text_zs_dev, a->text_pt_t_dev, a->text_hand_t_dev, a->text_zs_t_dev,
                          a->lp.scale1, a->lp.bias1, a->lp.fc_w, a->lp.fc_b};
     for (int i = 0; i < 10; ++i) g->ptrs[i] = p[i];

@@ -1,19 +1,10 @@
-// Fused single-tile multi-head attention for short sequences: softmax(Q K^T / sqrt(64)) V per (sequence, head)
-// with Q, K and V held in shared memory, scores and probabilities never leaving registers.
-//   image tower : T <= 64 tokens (50 for ViT-B/32, 54 for the VPT variant), no mask                -> TP = 64
-//   text tower  : T <= 80 tokens (77), causal mask (jclip/model.py:189-193 build_attention_mask)    -> TP = 80
-//
-// One CTA = one sequence x HEADS_PER_CTA heads; each warp owns MT 16-row query tiles of one head.  Q K^T and P V
-// run on mma.sync m16n8k16 bf16 tiles with fp32 accumulation (a 64x64x64 problem per head is far below the
-// size where a tcgen05/TMEM round trip pays; this kernel is 1 % of the tower's FLOPs and is bounded by the
-// 8 B/element it streams).  Softmax is fp32 with exp2 and the 1/8 scale folded in.
-// Measured on B200 (tools/bench_kernel.py attention): 1 head per CTA, 1 query tile per warp -> 4.4 TB/s;
-// the first cut (4 heads per CTA, 2 tiles per warp, 148 registers) -> 2.5 TB/s.
+// Attention entry points: launch_attention (every full attention, on the tcgen05 / TMEM kernel of attention_tc.cu)
+// and the class-token-only kernel below.  The tcgen05 kernel replaced a round-1 mma.sync kernel (Q, K, V in smem) that
+// spent 2/3 of its time in the shared-memory pipe (profiles/r01f): 0.366 vs 0.568 ms per launch of 8320 views on a
+// B200 (DESIGN.md section 4).
 //
 // Reference: jclip/mha.py:55-83 scaled_dot_product_attention (attn_mask None for the vision tower,
 // jclip/model.py:99; dropout 0 in eval), head split jclip/mha.py:351-362 / test.py:584-590.
-#include <cstdlib>
-
 #include "kernels.h"
 #include "ptx.cuh"
 
@@ -22,189 +13,6 @@ namespace jcb {
 namespace {
 
 constexpr int HD = 64;       // head dim
-constexpr int LDS = HD + 8;  // smem row stride (bf16): 144 B, conflict-free for ldmatrix
-
-template <int HEADS_PER_CTA, int MT, int TP, bool CAUSAL, bool F16>
-__global__ void __launch_bounds__(HEADS_PER_CTA * (TP / 16 / MT) * 32)
-attention_kernel(const __nv_bfloat16* __restrict__ qkv, int T, int heads, __nv_bfloat16* __restrict__ out) {
-  constexpr int WPH = TP / 16 / MT;  // warps per head
-  constexpr int ATT_THREADS = HEADS_PER_CTA * WPH * 32;
-  constexpr int TILE_ELEMS = TP * LDS;
-  constexpr int NT = TP / 8;   // 8-wide key tiles
-  constexpr int KS = TP / 16;  // 16-deep key steps of P V
-  extern __shared__ __align__(16) uint8_t att_smem[];
-  __nv_bfloat16* sm = reinterpret_cast<__nv_bfloat16*>(att_smem);
-  const int W = heads * HD;
-  const int groups = heads / HEADS_PER_CTA;
-  const long long view = blockIdx.x / groups;
-  const int hg = blockIdx.x % groups;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const __nv_bfloat16* base = qkv + view * T * (3LL * W) + hg * HEADS_PER_CTA * HD;
-
-  // ---- stage Q, K, V of the CTA's heads: tile (h, m) at sm + (h*3 + m) * TILE_ELEMS, rows >= T zeroed
-  constexpr int CH_PER_ROW = HEADS_PER_CTA * HD / 8;  // 16-byte chunks per (row, matrix)
-  for (int i = tid; i < 3 * TP * CH_PER_ROW; i += ATT_THREADS) {
-    const int m = i / (TP * CH_PER_ROW);
-    const int rem = i % (TP * CH_PER_ROW);
-    const int row = rem / CH_PER_ROW, ch = rem % CH_PER_ROW;
-    const int h = ch / (HD / 8), c8 = (ch % (HD / 8)) * 8;
-    __nv_bfloat16* dst = sm + (h * 3 + m) * TILE_ELEMS + row * LDS + c8;
-    if (row < T) {
-      cp_async_16(smem_u32(dst), base + static_cast<long long>(row) * (3 * W) + m * W + ch * 8);
-    } else {
-      *reinterpret_cast<uint4*>(dst) = make_uint4(0u, 0u, 0u, 0u);
-    }
-  }
-  cp_async_commit_wait_all();
-  __syncthreads();
-
-  const int h = warp / WPH;                 // head within the group
-  const int r0 = (warp % WPH) * (16 * MT);  // first query row of this warp
-  const uint32_t sQ = smem_u32(sm + (h * 3 + 0) * TILE_ELEMS);
-  const uint32_t sK = smem_u32(sm + (h * 3 + 1) * TILE_ELEMS);
-  const uint32_t sV = smem_u32(sm + (h * 3 + 2) * TILE_ELEMS);
-
-  // ---- S = Q K^T : MT m-tiles x NT key tiles x 4 k-steps (head dim)
-  float s[MT][NT][4];
-#pragma unroll
-  for (int mt = 0; mt < MT; ++mt)
-#pragma unroll
-    for (int nt = 0; nt < NT; ++nt)
-#pragma unroll
-      for (int e = 0; e < 4; ++e) s[mt][nt][e] = 0.f;
-#pragma unroll
-  for (int kk = 0; kk < 4; ++kk) {
-    uint32_t a[MT][4];
-#pragma unroll
-    for (int mt = 0; mt < MT; ++mt) {
-      const int row = r0 + mt * 16 + (lane & 15);
-      const int col = kk * 16 + ((lane >> 4) << 3);
-      ldmatrix_x4(a[mt], sQ + (row * LDS + col) * 2);
-    }
-#pragma unroll
-    for (int np = 0; np < NT / 2; ++np) {  // pairs of key tiles
-      uint32_t b[4];
-      const int krow = np * 16 + (lane & 7) + ((lane >> 4) << 3);
-      const int col = kk * 16 + (((lane >> 3) & 1) << 3);
-      ldmatrix_x4(b, sK + (krow * LDS + col) * 2);
-#pragma unroll
-      for (int mt = 0; mt < MT; ++mt) {
-        if (F16) {
-          mma_f16_16816(s[mt][2 * np], a[mt], b[0], b[1]);
-          mma_f16_16816(s[mt][2 * np + 1], a[mt], b[2], b[3]);
-        } else {
-          mma_bf16_16816(s[mt][2 * np], a[mt], b[0], b[1]);
-          mma_bf16_16816(s[mt][2 * np + 1], a[mt], b[2], b[3]);
-        }
-      }
-    }
-  }
-
-  // ---- softmax over keys (fp32); thread holds rows g and g+8 of each m-tile, cols nt*8 + 2*(lane&3) + {0,1}
-  const float scale_log2 = 0.125f * 1.4426950408889634f;  // 1/sqrt(64) * log2(e)
-  float inv_sum[MT][2];
-  uint32_t pfrag[MT][NT][2];  // P as bf16 pairs: [mt][nt][row half]
-#pragma unroll
-  for (int mt = 0; mt < MT; ++mt) {
-    const int q0 = r0 + mt * 16 + (lane >> 2);  // this thread's query rows: q0 and q0 + 8
-    float mx[2] = {-INFINITY, -INFINITY};
-#pragma unroll
-    for (int nt = 0; nt < NT; ++nt) {
-      const int c0 = nt * 8 + 2 * (lane & 3);
-      // keys beyond the sequence and (text tower) keys after the query are masked out
-      if (c0 >= T || (CAUSAL && c0 > q0)) s[mt][nt][0] = -INFINITY;
-      if (c0 + 1 >= T || (CAUSAL && c0 + 1 > q0)) s[mt][nt][1] = -INFINITY;
-      if (c0 >= T || (CAUSAL && c0 > q0 + 8)) s[mt][nt][2] = -INFINITY;
-      if (c0 + 1 >= T || (CAUSAL && c0 + 1 > q0 + 8)) s[mt][nt][3] = -INFINITY;
-      mx[0] = fmaxf(mx[0], fmaxf(s[mt][nt][0], s[mt][nt][1]));
-      mx[1] = fmaxf(mx[1], fmaxf(s[mt][nt][2], s[mt][nt][3]));
-    }
-    float sum[2] = {0.f, 0.f};
-#pragma unroll
-    for (int hh = 0; hh < 2; ++hh) {
-      mx[hh] = fmaxf(mx[hh], __shfl_xor_sync(0xffffffffu, mx[hh], 1));
-      mx[hh] = fmaxf(mx[hh], __shfl_xor_sync(0xffffffffu, mx[hh], 2));
-    }
-#pragma unroll
-    for (int nt = 0; nt < NT; ++nt) {
-      const float p0 = exp2f((s[mt][nt][0] - mx[0]) * scale_log2);
-      const float p1 = exp2f((s[mt][nt][1] - mx[0]) * scale_log2);
-      const float p2 = exp2f((s[mt][nt][2] - mx[1]) * scale_log2);
-      const float p3 = exp2f((s[mt][nt][3] - mx[1]) * scale_log2);
-      sum[0] += p0 + p1;
-      sum[1] += p2 + p3;
-      pfrag[mt][nt][0] = pack_h2<F16>(p0, p1);
-      pfrag[mt][nt][1] = pack_h2<F16>(p2, p3);
-    }
-#pragma unroll
-    for (int hh = 0; hh < 2; ++hh) {
-      sum[hh] += __shfl_xor_sync(0xffffffffu, sum[hh], 1);
-      sum[hh] += __shfl_xor_sync(0xffffffffu, sum[hh], 2);
-      inv_sum[mt][hh] = 1.0f / sum[hh];
-    }
-  }
-
-  // ---- O = P V : MT m-tiles x 8 d-tiles x KS k-steps (keys)
-  float o[MT][8][4];
-#pragma unroll
-  for (int mt = 0; mt < MT; ++mt)
-#pragma unroll
-    for (int dt = 0; dt < 8; ++dt)
-#pragma unroll
-      for (int e = 0; e < 4; ++e) o[mt][dt][e] = 0.f;
-#pragma unroll
-  for (int ks = 0; ks < KS; ++ks) {
-    uint32_t a[MT][4];
-#pragma unroll
-    for (int mt = 0; mt < MT; ++mt) {
-      a[mt][0] = pfrag[mt][2 * ks][0];
-      a[mt][1] = pfrag[mt][2 * ks][1];
-      a[mt][2] = pfrag[mt][2 * ks + 1][0];
-      a[mt][3] = pfrag[mt][2 * ks + 1][1];
-    }
-#pragma unroll
-    for (int dp = 0; dp < 4; ++dp) {  // pairs of d tiles
-      uint32_t b[4];
-      const int krow = ks * 16 + (lane & 7) + (((lane >> 3) & 1) << 3);
-      const int col = dp * 16 + ((lane >> 4) << 3);
-      ldmatrix_x4_trans(b, sV + (krow * LDS + col) * 2);
-#pragma unroll
-      for (int mt = 0; mt < MT; ++mt) {
-        if (F16) {
-          mma_f16_16816(o[mt][2 * dp], a[mt], b[0], b[1]);
-          mma_f16_16816(o[mt][2 * dp + 1], a[mt], b[2], b[3]);
-        } else {
-          mma_bf16_16816(o[mt][2 * dp], a[mt], b[0], b[1]);
-          mma_bf16_16816(o[mt][2 * dp + 1], a[mt], b[2], b[3]);
-        }
-      }
-    }
-  }
-
-  // ---- normalise, stage through this warp's own Q rows (dead by now), coalesced store
-  __nv_bfloat16* stage = sm + (h * 3 + 0) * TILE_ELEMS;
-  __syncwarp();
-#pragma unroll
-  for (int mt = 0; mt < MT; ++mt) {
-    const int row = r0 + mt * 16 + (lane >> 2);
-#pragma unroll
-    for (int dt = 0; dt < 8; ++dt) {
-      const int col = dt * 8 + 2 * (lane & 3);
-      *reinterpret_cast<uint32_t*>(stage + row * LDS + col) =
-          pack_h2<F16>(o[mt][dt][0] * inv_sum[mt][0], o[mt][dt][1] * inv_sum[mt][0]);
-      *reinterpret_cast<uint32_t*>(stage + (row + 8) * LDS + col) =
-          pack_h2<F16>(o[mt][dt][2] * inv_sum[mt][1], o[mt][dt][3] * inv_sum[mt][1]);
-    }
-  }
-  __syncthreads();
-  __nv_bfloat16* obase = out + view * T * static_cast<long long>(W) + hg * HEADS_PER_CTA * HD;
-  for (int i = tid; i < T * CH_PER_ROW; i += ATT_THREADS) {
-    const int row = i / CH_PER_ROW, ch = i % CH_PER_ROW;
-    const int hh = ch / (HD / 8), c8 = (ch % (HD / 8)) * 8;
-    const uint4 v = *reinterpret_cast<const uint4*>(sm + (hh * 3 + 0) * TILE_ELEMS + row * LDS + c8);
-    *reinterpret_cast<uint4*>(obase + static_cast<long long>(row) * W + ch * 8) = v;
-  }
-}
 
 // Attention for the class token only: softmax(q_0 K^T / 8) V for query row 0 of every (sequence, head).  Used by
 // the opt-in "last block on the class token only" schedule (api.cu): encode_image returns ln_post(x[:, 0, :]) @ proj
@@ -273,30 +81,6 @@ attention_cls_kernel(const __nv_bfloat16* __restrict__ qkv, long long n_items, i
   *reinterpret_cast<uint32_t*>(out + seq * W + h * HD + 2 * lane) = pack_h2<F16>(o0 * inv, o1 * inv);
 }
 
-template <int TP, bool CAUSAL, bool F16>
-cudaError_t launch_attention_cfg(const __nv_bfloat16* qkv, int64_t n_views, int T, int heads, __nv_bfloat16* out,
-                                 cudaStream_t stream) {
-  // one head per CTA, one 16-row query tile per warp: the fastest of the configurations tried in round 1 (4.4 TB/s;
-  // 4 heads per CTA and 2 tiles per warp: 2.5 TB/s)
-  constexpr int SMEM = 3 * TP * LDS * 2;
-  constexpr int THREADS = (TP / 16) * 32;
-  {
-    cudaError_t e = ensure_dynamic_smem(attention_kernel<1, 1, TP, CAUSAL, F16>, SMEM);
-    if (e != cudaSuccess) return e;
-  }
-  const long long grid = n_views * heads;
-  attention_kernel<1, 1, TP, CAUSAL, F16><<<static_cast<unsigned>(grid), THREADS, SMEM, stream>>>(qkv, T, heads, out);
-  return cudaGetLastError();
-}
-
-template <bool F16>
-cudaError_t launch_attention_mma(const __nv_bfloat16* qkv, int64_t n_views, int T, int heads, __nv_bfloat16* out,
-                                 cudaStream_t stream, int causal) {
-  if (causal) return launch_attention_cfg<80, true, F16>(qkv, n_views, T, heads, out, stream);
-  if (T > 64) return launch_attention_cfg<80, false, F16>(qkv, n_views, T, heads, out, stream);
-  return launch_attention_cfg<64, false, F16>(qkv, n_views, T, heads, out, stream);
-}
-
 }  // namespace
 
 cudaError_t launch_attention_cls(const __nv_bfloat16* qkv, int64_t n_views, int T, int heads, __nv_bfloat16* out,
@@ -310,22 +94,11 @@ cudaError_t launch_attention_cls(const __nv_bfloat16* qkv, int64_t n_views, int 
   return cudaGetLastError();
 }
 
-// Default: the tcgen05 / TMEM kernel (attention_tc.cu) for every shape it supports (T <= 128: both towers).  The
-// mma.sync kernel above remains as the A/B baseline (JCB_ATT_IMPL=mma; T <= 80) it was in round 1.
 cudaError_t launch_attention(const __nv_bfloat16* qkv, int64_t n_views, int T, int heads, __nv_bfloat16* out,
                              cudaStream_t stream, int causal, int* dev_status, int num_sms, int f16) {
   if (T < 1 || T > 128 || heads < 1) return cudaErrorInvalidValue;
   if (n_views == 0) return cudaSuccess;
-  static int impl = -1;  // 1: tcgen05 kernel (default), 0: mma.sync kernel
-  if (impl < 0) {
-    const char* env = getenv("JCB_ATT_IMPL");
-    impl = (env && env[0] == 'm') ? 0 : 1;
-  }
-  if (impl == 1 && dev_status != nullptr && num_sms > 0 && attention_tc_supported(T, heads, causal))
-    return launch_attention_tc(qkv, n_views, T, heads, out, stream, dev_status, num_sms, f16, causal);
-  if (T > 80) return cudaErrorInvalidValue;
-  return f16 ? launch_attention_mma<true>(qkv, n_views, T, heads, out, stream, causal)
-             : launch_attention_mma<false>(qkv, n_views, T, heads, out, stream, causal);
+  return launch_attention_tc(qkv, n_views, T, heads, out, stream, dev_status, num_sms, f16, causal);
 }
 
 }  // namespace jcb

@@ -103,7 +103,6 @@ attention_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid
   tc_fence_after();
   const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(tmem_ptr_smem);
   griddep_wait();               // programmatic dependent launch (ptx.cuh): nothing global is touched above
-  griddep_launch_dependents();
 
   if (warp_idx == 0) {
     // ===================================================================== TMA producer

@@ -8,14 +8,11 @@
 //                                vectorised global stores; TMEM accumulators are double buffered so the
 //                                epilogue of tile i overlaps the main loop of tile i+1
 //
-// Two tile configurations of the same kernel (template parameter CTAS):
-//   CTAS = 2 (default)  CTA pairs (cluster 2x1x1, tcgen05 cta_group::2): UMMA 256 x BN x 16 across two SMs.
-//                       Each CTA stages its 128 rows of A and HALF of the B tile (BN/2 rows); the tensor core
-//                       reads both halves.  Per CTA and k-block that is 32 KB of TMA writes + 8 KB/MMA of
-//                       operand reads = 128 B/cycle, exactly the shared-memory bandwidth of an SM.
-//   CTAS = 1            UMMA 128 x BN x 16 from one CTA: 48 KB written + 12 KB/MMA read = 192 B/cycle demanded of
-//                       a 128 B/cycle SMEM -> the tensor pipe cannot exceed ~66 % (measured 64 %, profiles/r01a).
-//                       Kept selectable (JCB_GEMM_CTAS=1) as the A/B baseline.
+// CTA pairs (cluster 2x1x1, tcgen05 cta_group::2): UMMA 256 x BN x 16 across two SMs.  Each CTA stages its 128 rows
+// of A and HALF of the B tile (BN/2 rows); the tensor core reads both halves.  Per CTA and k-block that is 32 KB of
+// TMA writes + 8 KB/MMA of operand reads = 128 B/cycle, exactly the shared-memory bandwidth of an SM.  A single-CTA
+// UMMA 128 x BN x 16 would demand 48 KB written + 12 KB/MMA read = 192 B/cycle of a 128 B/cycle SMEM: its tensor pipe
+// cannot exceed ~66 % (measured 64 %, profiles/r01a), so that form was removed.
 //
 // This replaces the reference's fp32 `nn.Linear` calls on the hot path: packed QKV projection
 // (jclip/mha.py:129-146, test.py:557-559), attention out-proj (jclip/mha.py:461, test.py:594), MLP
@@ -23,10 +20,8 @@
 // (jclip/model.py:105-108).  Residual adds (jclip/model.py:60-61), QuickGELU (jclip/model.py:27) and the
 // positional-embedding add (jclip/model.py:114) are fused into the epilogues.
 #include <cstdio>
-#include <cstdlib>
 #include <mutex>
 #include <unordered_map>
-#include <vector>
 #include <cudaTypedefs.h>
 
 #include "kernels.h"
@@ -41,7 +36,7 @@ constexpr int BLOCK_K = 64;   // 64 bf16 = 128 B = one swizzle atom row
 constexpr int UMMA_K = 16;
 // epilogue warps: 4 (one per TMEM lane quarter, all BN columns each); 8 (two per quarter, half the columns each) is
 // supported by the tile configuration but never pays: the epilogues are idle more than half of every tile
-// (JCB_GEMM_TRACE) -- measured c_fc 1284 (8 warps) vs 1337 (4 warps) TFLOP/s.
+// (clock64 role timeline of CTA 0, DESIGN.md) -- measured c_fc 1284 (8 warps) vs 1337 (4 warps) TFLOP/s.
 #ifndef JCB_GELU_WARPS
 #define JCB_GELU_WARPS 4
 #endif
@@ -51,9 +46,9 @@ __host__ __device__ constexpr int epi_warps_of(int epi) {
 
 // chunks converted per generic->async proxy fence / per batch of TMA stores = staging buffers per epilogue warp.
 // Every epilogue fences every 2 chunks and leaves the ring 5 stages (160 KB in flight per SM).  The role timeline
-// (JCB_GEMM_TRACE) shows why staging must not eat a ring stage: with 4 stages the c_fc GEMM's MMA issuer waits for
-// operands (157 cycles per UMMA instead of the pipe's 135-138) while its GELU epilogue idles 4.4 k of every 7.8 k
-// cycles -- the loads are latency-bound (~1.7 us under load), so bytes in flight set the rate.  Measured on B200
+// (clock64 stamps of CTA 0, DESIGN.md) shows why staging must not eat a ring stage: with 4 stages the c_fc GEMM's MMA
+// issuer waits for operands (157 cycles per UMMA instead of the pipe's 135-138) while its GELU epilogue idles 4.4 k of
+// every 7.8 k cycles -- the loads are latency-bound (~1.7 us under load), so bytes in flight set the rate.  Measured on B200
 // (tools/gpu_ab.sh): c_fc 1309 -> 1432 TFLOP/s with 5 stages; 6 stages with per-chunk fences gain 3 % on QKV but
 // cost the HBM-bound out_proj 10 %.  (JCB_* macros: A/B builds via build.py --variant.)
 #ifndef JCB_GELU_GROUP
@@ -85,7 +80,9 @@ __host__ __device__ constexpr int lnprep_nb(int epi) { return epi == EPI_RESID_L
 __host__ __device__ constexpr int lnprep_d(int epi) { return epi == EPI_RESID_LNPREP_SHORT ? JCB_LNS_D : 1; }
 __host__ __device__ constexpr int lnprep_nh(int epi) { return epi == EPI_RESID_LNPREP_SHORT ? JCB_LNS_NH : 1; }
 
-template <int BN, int CTAS, int EPI>
+constexpr int CTAS = 2;       // CTAs of a pair (one cluster) sharing each 256-row UMMA
+
+template <int BN, int EPI>
 struct TileCfg {
   static constexpr int EPI_WARPS = epi_warps_of(EPI);
   static constexpr int NUM_THREADS = 64 + 32 * EPI_WARPS;
@@ -125,27 +122,23 @@ struct GemmDev {
   float* shift_out;          // [M] new shift (written by the n_blk == 0 tiles)
   long long stats_in_stride; // row r of this GEMM = row r * stride of stats_in / shift_in (class-token-only last block)
   uint32_t idesc;            // tcgen05 instruction descriptor (operand formats, M, N)
-  int arrive_release;    // A/B: 1 = the old `.release.cluster` accumulator hand-back
-  long long* trace;      // debug (JCB_GEMM_TRACE=file): clock64 stamps of CTA 0's roles, [TRACE_TILES][8]
 };
-constexpr int TRACE_TILES = 96;
-#define JCB_TRACE(slot)                                                                  \
-  do {                                                                                   \
-    if (p.trace != nullptr && blockIdx.x == 0 && it < TRACE_TILES) p.trace[it * 8 + (slot)] = clock64(); \
-  } while (0)
 
-template <int BN, int EPI, int CTAS, bool F16>
-__device__ __forceinline__ void gemm_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmOut,
-                                          const CUtensorMap& tmOut2, const CUtensorMap& tmA2, const CUtensorMap& tmB2,
-                                          const GemmDev& p) {
-  using Cfg = TileCfg<BN, CTAS, EPI>;
+// F16 selects the element type of 16-bit OUTPUTS (the conversion instruction of the epilogue); the operand formats
+// the tensor core assumes travel in p.idesc, so the fp32-output epilogues need no second instantiation.
+template <int BN, int EPI, bool F16>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(64 + 32 * epi_warps_of(EPI), 1)
+gemm_tcgen05_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
+                         const __grid_constant__ CUtensorMap tmOut, const __grid_constant__ CUtensorMap tmOut2,
+                         const __grid_constant__ CUtensorMap tmA2, const __grid_constant__ CUtensorMap tmB2,
+                         const GemmDev p) {
+  using Cfg = TileCfg<BN, EPI>;
   constexpr int STAGES = Cfg::STAGES;
   constexpr int GROUP = Cfg::GROUP;
   constexpr int WARP_STAGING = Cfg::WARP_STAGING;
   constexpr int STAGING_BYTES = Cfg::STAGING_BYTES;
   constexpr int EPI_WARPS = Cfg::EPI_WARPS;
   constexpr int CW = Cfg::CW;
-  constexpr bool PAIR = CTAS == 2;
   extern __shared__ uint8_t smem_raw[];
   // 128B-swizzled TMA/UMMA tiles need 1024-byte alignment in the shared address space.
   const uint32_t raw_addr = smem_u32(smem_raw);
@@ -163,12 +156,12 @@ __device__ __forceinline__ void gemm_body(const CUtensorMap& tmA, const CUtensor
 
   const int warp_idx = __shfl_sync(0xffffffffu, static_cast<int>(threadIdx.x >> 5), 0);
   const int lane = threadIdx.x & 31;
-  const uint32_t cta_rank = PAIR ? cluster_ctarank() : 0u;
+  const uint32_t cta_rank = cluster_ctarank();
   const bool leader = cta_rank == 0;
 
-  // one work unit = one (CTA or CTA pair) x one output tile of (CTAS * 128) x BN
-  const int unit = PAIR ? static_cast<int>(blockIdx.x >> 1) : static_cast<int>(blockIdx.x);
-  const int num_units = PAIR ? static_cast<int>(gridDim.x >> 1) : static_cast<int>(gridDim.x);
+  // one work unit = one CTA pair x one output tile of (CTAS * 128) x BN
+  const int unit = static_cast<int>(blockIdx.x >> 1);
+  const int num_units = static_cast<int>(gridDim.x >> 1);
   constexpr int TILE_M = BLOCK_M * CTAS;
   const int m_tiles = (p.M + TILE_M - 1) / TILE_M;
   const int n_tiles = p.N / BN;
@@ -202,22 +195,16 @@ __device__ __forceinline__ void gemm_body(const CUtensorMap& tmA, const CUtensor
     fence_proxy_async_smem();
   }
   if (warp_idx == 1) {  // the same warp of BOTH CTAs of a pair takes part in a cta_group::2 allocation
-    if (PAIR) {
-      tmem_alloc_pair(tmem_ptr_smem, Cfg::TMEM_COLS);
-      tmem_relinquish_pair();
-    } else {
-      tmem_alloc(tmem_ptr_smem, Cfg::TMEM_COLS);
-      tmem_relinquish();
-    }
+    tmem_alloc_pair(tmem_ptr_smem, Cfg::TMEM_COLS);
+    tmem_relinquish_pair();
   }
   tc_fence_before();
-  if (PAIR) cluster_sync_all(); else __syncthreads();   // barriers of both CTAs initialised before anyone signals them
+  cluster_sync_all();   // barriers of both CTAs initialised before anyone signals them
   tc_fence_after();
   const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(tmem_ptr_smem);
   // programmatic dependent launch: everything above overlapped the previous kernel's tail; operands, bias, statistics
   // and the residual stream are touched only below
   griddep_wait();
-  griddep_launch_dependents();
 
   if (warp_idx == 0) {
     // ===================================================================== TMA producer (every CTA)
@@ -225,32 +212,23 @@ __device__ __forceinline__ void gemm_body(const CUtensorMap& tmA, const CUtensor
       int stage = 0;
       uint32_t phase = 0;
       bool ok = true;
-      int it = 0;
-      for (int tile = unit; tile < num_tiles && ok; tile += num_units, ++it) {
+      for (int tile = unit; tile < num_tiles && ok; tile += num_units) {
         const int m_blk = tile / n_tiles, n_blk = tile % n_tiles;
         const int m0 = m_blk * TILE_M + static_cast<int>(cta_rank) * BLOCK_M;
         const int n0 = n_blk * BN + static_cast<int>(cta_rank) * Cfg::B_ROWS;
         for (int kb = 0; kb < num_kb; ++kb) {
           if (!mbar_wait(&empty_bar[stage], phase ^ 1u, p.status, JCB_DEV_TIMEOUT_PRODUCER)) { ok = false; break; }
-          if (kb == 0) JCB_TRACE(5);
-          if (kb == num_kb - 1) JCB_TRACE(6);
           uint8_t* sa = ring + stage * Cfg::STAGE_BYTES;
           uint8_t* sb = sa + Cfg::A_BYTES;
           const bool second = kb >= num_kb1;
           const CUtensorMap* ta = second ? &tmA2 : &tmA;
           const CUtensorMap* tb = second ? &tmB2 : &tmB;
           const int k0 = (second ? kb - num_kb1 : kb) * BLOCK_K;
-          if (PAIR) {
-            // the leader's barrier collects the bytes of BOTH CTAs; a complete_tx that lands before the
-            // leader's expect_tx just drives the transaction count negative for a moment
-            if (leader) mbar_arrive_expect_tx(&full_bar[stage], 2 * Cfg::STAGE_BYTES);
-            tma_load_2d_pair(sa, ta, &full_bar[stage], k0, m0);
-            tma_load_2d_pair(sb, tb, &full_bar[stage], k0, n0);
-          } else {
-            mbar_arrive_expect_tx(&full_bar[stage], Cfg::STAGE_BYTES);
-            tma_load_2d(sa, ta, &full_bar[stage], k0, m0);
-            tma_load_2d(sb, tb, &full_bar[stage], k0, n0);
-          }
+          // the leader's barrier collects the bytes of BOTH CTAs; a complete_tx that lands before the
+          // leader's expect_tx just drives the transaction count negative for a moment
+          if (leader) mbar_arrive_expect_tx(&full_bar[stage], 2 * Cfg::STAGE_BYTES);
+          tma_load_2d_pair(sa, ta, &full_bar[stage], k0, m0);
+          tma_load_2d_pair(sb, tb, &full_bar[stage], k0, n0);
           if (++stage == STAGES) { stage = 0; phase ^= 1u; }
         }
       }
@@ -268,7 +246,6 @@ __device__ __forceinline__ void gemm_body(const CUtensorMap& tmA, const CUtensor
         const uint32_t aphase = (it >> 1) & 1;
         if (!mbar_wait(&tmem_empty_bar[as], aphase ^ 1u, p.status, JCB_DEV_TIMEOUT_MMA)) { ok = false; break; }
         tc_fence_after();
-        JCB_TRACE(0);
         const uint32_t tmem_d = tmem_base + static_cast<uint32_t>(as * BN);
         for (int kb = 0; kb < num_kb; ++kb) {
           if (!mbar_wait(&full_bar[stage], phase, p.status, JCB_DEV_TIMEOUT_MMA)) { ok = false; break; }
@@ -279,21 +256,14 @@ __device__ __forceinline__ void gemm_body(const CUtensorMap& tmA, const CUtensor
 #pragma unroll
           for (int k = 0; k < BLOCK_K / UMMA_K; ++k) {
             // +32 B per UMMA_K step inside the 128-B swizzle atom = +2 in the (addr >> 4) field
-            if (PAIR)
-              umma_bf16_pair(tmem_d, da + static_cast<uint64_t>(2 * k), db + static_cast<uint64_t>(2 * k), idesc,
-                             (kb | k) != 0 ? 1u : 0u);
-            else
-              umma_bf16(tmem_d, da + static_cast<uint64_t>(2 * k), db + static_cast<uint64_t>(2 * k), idesc,
-                        (kb | k) != 0 ? 1u : 0u);
+            umma_bf16_pair(tmem_d, da + static_cast<uint64_t>(2 * k), db + static_cast<uint64_t>(2 * k), idesc,
+                           (kb | k) != 0 ? 1u : 0u);
           }
           // smem slot reusable (in both CTAs) once these MMAs have read it
-          if (PAIR) umma_commit_pair(&empty_bar[stage]); else umma_commit(&empty_bar[stage]);
+          umma_commit_pair(&empty_bar[stage]);
           if (++stage == STAGES) { stage = 0; phase ^= 1u; }
         }
-        if (ok) {  // accumulator complete -> epilogue warps of both CTAs
-          if (PAIR) umma_commit_pair(&tmem_full_bar[as]); else umma_commit(&tmem_full_bar[as]);
-        }
-        JCB_TRACE(1);
+        if (ok) umma_commit_pair(&tmem_full_bar[as]);  // accumulator complete -> epilogue warps of both CTAs
       }
     }
   } else {
@@ -307,7 +277,7 @@ __device__ __forceinline__ void gemm_body(const CUtensorMap& tmA, const CUtensor
     float* s_csum = s_bias + CW;                          // ... and, LNFOLD only, the column sums S[n]
     uint64_t* my_lbar = load_bar + ew * 8;
     uint32_t lphase = 0;                                  // LNPREP: parity bit per staging buffer
-    const uint32_t empty_addr0 = smem_u32(&tmem_empty_bar[0]) & (PAIR ? PEER_BIT_MASK : 0xFFFFFFFFu);
+    const uint32_t empty_addr0 = smem_u32(&tmem_empty_bar[0]) & PEER_BIT_MASK;
     int it = 0;
     bool ok = true;
     for (int tile = unit; tile < num_tiles && ok; tile += num_units, ++it) {
@@ -347,7 +317,6 @@ __device__ __forceinline__ void gemm_body(const CUtensorMap& tmA, const CUtensor
       ok = __all_sync(0xffffffffu, ok);
       if (!ok) break;
       tc_fence_after();
-      if (ew == 0 && lane == 0) JCB_TRACE(2);
 
       const int row0 = m_blk * TILE_M + static_cast<int>(cta_rank) * BLOCK_M + q * 32;  // this warp's 32 rows
       const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + static_cast<uint32_t>(as * BN + col0);
@@ -390,11 +359,7 @@ __device__ __forceinline__ void gemm_body(const CUtensorMap& tmA, const CUtensor
           } else {
             tc_fence_before();
             __syncwarp();
-            if (ew == 0 && lane == 0) JCB_TRACE(3);
-            if (lane == 0) {
-              if (PAIR) { if (p.arrive_release) mbar_arrive_cluster_release(empty_addr0 + static_cast<uint32_t>(as * 8)); else mbar_arrive_cluster(empty_addr0 + static_cast<uint32_t>(as * 8)); }
-              else mbar_arrive(&tmem_empty_bar[as]);
-            }
+            if (lane == 0) mbar_arrive_cluster(empty_addr0 + static_cast<uint32_t>(as * 8));
           }
           const int b = c % NB;
           ok = mbar_wait(&my_lbar[b], (lphase >> b) & 1u, p.status, JCB_DEV_TIMEOUT_EPILOGUE);   // old chunk landed
@@ -506,11 +471,7 @@ __device__ __forceinline__ void gemm_body(const CUtensorMap& tmA, const CUtensor
             // (leader CTA) before the last chunk is even converted
             tc_fence_before();
             __syncwarp();
-            if (ew == 0 && lane == 0) JCB_TRACE(3);
-            if (lane == 0) {
-              if (PAIR) { if (p.arrive_release) mbar_arrive_cluster_release(empty_addr0 + static_cast<uint32_t>(as * 8)); else mbar_arrive_cluster(empty_addr0 + static_cast<uint32_t>(as * 8)); }
-              else mbar_arrive(&tmem_empty_bar[as]);
-            }
+            if (lane == 0) mbar_arrive_cluster(empty_addr0 + static_cast<uint32_t>(as * 8));
           }
           uint8_t* rowp = my_stage + (c % GROUP) * 4096 + lane * 128;
 #pragma unroll
@@ -565,43 +526,21 @@ __device__ __forceinline__ void gemm_body(const CUtensorMap& tmA, const CUtensor
           }
         }
       }
-      if (ew == 0 && lane == 0) JCB_TRACE(4);
     }
     if (lane == 0) bulk_wait<0>();  // every TMA store / reduce of this warp has been performed
   }
 
   tc_fence_before();
   // a CTA of a pair must not retire while its partner can still touch its smem / TMEM / barriers
-  if (PAIR) cluster_sync_all(); else __syncthreads();
+  cluster_sync_all();
   if (warp_idx == 1) {
     tc_fence_after();
-    if (PAIR) tmem_dealloc_pair(tmem_base, Cfg::TMEM_COLS); else tmem_dealloc(tmem_base, Cfg::TMEM_COLS);
+    tmem_dealloc_pair(tmem_base, Cfg::TMEM_COLS);
   }
-}
-
-// F16 selects the element type of 16-bit OUTPUTS (the conversion instruction of the epilogue); the operand formats
-// the tensor core assumes travel in p.idesc, so the fp32-output epilogues need no second instantiation.
-template <int BN, int EPI, bool F16>
-__global__ void __launch_bounds__(64 + 32 * epi_warps_of(EPI), 1)
-gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-                    const __grid_constant__ CUtensorMap tmOut, const __grid_constant__ CUtensorMap tmOut2,
-                    const __grid_constant__ CUtensorMap tmA2, const __grid_constant__ CUtensorMap tmB2,
-                    const GemmDev p) {
-  gemm_body<BN, EPI, 1, F16>(tmA, tmB, tmOut, tmOut2, tmA2, tmB2, p);
-}
-
-template <int BN, int EPI, bool F16>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(64 + 32 * epi_warps_of(EPI), 1)
-gemm_tcgen05_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-                         const __grid_constant__ CUtensorMap tmOut, const __grid_constant__ CUtensorMap tmOut2,
-                         const __grid_constant__ CUtensorMap tmA2, const __grid_constant__ CUtensorMap tmB2,
-                         const GemmDev p) {
-  gemm_body<BN, EPI, 2, F16>(tmA, tmB, tmOut, tmOut2, tmA2, tmB2, p);
 }
 
 PFN_cuTensorMapEncodeTiled_v12000 g_encode_tiled = nullptr;
 char g_driver_err[256] = {0};
-int g_ctas = 0;  // 0 = not decided yet
 
 // Encoded tensor maps are pure functions of (base, shape, strides, box, type): the towers launch the same few
 // hundred (pointer, shape) combinations every pass, so they are encoded once and looked up afterwards
@@ -654,9 +593,9 @@ bool make_tmap_2d(CUtensorMap* tm, int dtype, const void* base, uint64_t rows, u
   return true;
 }
 
-template <int BN, int EPI, int CTAS, bool F16>
+template <int BN, int EPI, bool F16>
 cudaError_t launch_cfg(const GemmArgs& a, int* dev_status, int num_sms, cudaStream_t stream) {
-  using Cfg = TileCfg<BN, CTAS, EPI>;
+  using Cfg = TileCfg<BN, EPI>;
   const int op_dt = a.f16 ? TM_F16 : TM_BF16;
   CUtensorMap tmA, tmB, tmOut;
   if (!make_tmap_2d(&tmA, op_dt, a.A, a.M, a.K, a.lda, BLOCK_M, BLOCK_K)) return cudaErrorInvalidValue;
@@ -676,7 +615,7 @@ cudaError_t launch_cfg(const GemmArgs& a, int* dev_status, int num_sms, cudaStre
     if (!make_tmap_2d(&tmA2, op_dt, a.A2, a.M, a.K2, a.lda2, BLOCK_M, BLOCK_K)) return cudaErrorInvalidValue;
     if (!make_tmap_2d(&tmB2, op_dt, a.B2, a.N, a.K2, a.ldb2, Cfg::B_ROWS, BLOCK_K)) return cudaErrorInvalidValue;
   }
-  auto kern = CTAS == 2 ? gemm_tcgen05_2cta_kernel<BN, EPI, F16> : gemm_tcgen05_kernel<BN, EPI, F16>;
+  auto kern = gemm_tcgen05_2cta_kernel<BN, EPI, F16>;
   {
     cudaError_t e = ensure_dynamic_smem(kern, Cfg::SMEM_BYTES);
     if (e != cudaSuccess) return e;
@@ -688,53 +627,22 @@ cudaError_t launch_cfg(const GemmArgs& a, int* dev_status, int num_sms, cudaStre
   p.stats_in = a.stats_in; p.shift_in = a.shift_in; p.shift_out = a.shift_out;
   p.stats_in_stride = a.stats_in_row_stride > 0 ? a.stats_in_row_stride : 1;
   p.idesc = umma_idesc_f32acc(a.f16 != 0, BLOCK_M * CTAS, BN);
-  static int arrive_release = -1;
-  if (arrive_release < 0) {
-    const char* env = getenv("JCB_GEMM_ARRIVE_RELEASE");
-    arrive_release = (env && env[0] == '1') ? 1 : 0;
-  }
-  p.arrive_release = arrive_release;
-  static const char* trace_path = getenv("JCB_GEMM_TRACE");
-  static long long* trace_dev = nullptr;
-  p.trace = nullptr;
-  if (trace_path) {
-    if (!trace_dev) cudaMalloc(&trace_dev, TRACE_TILES * 8 * sizeof(long long));
-    cudaMemsetAsync(trace_dev, 0, TRACE_TILES * 8 * sizeof(long long), stream);
-    p.trace = trace_dev;
-  }
   const int tile_m = BLOCK_M * CTAS;
   const int tiles = ((a.M + tile_m - 1) / tile_m) * (a.N / BN);
-  const int units = num_sms / CTAS;                       // CTAs or CTA pairs that fit the chip
+  const int units = num_sms / CTAS;                       // CTA pairs that fit the chip
   const int grid = (tiles < units ? tiles : units) * CTAS;
   {
     cudaError_t e = launch_pdl(kern, dim3(grid), dim3(Cfg::NUM_THREADS), Cfg::SMEM_BYTES, stream, 1, tmA, tmB, tmOut, tmOut2,
                                tmA2, tmB2, p);
     if (e != cudaSuccess) return e;
   }
-  if (trace_path) {   // debug only: synchronous dump of CTA 0's role timeline (cycles relative to its first stamp)
-    std::vector<long long> h(TRACE_TILES * 8);
-    cudaStreamSynchronize(stream);
-    cudaMemcpy(h.data(), trace_dev, h.size() * sizeof(long long), cudaMemcpyDeviceToHost);
-    if (FILE* f = fopen(trace_path, "a")) {
-      fprintf(f, "# gemm M=%d N=%d K=%d epi=%d: it mma_start mma_commit epi_full epi_release epi_done prod_first prod_last\n", a.M, a.N, a.K, EPI);
-      long long t0 = 0;
-      for (size_t i = 0; i < h.size(); ++i) if (h[i] && (!t0 || h[i] < t0)) t0 = h[i];
-      for (int i = 0; i < TRACE_TILES; ++i) {
-        if (!h[i * 8]) break;
-        fprintf(f, "%d", i);
-        for (int s = 0; s < 7; ++s) fprintf(f, " %lld", h[i * 8 + s] ? h[i * 8 + s] - t0 : -1);
-        fprintf(f, "\n");
-      }
-      fclose(f);
-    }
-  }
   return cudaGetLastError();
 }
 
-template <int BN, int CTAS>
+template <int BN>
 cudaError_t launch_bn(const GemmArgs& a, int* st, int sms, cudaStream_t s) {
 #define JCB_CASE16(E) \
-  case E: return a.f16 ? launch_cfg<BN, E, CTAS, true>(a, st, sms, s) : launch_cfg<BN, E, CTAS, false>(a, st, sms, s)
+  case E: return a.f16 ? launch_cfg<BN, E, true>(a, st, sms, s) : launch_cfg<BN, E, false>(a, st, sms, s)
   switch (a.epilogue) {
     JCB_CASE16(EPI_BIAS_BF16);
     JCB_CASE16(EPI_BIAS_GELU_BF16);
@@ -742,8 +650,8 @@ cudaError_t launch_bn(const GemmArgs& a, int* st, int sms, cudaStream_t s) {
     JCB_CASE16(EPI_LNFOLD_GELU_BF16);
     JCB_CASE16(EPI_RESID_LNPREP_SHORT);
     JCB_CASE16(EPI_RESID_LNPREP_LONG);
-    case EPI_BIAS_RESID_F32: return launch_cfg<BN, EPI_BIAS_RESID_F32, CTAS, false>(a, st, sms, s);
-    case EPI_F32: return launch_cfg<BN, EPI_F32, CTAS, false>(a, st, sms, s);
+    case EPI_BIAS_RESID_F32: return launch_cfg<BN, EPI_BIAS_RESID_F32, false>(a, st, sms, s);
+    case EPI_F32: return launch_cfg<BN, EPI_F32, false>(a, st, sms, s);
     default: return cudaErrorInvalidValue;
   }
 #undef JCB_CASE16
@@ -770,8 +678,6 @@ const char* gemm_init_driver_api() {
     return g_driver_err;
   }
   g_encode_tiled = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(fn);
-  const char* env = getenv("JCB_GEMM_CTAS");
-  g_ctas = (env && env[0] == '1') ? 1 : 2;
   return nullptr;
 }
 
@@ -786,12 +692,8 @@ cudaError_t launch_gemm(const GemmArgs& a, int* dev_status, int num_sms, cudaStr
                    (a.lda2 % 8) || (a.ldb2 % 8) || a.lda2 < a.K2 || a.ldb2 < a.K2))
     return cudaErrorInvalidValue;
   // BN = 256 whenever N allows it; 128 otherwise (only used by generic/test shapes).
-  if (g_ctas == 2) {
-    if (a.N % 256 == 0) return launch_bn<256, 2>(a, dev_status, num_sms, stream);
-    return launch_bn<128, 2>(a, dev_status, num_sms, stream);
-  }
-  if (a.N % 256 == 0) return launch_bn<256, 1>(a, dev_status, num_sms, stream);
-  return launch_bn<128, 1>(a, dev_status, num_sms, stream);
+  if (a.N % 256 == 0) return launch_bn<256>(a, dev_status, num_sms, stream);
+  return launch_bn<128>(a, dev_status, num_sms, stream);
 }
 
 }  // namespace jcb

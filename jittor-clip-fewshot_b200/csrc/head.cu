@@ -87,7 +87,6 @@ __global__ void __launch_bounds__(HEAD_THREADS) head_kernel(const HeadArgs a) {
   cg::cluster_group cluster = cg::this_cluster();
   const int crank = static_cast<int>(cluster.block_rank()), csize = static_cast<int>(cluster.num_blocks());
   griddep_wait();               // programmatic dependent launch (ptx.cuh): nothing global is touched above
-  griddep_launch_dependents();
   const int C = a.C, D = a.D;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const long long img = blockIdx.x / csize;

@@ -99,11 +99,10 @@ cudaError_t launch_text_embed_ln(const long long* ids, int64_t n_seq, int T, int
                                  int* eot, cudaStream_t stream, float* stats = nullptr, int stats_slots = 0,
                                  float* shift = nullptr, int f16 = 0);
 // qkv [B*T, 3W] bf16 (q | k | v, heads = 64-wide column blocks) -> out [B*T, W] bf16
-// causal != 0: key j is visible to query i only if j <= i (text tower); T <= 80
-// dev_status + num_sms given: the tcgen05 / TMEM kernel (attention_tc.cu) runs when the shape allows it (no mask,
-// T <= 64, even head count; JCB_ATT_IMPL=mma forces the mma.sync kernel); otherwise the mma.sync kernel (attention.cu)
+// causal != 0: key j is visible to query i only if j <= i (text tower); T <= 128.  Runs the tcgen05 / TMEM kernel
+// (attention_tc.cu): two heads per work item without a mask at T <= 64 and an even head count, one head otherwise
 cudaError_t launch_attention(const __nv_bfloat16* qkv, int64_t n_views, int T, int heads, __nv_bfloat16* out,
-                             cudaStream_t stream, int causal = 0, int* dev_status = nullptr, int num_sms = 0, int f16 = 0);
+                             cudaStream_t stream, int causal, int* dev_status, int num_sms, int f16 = 0);
 // query row 0 only (no mask, T <= 64): out [n_views, W] bf16, dense
 cudaError_t launch_attention_cls(const __nv_bfloat16* qkv, int64_t n_views, int T, int heads, __nv_bfloat16* out,
                                  cudaStream_t stream, int f16 = 0);
@@ -148,10 +147,10 @@ bool mta_shape_supported(int V, int C, int D);
 // bytes of global scratch launch_mta needs (0 when a problem fits in shared memory)
 size_t mta_scratch_bytes(int64_t n_problems, int V, int C, int D);
 // n_sets independent (feats, text) problems per image in one launch: grid = (I, n_sets)
-// dev_status + num_sms given: softmax(100 X T) runs as a bf16 x 3-limb GEMM on the tensor cores (launch_gemm) for
-// C <= 512; otherwise (or JCB_MTA_PROBS=simt) the fp32 SIMT kernel
+// softmax(100 X T) runs as a bf16 x 3-limb GEMM on the tensor cores (launch_gemm) for C <= 512 and D % 64 == 0;
+// otherwise the fp32 SIMT kernel
 cudaError_t launch_mta(const MtaSet* sets, int n_sets, int64_t I, int V, int C, int D, const MtaParams& p,
-                       float* scratch, cudaStream_t stream, int* dev_status = nullptr, int num_sms = 0,
+                       float* scratch, cudaStream_t stream, int* dev_status, int num_sms,
                        const MtaDebug* debug = nullptr);
 
 enum HeadScore : int { SCORE_LOGITS = 0, SCORE_CS = 1, SCORE_CS1 = 2, SCORE_CS2 = 3, SCORE_CS3 = 4, SCORE_CS4 = 5, SCORE_CS5 = 6, SCORE_COUNT = 7 };

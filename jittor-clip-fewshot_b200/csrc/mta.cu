@@ -13,7 +13,6 @@
 //
 // X [V, D] unit rows (row 0 = un-augmented view), T given as [D, C] (the orientation the reference
 // passes: `text_features.t()`), so class-parallel threads read it coalesced.
-#include <cstdlib>
 
 #include "kernels.h"
 #include "ptx.cuh"
@@ -245,7 +244,6 @@ __device__ __forceinline__ void split3(float x, uint16_t (&l)[3]) {
 __global__ void __launch_bounds__(256) mta_split_x_kernel(const float* __restrict__ X, long long rows, int D,
                                                           uint16_t* __restrict__ out) {
   griddep_wait();               // programmatic dependent launch (ptx.cuh): nothing global is touched above
-  griddep_launch_dependents();
   const long long i = static_cast<long long>(blockIdx.x) * 256 + threadIdx.x;
   if (i >= rows * D) return;
   const long long r = i / D;
@@ -259,7 +257,6 @@ __global__ void __launch_bounds__(256) mta_split_x_kernel(const float* __restric
 __global__ void __launch_bounds__(256) mta_split_t_kernel(const float* __restrict__ Tt, int C, int CP, int D,
                                                           uint16_t* __restrict__ out) {
   griddep_wait();               // programmatic dependent launch (ptx.cuh): nothing global is touched above
-  griddep_launch_dependents();
   const int i = blockIdx.x * 256 + threadIdx.x;
   if (i >= CP * D) return;
   const int d = i / CP, c = i - d * CP;          // threads along c: coalesced reads of Tt
@@ -272,7 +269,6 @@ __global__ void __launch_bounds__(256) mta_split_t_kernel(const float* __restric
 __global__ void __launch_bounds__(256) mta_softmax_rows_kernel(const float* __restrict__ L, long long rows, int C, int CP,
                                                                float scale, float* __restrict__ P) {
   griddep_wait();               // programmatic dependent launch (ptx.cuh): nothing global is touched above
-  griddep_launch_dependents();
   const int lane = threadIdx.x & 31;
   const long long r = static_cast<long long>(blockIdx.x) * 8 + (threadIdx.x >> 5);
   if (r >= rows) return;
@@ -981,7 +977,6 @@ __global__ void __launch_bounds__(NT, NT == 512 ? 1 : (NT == 128 ? 4 : (NT == 64
   constexpr int NW = NT / 32;
   extern __shared__ __align__(16) float mta_smem[];
   griddep_wait();               // programmatic dependent launch (ptx.cuh): nothing global is touched above
-  griddep_launch_dependents();
   const int V = a.V, C = a.C, D = a.D, ldA = a.ldA, ldx = a.ldx, ldp = a.ldp;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const long long img = blockIdx.x;
@@ -1089,14 +1084,6 @@ static bool mta_fits_smem(int V, int C, int D) {
 }
 
 static bool mta_use_probs_kernel(int C, int D) { return C <= PB_CPAD && D % PB_KC == 0; }
-static bool mta_fast_enabled() {   // JCB_MTA_FAST=0 keeps the first (256-thread, per-pair dot) kernel for A/B runs
-  static int v = -1;
-  if (v < 0) {
-    const char* env = getenv("JCB_MTA_FAST");
-    v = (env && env[0] == '0') ? 0 : 1;
-  }
-  return v != 0;
-}
 
 // floats per problem of the large-V path: affinity [V, ldA] + Gram of X [V, ldA] + bandwidths [V]
 static long long big_pre_elems(int V, int ldA) {
@@ -1104,7 +1091,7 @@ static long long big_pre_elems(int V, int ldA) {
   return 2 * m + ((V + 3) & ~3);
 }
 static bool mta_fast_fits(int V, int C, int D) {
-  return mta_use_probs_kernel(C, D) && D % 128 == 0 && mf_smem_bytes(V, C, D) <= MTA_SMEM_LIMIT && mta_fast_enabled();
+  return mta_use_probs_kernel(C, D) && D % 128 == 0 && mf_smem_bytes(V, C, D) <= MTA_SMEM_LIMIT;
 }
 
 // bytes of the tensor-core probabilities path for `rows` view rows per bank and `n_sets` banks: A' limbs (one copy per
@@ -1157,12 +1144,9 @@ cudaError_t launch_mta(const MtaSet* sets, int n_sets, int64_t I, int V, int C, 
     if (scratch == nullptr) return cudaErrorInvalidValue;
     const size_t p_bytes = (static_cast<size_t>(n_sets) * I * V * C * sizeof(float) + 255) / 256 * 256;
     const long long rows = static_cast<long long>(I) * V;
-    static int tc_env = -1;   // A/B: JCB_MTA_PROBS=simt keeps the fp32 SIMT kernel
-    if (tc_env < 0) { const char* e = getenv("JCB_MTA_PROBS"); tc_env = (e && e[0] == 's') ? 0 : 1; }
     // taken at EVERY batch size: a row's probabilities must not depend on how many other rows share the launch (the
     // path's pass-size and batch-split invariance is bit-exact); at one image the three extra launches per bank cost ~40 us
-    const bool tc = tc_env && dev_status != nullptr && num_sms > 0 && mta_tc_probs_possible(C, D);
-    if (tc) {
+    if (mta_tc_probs_possible(C, D)) {
       auto up = [](size_t x) { return (x + 255) / 256 * 256; };
       uint8_t* w = reinterpret_cast<uint8_t*>(scratch) + p_bytes;     // behind P; sized by mta_scratch_bytes
       const size_t a_b = up(static_cast<size_t>(rows) * 6 * D * 2), b_b = up(static_cast<size_t>(TCP_CP) * 6 * D * 2);
@@ -1219,7 +1203,7 @@ cudaError_t launch_mta(const MtaSet* sets, int n_sets, int64_t I, int V, int C, 
     scratch = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(scratch) + p_bytes +
                                        (mta_tc_probs_possible(C, D) ? tcp_bytes(static_cast<size_t>(n_sets), static_cast<size_t>(rows), D) : 0));
   }
-  if (a.P != nullptr && D % 128 == 0 && mf_smem_bytes(V, C, D) <= MTA_SMEM_LIMIT && mta_fast_enabled()) {
+  if (mta_fast_fits(V, C, D)) {
     a.ldx = mf_pad(D);
     a.ldp = mf_pad(C);
     a.in_smem = 1;
@@ -1238,15 +1222,7 @@ cudaError_t launch_mta(const MtaSet* sets, int n_sets, int64_t I, int V, int C, 
     // Sharing pays when there are more problems than SMs (a wave of one-bank CTAs would not fit anyway); with a handful
     // of images (the reference's one-image-per-call loop) three CTAs in parallel beat one CTA doing three solves in a
     // row.  Either way a bank's arithmetic is the same instruction sequence: the results are bit-identical.
-    int sms = num_sms;
-    if (sms <= 0) {
-      int dev = 0;
-      cudaGetDevice(&dev);
-      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    }
-    static int group_env = -1;   // A/B: JCB_MTA_GROUP=0 keeps one bank per CTA
-    if (group_env < 0) { const char* e = getenv("JCB_MTA_GROUP"); group_env = (e && e[0] == '0') ? 0 : 1; }
-    if (mf_smem_bytes(V, C, D, a.max_group) > MTA_SMEM_LIMIT || I * n_sets <= sms || !group_env) {   // (or no room for several affinities: V > 65)
+    if (mf_smem_bytes(V, C, D, a.max_group) > MTA_SMEM_LIMIT || I * n_sets <= num_sms) {   // (or no room for several affinities: V > 65)
       a.n_groups = n_sets;
       a.max_group = 1;
       for (int s2 = 0; s2 < n_sets; ++s2) { a.group_count[s2] = 1; a.group_sets[s2][0] = s2; }
@@ -1254,9 +1230,8 @@ cudaError_t launch_mta(const MtaSet* sets, int n_sets, int64_t I, int V, int C, 
     dim3 fgrid(static_cast<unsigned>(I), static_cast<unsigned>(a.n_groups));
     const size_t fsmem = mf_smem_bytes(V, C, D, a.max_group);
     if (V <= 32) {
-      static int nt_env = -1;     // A/B: JCB_MTA_NT = 32 | 64 | 128 forces the small-V thread count
-      if (nt_env < 0) { const char* e = getenv("JCB_MTA_NT"); nt_env = e ? atoi(e) : 0; }
-      const int nt = nt_env ? nt_env : (V <= 4 ? 32 : (V <= 12 ? 64 : 128));
+      // threads per CTA by view count, as measured at N = 1 and N = 16 crops (profiles/r02q_mta_small_v_thread_count.log)
+      const int nt = V <= 4 ? 32 : (V <= 12 ? 64 : 128);
       cudaError_t e = cudaSuccess;
       if (nt == 32) {
         if ((e = ensure_dynamic_smem(mta_fast_kernel<32>, fsmem)) != cudaSuccess) return e;

@@ -1,5 +1,5 @@
 // Thin inline-PTX wrappers for sm_100a: mbarrier, TMA (cp.async.bulk.tensor), tcgen05 (MMA / TMEM),
-// ldmatrix / mma.sync (attention), cp.async.  No CUTLASS/CuTe dependency: every encoding used here
+// cp.async.  No CUTLASS/CuTe dependency: every encoding used here
 // is written out so the SASS can be checked (UTCHMMA / UTMALDG / LDTM).
 #pragma once
 #include <cstdint>
@@ -302,17 +302,13 @@ __device__ __forceinline__ float ex2_approx(float x) {
 // initialisation, TMEM allocation, tensor-map prefetch, the cluster's first synchronisation -- overlaps that kernel's
 // tail, and the launch latency itself disappears from the chain (~70 dependent kernels per pipeline call).
 // griddep_wait() returns once ALL prerequisite grids have completed and their memory is visible; nothing that another
-// kernel wrote may be read, and nothing it may still read may be written, before it.  Both are no-ops in a kernel
-// launched without the attribute / without a dependent.  The attribute is opt-in (JCB_PDL=1, api.cu pdl_enabled).
+// kernel wrote may be read, and nothing it may still read may be written, before it.  It is a no-op in a kernel launched
+// without the attribute.  The attribute is opt-in (JCB_PDL=1, api.cu pdl_enabled).
 __device__ __forceinline__ void griddep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-// The explicit early trigger is compiled in only with -DJCB_PDL_EARLY_TRIGGER: with it, two full-size pipeline calls adjacent
-// in a stream hang (tools/pdl_first_calls_probe.py, profiles/r02_pdl_hang_probes.log); without it the dependents are released
-// by the exit of the primary's CTAs -- the same probe finishes (0.55 s) -- and still overlap their prologue with its last wave.
-__device__ __forceinline__ void griddep_launch_dependents() {
-#ifdef JCB_PDL_EARLY_TRIGGER
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
-}
+// No kernel issues griddepcontrol.launch_dependents: with that early trigger right after the wait, two full-size pipeline
+// calls adjacent in a stream hang (tools/pdl_first_calls_probe.py, profiles/r02_pdl_hang_probes.log).  The dependents are
+// released by the exit of the primary's CTAs instead -- the same probe finishes (0.55 s) -- and still overlap their
+// prologue with its last wave.
 
 __device__ __forceinline__ void named_bar_sync(int id, int threads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(threads) : "memory");
@@ -339,9 +335,6 @@ __device__ __forceinline__ void cluster_sync_all() {
 // tcgen05.fence::before_thread_sync, not by the memory model.
 __device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
   asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_cluster_release(uint32_t cluster_addr) {   // A/B only (JCB_GEMM_ARRIVE_RELEASE=1)
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
 }
 // 2-D tiled load issued by either CTA of a pair into ITS OWN shared memory; the bytes are reported
 // on the LEADER CTA's mbarrier (which the single MMA-issuing thread waits on).
@@ -386,37 +379,9 @@ __device__ __forceinline__ void umma_bf16_pair(uint32_t tmem_d, uint64_t desc_a,
       : "memory");
 }
 
-// ---------------------------------------------------------------- legacy warp MMA (attention only)
-__device__ __forceinline__ void ldmatrix_x4(uint32_t (&r)[4], uint32_t saddr) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0, %1, %2, %3}, [%4];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
-               : "r"(saddr));
-}
-__device__ __forceinline__ void ldmatrix_x4_trans(uint32_t (&r)[4], uint32_t saddr) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0, %1, %2, %3}, [%4];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
-               : "r"(saddr));
-}
-// D(16x8,f32) += A(16x16,bf16,row) * B(16x8,bf16,col)
-__device__ __forceinline__ void mma_bf16_16816(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm volatile(
-      "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, "
-      "{%0, %1, %2, %3};"
-      : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ void mma_f16_16816(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm volatile(
-      "mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, "
-      "{%0, %1, %2, %3};"
-      : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
+// ---------------------------------------------------------------- cp.async (MTA probabilities)
 __device__ __forceinline__ void cp_async_16(uint32_t saddr, const void* gptr) {
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(saddr), "l"(gptr) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit_wait_all() {
-  asm volatile("cp.async.commit_group;\n\tcp.async.wait_group 0;" ::: "memory");
 }
 
 __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {

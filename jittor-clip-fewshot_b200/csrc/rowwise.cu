@@ -40,7 +40,6 @@ __global__ void __launch_bounds__(384)
 im2col_kernel(const void* __restrict__ images, unsigned n_patches, int R, int P, int G, int apply_norm,
               __nv_bfloat16* __restrict__ patches) {
   griddep_wait();               // programmatic dependent launch (ptx.cuh): nothing global is touched above
-  griddep_launch_dependents();
   constexpr int EPT = 8;   // 8 pixels per thread for every input type: one fully coalesced 16-byte store per lane
   const int K = 3 * P * P;
   const int col = static_cast<int>(threadIdx.x) * EPT;  // (c, i, j) with j % EPT == 0
@@ -216,7 +215,6 @@ embed_ln_kernel(float* __restrict__ tokens, long long rows, int T, const float* 
                 float* __restrict__ stats, int stats_slots, const float* __restrict__ patch_out,
                 float* __restrict__ shift) {
   griddep_wait();               // programmatic dependent launch (ptx.cuh): nothing global is touched above
-  griddep_launch_dependents();
   constexpr int W = NV * 128;
   const int lane = threadIdx.x & 31;
   const long long row = static_cast<long long>(blockIdx.x) * LN_WARPS + (threadIdx.x >> 5);
@@ -346,7 +344,6 @@ tail_kernel(const float* __restrict__ tokens, long long n_views, int T, const fl
   float (*s_in)[TAIL_VIEWS][64] = reinterpret_cast<float (*)[TAIL_VIEWS][64]>(tail_smem + TAIL_VIEWS * W + TAIL_SPLIT * TAIL_VIEWS);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   griddep_wait();               // programmatic dependent launch (ptx.cuh): nothing global is touched above
-  griddep_launch_dependents();
   const int crank = CLUSTER ? static_cast<int>(cg::this_cluster().block_rank()) : 0;
   const long long v0 = static_cast<long long>(CLUSTER ? blockIdx.x / TAIL_SPLIT : blockIdx.x) * TAIL_VIEWS;
   for (int vv = warp; vv < TAIL_VIEWS; vv += TAIL_THREADS / 32) {  // ln_post on the CLS row of view v0 + vv  (jclip/model.py:121)

@@ -1,5 +1,5 @@
 """Oracle with operand rounding: the fp32 tower of oracle/vit.py with the GEMM operands rounded to bf16 or
-fp16 at exactly the points where the CUDA schedule rounds them (JCB_LN_FOLD=2).  TEST INFRASTRUCTURE ONLY.
+fp16 at exactly the points where the CUDA schedule rounds them (the folded schedule).  TEST INFRASTRUCTURE ONLY.
 
 Purpose: attribute the end-to-end logit deviation of the tensor-core path (VERDICT r01 "what's weak" 1) without
 GPU time.  Accumulation stays fp32 (as in TMEM); only what the kernels store as 16-bit operands is rounded:
@@ -36,7 +36,7 @@ def vit_encode_image_rounded(sd, images, lora=None, scaling=0.5, apply_clip_norm
     ln1_copy, qkv_w, qkv, p, attn, out_w, ln2_copy, fc_w, hidden, proj_w (per-class attribution of the deviation).
     layer_kind: optional callable block index -> operand type of EVERY 16-bit tensor of that block (overrides act / wgt /
     kinds inside the blocks; per-layer attribution).
-    fold: LayerNorm folded into the consuming GEMM (JCB_LN_FOLD=2) instead of a rounded stand-alone LayerNorm.
+    fold: LayerNorm folded into the consuming GEMM (the folded schedule) instead of a rounded stand-alone LayerNorm.
     centre: the 16-bit copy of the residual row is x - shift, shift = the row's mean at the previous LayerNorm point
     (what the EPI_RESID_LNPREP_* epilogues write since round 2); False = the round-1 raw copy.
     lora_mode: "merged" (W + s B A in fp32, then rounded: api.cu Packer) or "applied" (jcb_ctx_set_lora_mode: base weights

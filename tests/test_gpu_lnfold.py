@@ -1,10 +1,10 @@
-"""GPU: the three LayerNorm schedules of the tower (JCB_LN_FOLD = 0 stand-alone LayerNorm passes, 1 = ln_1 folded
-into c_proj's epilogue + the QKV GEMM, 2 = ln_2 folded as well (default)) all meet the embedding tolerance against
-the fp32 oracle -- for both operand types, on random-init weights AND on weights that give the residual stream the
-statistics of trained CLIP towers (synth.make_vit_state_dict(trained_like=...): row mean 20 x the spread, outlier
-channels 100 x the rest), where a fold that rounds the RAW residual copy loses the tolerance (oracle/quantized.py:
-cosine 0.99976 for bf16) and the centred copy does not.  The mode is read when the context is created, hence one
-subprocess per mode.  Reference: jclip/model.py:17-21, :59-62."""
+"""GPU: both LayerNorm schedules of the tower -- ln_1 and ln_2 folded into the GEMMs (towers packed with merged LoRA,
+the default) and the stand-alone LayerNorm passes (towers packed with LoRA applied as low-rank GEMMs) -- meet the
+embedding tolerance against the fp32 oracle -- for both operand types, on random-init weights AND on weights that give
+the residual stream the statistics of trained CLIP towers (synth.make_vit_state_dict(trained_like=...): row mean 20 x
+the spread, outlier channels 100 x the rest), where a fold that rounds the RAW residual copy loses the tolerance
+(oracle/quantized.py: cosine 0.99976 for bf16) and the centred copy does not.  The LoRA mode is read when the context
+is created (JCB_LORA), hence one subprocess per mode.  Reference: jclip/model.py:17-21, :59-62."""
 import os
 import subprocess
 import sys
@@ -54,9 +54,9 @@ for trained_like in (False, "offset", "outliers", "both"):
 ''' % ROOT
 
 
-@pytest.mark.parametrize("mode", ["0", "1", "2"])
-def test_layernorm_schedules(mode, cuda_dev):
-    env = dict(os.environ, JCB_LN_FOLD=mode)
+@pytest.mark.parametrize("lora", ["merged", "applied"])
+def test_layernorm_schedules(lora, cuda_dev):
+    env = dict(os.environ, JCB_LORA=lora)
     r = subprocess.run([sys.executable, "-c", SNIPPET], env=env, capture_output=True, text=True, timeout=900)
     print(r.stdout[-3000:])
     assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]

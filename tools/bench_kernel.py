@@ -40,7 +40,7 @@ if what == "attention":
     out = torch.empty(n * T, 768, dtype=OP, device=dev)
     ms = timeit(lambda: jb.blocks.attention(qkv, n, T, H, out, sync=False))
     gb = n * T * 768 * 8 / 1e9
-    print(f"attention cfg={os.environ.get('JCB_ATT_CFG', 'default')} n={n}: {ms:.3f} ms  {gb / ms * 1e3:.0f} GB/s")
+    print(f"attention n={n}: {ms:.3f} ms  {gb / ms * 1e3:.0f} GB/s")
 elif what == "layernorm":
     x = torch.randn(n * 50, 768, device=dev)
     g, b = torch.ones(768, device=dev), torch.zeros(768, device=dev)

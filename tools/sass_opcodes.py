@@ -5,7 +5,7 @@
 
 UTCHMMA = tcgen05.mma (.2CTA = cta_group::2), LDTM / STTM = tcgen05.ld / st (TMEM), UTMALDG / UTMASTG / UTMAREDG = TMA
 tensor load / store / reduce-add (cp.async.bulk.tensor, cp.reduce.async.bulk.tensor), UTCBAR = tcgen05.commit,
-HMMA = legacy mma.sync (the A/B baseline attention kernel only), SYNCS = mbarrier operations, ACQBULK / PREEXIT =
+HMMA = legacy mma.sync, SYNCS = mbarrier operations, ACQBULK / PREEXIT =
 griddepcontrol.wait / launch_dependents (programmatic dependent launch), UCGABAR = barrier.cluster (thread-block clusters).
 """
 import collections
