@@ -77,7 +77,9 @@ int jcb_ctx_set_stream(jcb_ctx* ctx, void* cuda_stream);
 /* Upper bound on the views processed per pass through the tower (workspace = ~1.2 MB per view); a batch
  * is split into the fewest equal passes that respect it.  Default 16384 for device-resident input
  * (measured on B200: larger passes are faster, intermediates never fit L2 anyway) and min(2048, bound)
- * for host input, so that the copy of pass i+1 overlaps the compute of pass i. */
+ * for host input, so that the copy of pass i+1 overlaps the compute of pass i.  Both bounds count views of a tower
+ * of up to 64 tokens (ViT-B/32: 50); a tower of T > 64 tokens runs min(bound, bound * 64 / T) views per pass, about
+ * the same number of token rows (ViT-B/16, 197 tokens: 5322 views of the default 16384). */
 int jcb_ctx_set_chunk_views(jcb_ctx* ctx, int64_t chunk_views);
 int jcb_ctx_set_host_chunk_views(jcb_ctx* ctx, int64_t chunk_views);
 /* Opt-in schedule for the image tower (default off; env JCB_CLS_ONLY_LAST_BLOCK=1 sets the initial value): run the
@@ -85,7 +87,9 @@ int jcb_ctx_set_host_chunk_views(jcb_ctx* ctx, int64_t chunk_views);
  * ln_post(x[:, 0, :]) @ proj (jclip/model.py:121-124), so after that block's keys and values no other token row
  * reaches the result; the reference computes them anyway.  Embeddings agree with the full schedule to rounding
  * (different attention summation order for that one row).  Ignored by jcb_vit_debug_tokens consumers that read
- * other rows of the last block: with the option on, only row 0 of every view is defined there. */
+ * other rows of the last block: with the option on, only row 0 of every view is defined there.  Applies to towers
+ * of up to 64 tokens only (the class-token attention scores at most 64 keys); a longer tower such as ViT-B/16 runs
+ * the full last block with the option on or off. */
 int jcb_ctx_set_cls_only_last_block(jcb_ctx* ctx, int on);
 /* Element type of every 16-bit GEMM operand of the towers packed AFTER this call (weights, the residual copy the
  * LayerNorm-folded GEMMs read, q|k|v, softmax numerators, attention output, MLP hidden); accumulation is fp32 in
@@ -428,7 +432,8 @@ int jcb_layernorm(jcb_ctx* ctx, const float* x_dev, int64_t rows, int32_t width,
 int jcb_im2col(jcb_ctx* ctx, const void* images_dev, int32_t img_dtype, int64_t n_views, int32_t resolution,
                int32_t patch, int32_t apply_clip_norm, int32_t operand_type, void* patches16_dev);
 /* softmax(q k^T / 8 [+ causal mask]) v per (sequence, head) (jclip/mha.py:55-83; mask jclip/model.py:189-193):
- * qkv16_dev [n_views * tokens, 3 * 64 * heads] -> out16_dev [n_views * tokens, 64 * heads]; tokens <= 128 */
+ * qkv16_dev [n_views * tokens, 3 * 64 * heads] -> out16_dev [n_views * tokens, 64 * heads]; tokens <= 256 without the
+ * mask, tokens <= 128 with it (JCB_E_INVALID otherwise) */
 int jcb_attention(jcb_ctx* ctx, const void* qkv16_dev, int64_t n_views, int32_t tokens, int32_t heads, int32_t causal,
                   int32_t operand_type, void* out16_dev);
 /* hits / misses of the process-wide cache of encoded TMA tensor maps (one entry per (pointer, shape) launched) */

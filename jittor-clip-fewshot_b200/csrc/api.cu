@@ -539,8 +539,13 @@ int tower_forward(jcb_vit* v, const void* images, int dt, int64_t n, int apply_n
 // Views per pass through the tower.  Host input of a blocking call is cut into small passes so that the upload of
 // pass i+1 hides behind the compute of pass i; a submission queued behind a running one (jcb_pipeline_submit) hides
 // its WHOLE upload behind that one's compute and keeps the large, more efficient passes of device-resident input.
-int64_t views_bound(const jcb_ctx* ctx, bool on_host) {
-  return (on_host && !ctx->overlapped) ? std::min(ctx->host_chunk_views, ctx->chunk_views) : ctx->chunk_views;
+// The bounds count views of a tower of up to 64 tokens; a longer tower gets proportionally fewer views per pass, so
+// that a pass holds about the same number of token rows (and workspace) whatever the patch size.
+int64_t token_rows_bound(int64_t bound, int T) { return std::max<int64_t>(1, std::min(bound, bound * 64 / T)); }
+
+int64_t views_bound(const jcb_ctx* ctx, bool on_host, int T) {
+  return token_rows_bound(
+      (on_host && !ctx->overlapped) ? std::min(ctx->host_chunk_views, ctx->chunk_views) : ctx->chunk_views, T);
 }
 
 int64_t balanced_chunk(int64_t n, int64_t bound) {
@@ -572,7 +577,7 @@ int encode_views(jcb_vit* v, const void* images, int dt, bool on_host, int64_t n
   if (!images || !out_dev) return fail(ctx, JCB_E_INVALID, "null image / output pointer");
   // balanced chunks: the fewest passes that respect the bound, all (nearly) the same size, so no pass
   // runs the 148 SMs on a sliver of work
-  const int64_t chunk = balanced_chunk(n, views_bound(ctx, on_host));
+  const int64_t chunk = balanced_chunk(n, views_bound(ctx, on_host, v->tokens));
   int rc = ws_reserve(ctx, ws_extra + tower_ws_bytes(v, chunk));
   if (rc) return rc;
   Bump b(static_cast<uint8_t*>(ctx->ws) + ws_extra);
@@ -878,9 +883,9 @@ int jcb_vit_create(jcb_ctx* ctx, const jcb_vit_config* cfg, jcb_vit** out) {
   v->L = cfg->layers;
   v->prefix = "visual.transformer.resblocks.";
   v->kpatch = 3 * cfg->patch * cfg->patch;
-  if (v->tokens > 64 || v->heads % 4 != 0 || v->kpatch % 64 != 0) {
+  if (v->tokens > 256 || v->heads % 4 != 0 || v->kpatch % 64 != 0) {
     delete v;
-    return fail(ctx, JCB_E_INVALID, "tokens=%d (max 64) / heads=%d (multiple of 4) unsupported", v->tokens, v->heads);
+    return fail(ctx, JCB_E_INVALID, "tokens=%d (max 256) / heads=%d (multiple of 4) unsupported", v->tokens, v->heads);
   }
   build_expected(v);
   *out = v;
@@ -1270,7 +1275,7 @@ int jcb_encode_image_host(jcb_vit* v, const void* images_host, int img_dtype, in
   if (n_views == 0) return JCB_OK;
   if (n_views < 0 || !out_host) return fail(ctx, JCB_E_INVALID, "bad arguments");
   const size_t out_bytes = align_up(static_cast<size_t>(n_views) * v->cfg.embed_dim * 4);
-  if ((rc = ws_reserve(ctx, out_bytes + tower_ws_bytes(v, balanced_chunk(n_views, std::min(ctx->host_chunk_views, ctx->chunk_views)))))) return rc;
+  if ((rc = ws_reserve(ctx, out_bytes + tower_ws_bytes(v, balanced_chunk(n_views, token_rows_bound(std::min(ctx->host_chunk_views, ctx->chunk_views), v->tokens)))))) return rc;
   float* out_dev = static_cast<float*>(ctx->ws);
   if ((rc = encode_views(v, images_host, img_dtype, true, n_views, apply_clip_norm, normalize, out_dev, out_bytes)))
     return rc;
@@ -1550,9 +1555,9 @@ int pipeline_enqueue(jcb_vit* vit, jcb_vit* vit_zs, const jcb_pipeline_args* a) 
   // (encode_views reserves again per tower; if the second tower needed MORE than the first, ws_reserve would free
   // the buffer the first tower's embeddings, the modes and the scratch were carved from.)
   {
-    const int64_t chunk = balanced_chunk(NV, views_bound(ctx, a->images_on_host != 0));
+    const int64_t chunk = balanced_chunk(NV, views_bound(ctx, a->images_on_host != 0, vit->tokens));
     size_t tower_b = tower_ws_bytes(vit, chunk);
-    if (vit_zs) tower_b = std::max(tower_b, tower_ws_bytes(vit_zs, chunk));
+    if (vit_zs) tower_b = std::max(tower_b, tower_ws_bytes(vit_zs, balanced_chunk(NV, views_bound(ctx, a->images_on_host != 0, vit_zs->tokens))));
     if ((rc = ws_reserve(ctx, head_bytes + tower_b))) return rc;
   }
   Bump b(ctx->ws);

@@ -1,7 +1,7 @@
 // Attention entry points: launch_attention (every full attention, on the tcgen05 / TMEM kernel of attention_tc.cu)
 // and the class-token-only kernel below.  The tcgen05 kernel replaced a round-1 mma.sync kernel (Q, K, V in smem) that
 // spent 2/3 of its time in the shared-memory pipe (profiles/r01f): 0.366 vs 0.568 ms per launch of 8320 views on a
-// B200 (DESIGN.md section 4).
+// B200 (DESIGN.md section 4).  T <= 128 with the causal mask, T <= 256 without.
 //
 // Reference: jclip/mha.py:55-83 scaled_dot_product_attention (attn_mask None for the vision tower,
 // jclip/model.py:99; dropout 0 in eval), head split jclip/mha.py:351-362 / test.py:584-590.
@@ -96,7 +96,7 @@ cudaError_t launch_attention_cls(const __nv_bfloat16* qkv, int64_t n_views, int 
 
 cudaError_t launch_attention(const __nv_bfloat16* qkv, int64_t n_views, int T, int heads, __nv_bfloat16* out,
                              cudaStream_t stream, int causal, int* dev_status, int num_sms, int f16) {
-  if (T < 1 || T > 128 || heads < 1) return cudaErrorInvalidValue;
+  if (T < 1 || T > 256 || (causal && T > 128) || heads < 1) return cudaErrorInvalidValue;
   if (n_views == 0) return cudaSuccess;
   return launch_attention_tc(qkv, n_views, T, heads, out, stream, dev_status, num_sms, f16, causal);
 }

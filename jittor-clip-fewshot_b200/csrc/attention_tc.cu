@@ -22,6 +22,21 @@
 // matrix, P is dense, and the softmax applies the causal mask of the text tower (key j visible to query i iff j <= i,
 // jclip/model.py:189-193 build_attention_mask) on the fly.  Same shared-memory / TMEM layout and MMA sequence.
 //
+// LONG FORM (attention_tcgen05_long_kernel, 129 <= T <= 256, no mask: the ViT-B/16 image tower, 197 / 201 tokens):
+// work item = (sequence, head, query tile qt in {0, 1}); the two query tiles of a head are adjacent items, so they run
+// on neighbouring CTAs at the same time and the second read of the head's K and V hits L2.  Q = two 64-token boxes at
+// tokens 128 qt + {0, 64}, K and V = the head's whole key range, ceil(T / 64) boxes each (boxes wholly beyond T are
+// neither loaded nor multiplied: the K / V box at token 192 for T <= 192, and Q box 1 of tile 1).
+//   S[128, 64 nkb] = Q K^T      (UMMA 128 x 64nkb x 16, x4; S fills up to 256 TMEM columns)
+//   softmax                      two passes over S in 32-column chunks (maximum, then exponentials), exact: the whole
+//                                row stays on chip, no online rescaling; P as 16-bit pairs over the score columns already
+//                                read (P column j <- scores 2j, 2j + 1; columns 0..127)
+//   O[128, 64] = P V            (UMMA 128x64x16, 4 nkb steps, A = P from TMEM, B = V MN-major) into score columns
+//                                128..191 (read before P was published), then O / rowsum -> 16 bits -> TMA store
+// Everything aliases into 256 TMEM columns, so two CTAs (one 80 KB Q | K | V stage + 16 KB output staging each) share
+// an SM; the next item's scores wait until the epilogue has read O (tmem_free barrier).  One CTA per SM with two
+// Q | K | V stages measured 1.076 against 0.874 ms for this form (T = 197, 12 heads, 2048 sequences; DESIGN.md section 4).
+//
 // The 16-bit element type (bf16 | fp16) of Q, K, V, P and the output is the template parameter F16.
 //
 // Reference: jclip/mha.py:55-83 scaled_dot_product_attention (attn_mask None for the vision tower,
@@ -303,6 +318,222 @@ attention_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid
   }
 }
 
+// ---------------------------------------------------------------------------------------------------- long form
+constexpr int LQ_BYTES = 2 * TILE;                 // 128 query rows
+constexpr int LKV_BYTES = 4 * TILE;                // up to 256 key rows, 256 contiguous 128-byte rows
+constexpr int LSTAGE_BYTES = LQ_BYTES + 2 * LKV_BYTES;   // Q | K | V: 80 KB
+constexpr int LOUT_BYTES = 2 * TILE;
+constexpr int ATL_SMEM = LSTAGE_BYTES + LOUT_BYTES + BAR_BYTES;   // 98432 B -> two CTAs per SM
+constexpr uint32_t L_S_COL = 0, L_P_COL = 0, L_O_COL = 128;
+
+struct AtlDev {
+  long long n_items;   // sequences * heads * 2
+  int heads;
+  int T;
+  int* status;
+};
+
+template <bool F16>
+__global__ void __launch_bounds__(ATC_THREADS, 2)
+attention_tcgen05_long_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant__ CUtensorMap tmOut,
+                              const AtlDev p) {
+  extern __shared__ __align__(1024) uint8_t atl_smem[];
+  uint8_t* sq = atl_smem;
+  uint8_t* ostage = atl_smem + LSTAGE_BYTES;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(ostage + LOUT_BYTES);
+  uint64_t* full_bar = bars;        // TMA -> MMA
+  uint64_t* empty_bar = bars + 1;   // MMA (P V done) -> TMA
+  uint64_t* s_full = bars + 2;      // scores in TMEM          MMA -> softmax
+  uint64_t* p_full = bars + 3;      // probabilities in TMEM   softmax (128 arrivals) -> MMA
+  uint64_t* o_full = bars + 4;      // outputs in TMEM         MMA -> epilogue
+  uint64_t* tmem_free = bars + 5;   // outputs read            epilogue (128 arrivals) -> MMA (next item's scores)
+  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 6);
+
+  const int warp_idx = __shfl_sync(0xffffffffu, static_cast<int>(threadIdx.x >> 5), 0);
+  const int lane = threadIdx.x & 31;
+  const int T = p.T;
+  const int nkb = (T + 63) >> 6;   // 64-key boxes that hold valid keys: 3 (T <= 192) or 4
+
+  if (threadIdx.x == 0) {
+    if ((smem_u32(atl_smem) & 1023u) != 0u) atomicCAS(p.status, 0, JCB_DEV_SMEM_ALIGN);
+    tma_prefetch_desc(&tmQKV);
+    tma_prefetch_desc(&tmOut);
+    mbar_init(full_bar, 1);
+    mbar_init(empty_bar, 1);
+    mbar_init(s_full, 1);
+    mbar_init(p_full, 128);
+    mbar_init(o_full, 1);
+    mbar_init(tmem_free, 128);
+    fence_mbar_init();
+    fence_proxy_async_smem();
+  }
+  if (warp_idx == 1) {
+    tmem_alloc(tmem_ptr_smem, TMEM_COLS);
+    tmem_relinquish();
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(tmem_ptr_smem);
+  griddep_wait();               // programmatic dependent launch (ptx.cuh): nothing global is touched above
+
+  if (warp_idx == 0) {
+    // ===================================================================== TMA producer
+    if (elect_one()) {
+      int it = 0;
+      for (long long item = blockIdx.x; item < p.n_items; item += gridDim.x, ++it) {
+        if (!mbar_wait(empty_bar, (static_cast<uint32_t>(it) & 1u) ^ 1u, p.status, JCB_DEV_TIMEOUT_PRODUCER)) break;
+        const int qt = static_cast<int>(item & 1);
+        const long long sh = item >> 1;
+        const int seq = static_cast<int>(sh / p.heads);
+        const int h = static_cast<int>(sh % p.heads);
+        const int nq = 128 * qt + 64 < T ? 2 : 1;
+        mbar_arrive_expect_tx(full_bar, static_cast<uint32_t>((nq + 2 * nkb) * TILE));
+        // coordinates: (d, 64-wide column block of the [T, 3W] row, token, sequence); blocks: q | k | v heads
+        for (int b = 0; b < nq; ++b)
+          tma_load_4d(sq + b * TILE, &tmQKV, full_bar, 0, h, 128 * qt + 64 * b, seq);
+        for (int b = 0; b < nkb; ++b) {
+          tma_load_4d(sq + LQ_BYTES + b * TILE, &tmQKV, full_bar, 0, p.heads + h, 64 * b, seq);
+          tma_load_4d(sq + LQ_BYTES + LKV_BYTES + b * TILE, &tmQKV, full_bar, 0, 2 * p.heads + h, 64 * b, seq);
+        }
+      }
+    }
+  } else if (warp_idx == 1) {
+    // ===================================================================== MMA issuer
+    if (elect_one()) {
+      const uint32_t idesc_s = umma_idesc_f32acc(F16, 128, 64 * nkb);
+      constexpr uint32_t idesc_o = umma_idesc_f32acc(F16, 128, 64, /*b_mn_major=*/true);
+      const uint32_t sa = smem_u32(sq);
+      const uint64_t dq = umma_desc_sw128(sa);
+      const uint64_t dk = umma_desc_sw128(sa + LQ_BYTES);
+      const uint64_t dv = umma_desc_sw128_mn(sa + LQ_BYTES + LKV_BYTES);
+      int it = 0;
+      for (long long item = blockIdx.x; item < p.n_items; item += gridDim.x, ++it) {
+        const uint32_t iphase = static_cast<uint32_t>(it) & 1u;
+        if (!mbar_wait(full_bar, iphase, p.status, JCB_DEV_TIMEOUT_MMA)) break;
+        // S, P and O share the columns: the previous item's outputs must have been read out
+        if (it > 0 && !mbar_wait(tmem_free, iphase ^ 1u, p.status, JCB_DEV_TIMEOUT_MMA)) break;
+        tc_fence_after();
+#pragma unroll
+        for (int k = 0; k < HD / 16; ++k)
+          umma_bf16(tmem_base + L_S_COL, dq + static_cast<uint64_t>(2 * k), dk + static_cast<uint64_t>(2 * k), idesc_s,
+                    k != 0 ? 1u : 0u);
+        umma_commit(s_full);
+        if (!mbar_wait(p_full, iphase, p.status, JCB_DEV_TIMEOUT_MMA)) break;
+        tc_fence_after();
+        // keys in steps of 16: 8 TMEM columns of P, 16 rows (2048 B) of V per step; the V boxes are contiguous
+        for (int ks = 0; ks < 4 * nkb; ++ks)
+          umma_bf16_ts(tmem_base + L_O_COL, tmem_base + L_P_COL + static_cast<uint32_t>(8 * ks),
+                       dv + static_cast<uint64_t>(ks * (2048 >> 4)), idesc_o, ks != 0 ? 1u : 0u);
+        umma_commit(empty_bar);   // Q, K, V have been read
+        umma_commit(o_full);
+      }
+    }
+  } else {
+    // ===================================================================== softmax + epilogue (warps 2..5)
+    const int q = warp_idx & 3;              // TMEM lane quarter this warp may access
+    const int r = q * 32 + lane;             // query row within the tile
+    const bool leader = warp_idx == 2 && lane == 0;
+    const uint32_t lane_base = tmem_base + (static_cast<uint32_t>(q * 32) << 16);
+    const float scale_log2 = 0.125f * 1.4426950408889634f;  // 1/sqrt(64) * log2(e)
+    int it = 0;
+    bool ok = true;
+    for (long long item = blockIdx.x; item < p.n_items && ok; item += gridDim.x, ++it) {
+      const uint32_t iphase = static_cast<uint32_t>(it) & 1u;
+      ok = mbar_wait(s_full, iphase, p.status, JCB_DEV_TIMEOUT_EPILOGUE);
+      ok = __all_sync(0xffffffffu, ok);
+      if (!ok) break;
+      tc_fence_after();
+      // pass 1: row maximum over the keys < T, four independent chains.  Rows of tile 1 beyond T hold stale or zero
+      // queries; their results are clipped on store.
+      float m4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
+      for (int ch = 0; ch < 2 * nkb; ++ch) {
+        uint32_t sv[32];
+        tmem_ld_32x32b_x32(lane_base + L_S_COL + static_cast<uint32_t>(ch * 32), sv);
+        tmem_ld_wait();
+        if (ch * 32 + 32 <= T) {
+#pragma unroll
+          for (int c = 0; c < 32; ++c) m4[c & 3] = fmaxf(m4[c & 3], __uint_as_float(sv[c]));
+        } else {
+#pragma unroll
+          for (int c = 0; c < 32; ++c)
+            if (ch * 32 + c < T) m4[c & 3] = fmaxf(m4[c & 3], __uint_as_float(sv[c]));
+        }
+      }
+      const float nmx = -fmaxf(fmaxf(m4[0], m4[1]), fmaxf(m4[2], m4[3])) * scale_log2;
+      // pass 2: exponentials per 64-key box; P for keys 64 hf .. 64 hf + 63 goes to columns 32 hf .. 32 hf + 31,
+      // whose scores were read in this or the previous box
+      float s4[4] = {0.f, 0.f, 0.f, 0.f};
+      for (int hf = 0; hf < nkb; ++hf) {
+        uint32_t pv[32];
+#pragma unroll
+        for (int ch = 0; ch < 2; ++ch) {
+          uint32_t sv[32];
+          tmem_ld_32x32b_x32(lane_base + L_S_COL + static_cast<uint32_t>(hf * 64 + ch * 32), sv);
+          tmem_ld_wait();
+#pragma unroll
+          for (int c = 0; c < 16; ++c) {
+            const int k0 = hf * 64 + ch * 32 + 2 * c;
+            const float p0 = k0 < T ? ex2_approx(fmaf(__uint_as_float(sv[2 * c]), scale_log2, nmx)) : 0.f;
+            const float p1 = k0 + 1 < T ? ex2_approx(fmaf(__uint_as_float(sv[2 * c + 1]), scale_log2, nmx)) : 0.f;
+            s4[c & 3] += p0 + p1;
+            pv[ch * 16 + c] = pack_h2<F16>(p0, p1);
+          }
+        }
+        tmem_st_32x32b_x32(lane_base + L_P_COL + static_cast<uint32_t>(hf * 32), pv);
+      }
+      const float sum = (s4[0] + s4[1]) + (s4[2] + s4[3]);
+      tmem_st_wait();
+      tc_fence_before();
+      mbar_arrive(p_full);
+      const float inv = 1.0f / sum;
+
+      ok = mbar_wait(o_full, iphase, p.status, JCB_DEV_TIMEOUT_EPILOGUE);
+      ok = __all_sync(0xffffffffu, ok);
+      if (!ok) break;
+      tc_fence_after();
+      uint32_t ov[64];
+      tmem_ld_32x32b_x32(lane_base + L_O_COL, *reinterpret_cast<uint32_t(*)[32]>(&ov[0]));
+      tmem_ld_32x32b_x32(lane_base + L_O_COL + 32, *reinterpret_cast<uint32_t(*)[32]>(&ov[32]));
+      tmem_ld_wait();
+      tc_fence_before();   // this row's TMEM reads are complete: the next item's scores may overwrite the columns
+      mbar_arrive(tmem_free);
+      // the previous item's store must have finished reading the staging tile before it is overwritten
+      if (leader) bulk_wait_read<0>();
+      named_bar_sync(1, 128);
+      uint8_t* rowp = ostage + (r >> 6) * TILE + (r & 63) * 128;
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {  // 16-byte piece j of this row, XOR-swizzled by row % 8
+        uint4 o;
+        o.x = pack_h2<F16>(__uint_as_float(ov[8 * j + 0]) * inv, __uint_as_float(ov[8 * j + 1]) * inv);
+        o.y = pack_h2<F16>(__uint_as_float(ov[8 * j + 2]) * inv, __uint_as_float(ov[8 * j + 3]) * inv);
+        o.z = pack_h2<F16>(__uint_as_float(ov[8 * j + 4]) * inv, __uint_as_float(ov[8 * j + 5]) * inv);
+        o.w = pack_h2<F16>(__uint_as_float(ov[8 * j + 6]) * inv, __uint_as_float(ov[8 * j + 7]) * inv);
+        *reinterpret_cast<uint4*>(rowp + ((j ^ (r & 7)) << 4)) = o;
+      }
+      fence_proxy_async_smem();
+      named_bar_sync(1, 128);
+      if (leader) {
+        const int qt = static_cast<int>(item & 1);
+        const long long sh = item >> 1;
+        const int seq = static_cast<int>(sh / p.heads);
+        const int h = static_cast<int>(sh % p.heads);
+        tma_store_4d(&tmOut, ostage, 0, h, 128 * qt, seq);
+        if (128 * qt + 64 < T) tma_store_4d(&tmOut, ostage + TILE, 0, h, 128 * qt + 64, seq);
+        bulk_commit();
+      }
+    }
+    if (leader) bulk_wait<0>();
+  }
+
+  tc_fence_before();
+  __syncthreads();
+  if (warp_idx == 1) {
+    tc_fence_after();
+    tmem_dealloc(tmem_base, TMEM_COLS);
+  }
+}
+
 // [n_seq, T, blocks, 64] 16-bit elements as a 4-D tensor (d, block, token, sequence); boxes of 64 x 1 x 64 x 1 = one
 // head's [64 tokens][64] tile.  The token dimension is T long, so the rows T.. of a box are out of bounds: zero on
 // load, dropped on store.  Encoded once per (pointer, shape) and cached (same reason as gemm.cu's cache).
@@ -355,13 +586,25 @@ cudaError_t launch_atc(const CUtensorMap& tmQKV, const CUtensorMap& tmOut, const
   return launch_pdl(kernel, dim3(grid), dim3(ATC_THREADS), ATC_SMEM, stream, 1, tmQKV, tmOut, p);
 }
 
+cudaError_t launch_atl(const CUtensorMap& tmQKV, const CUtensorMap& tmOut, const AtlDev& p, int f16, int num_sms,
+                       cudaStream_t stream) {
+  auto kernel = f16 ? attention_tcgen05_long_kernel<true> : attention_tcgen05_long_kernel<false>;
+  cudaError_t e = ensure_dynamic_smem(kernel, ATL_SMEM);
+  if (e != cudaSuccess) return e;
+  const long long max_ctas = 2LL * num_sms;
+  const unsigned grid = static_cast<unsigned>(p.n_items < max_ctas ? p.n_items : max_ctas);
+  return launch_pdl(kernel, dim3(grid), dim3(ATC_THREADS), ATL_SMEM, stream, 1, tmQKV, tmOut, p);
+}
+
 }  // namespace
 
-// two heads per 128-row tile (T <= 64, no mask, even head count) or one head per tile (T <= 128, optional causal mask)
+// two heads per 128-row tile (T <= 64, no mask, even head count), one head per tile (T <= 128, optional causal mask)
+// or one head and one of two 128-row query tiles per item (129 <= T <= 256, no mask)
 bool attention_tc_supported(int T, int heads, int causal) {
   if (T < 1 || heads < 1) return false;
   if (!causal && T <= 64 && heads % 2 == 0) return true;
-  return T <= 128;
+  if (T <= 128) return true;
+  return !causal && T <= 256;
 }
 
 cudaError_t launch_attention_tc(const __nv_bfloat16* qkv, int64_t n_views, int T, int heads, __nv_bfloat16* out,
@@ -374,6 +617,14 @@ cudaError_t launch_attention_tc(const __nv_bfloat16* qkv, int64_t n_views, int T
     return cudaErrorInvalidValue;
   if (!make_tmap_heads(&tmOut, out, static_cast<uint64_t>(n_views), static_cast<uint64_t>(T), static_cast<uint64_t>(heads), f16))
     return cudaErrorInvalidValue;
+  if (T > 128) {
+    AtlDev p;
+    p.n_items = static_cast<long long>(n_views) * heads * 2;
+    p.heads = heads;
+    p.T = T;
+    p.status = dev_status;
+    return launch_atl(tmQKV, tmOut, p, f16, num_sms, stream);
+  }
   const bool paired = !causal && T <= 64 && heads % 2 == 0;
   AtcDev p;
   p.pairs = paired ? heads / 2 : heads;

@@ -99,8 +99,9 @@ cudaError_t launch_text_embed_ln(const long long* ids, int64_t n_seq, int T, int
                                  int* eot, cudaStream_t stream, float* stats = nullptr, int stats_slots = 0,
                                  float* shift = nullptr, int f16 = 0);
 // qkv [B*T, 3W] bf16 (q | k | v, heads = 64-wide column blocks) -> out [B*T, W] bf16
-// causal != 0: key j is visible to query i only if j <= i (text tower); T <= 128.  Runs the tcgen05 / TMEM kernel
-// (attention_tc.cu): two heads per work item without a mask at T <= 64 and an even head count, one head otherwise
+// causal != 0: key j is visible to query i only if j <= i (text tower); T <= 128 with the mask, T <= 256 without.
+// Runs the tcgen05 / TMEM kernels (attention_tc.cu): two heads per work item without a mask at T <= 64 and an even head
+// count, one head per item up to T = 128, one head and one 128-row query tile per item for 129 <= T <= 256
 cudaError_t launch_attention(const __nv_bfloat16* qkv, int64_t n_views, int T, int heads, __nv_bfloat16* out,
                              cudaStream_t stream, int causal, int* dev_status, int num_sms, int f16 = 0);
 // query row 0 only (no mask, T <= 64): out [n_views, W] bf16, dense

@@ -27,6 +27,8 @@ class Context:
         check(self.lib.jcb_ctx_create(self.device, byref(h)))
         self.handle = h
         self._stream = None
+        # the pass bounds last set through this object (the library's defaults until then, include/jclip_b200.h)
+        self.chunk_views, self.host_chunk_views = 16384, 2048
 
     def bind_current_stream(self):
         """Run the library's kernels on torch's current stream so they order with the caller's work."""
@@ -37,9 +39,11 @@ class Context:
 
     def set_chunk_views(self, n):
         check(self.lib.jcb_ctx_set_chunk_views(self.handle, int(n)), self.handle)
+        self.chunk_views = int(n)
 
     def set_host_chunk_views(self, n):
         check(self.lib.jcb_ctx_set_host_chunk_views(self.handle, int(n)), self.handle)
+        self.host_chunk_views = int(n)
 
     def set_cls_only_last_block(self, on):
         """Opt-in: last block of the image tower on the class-token rows only (include/jclip_b200.h)."""
