@@ -114,7 +114,8 @@ int jcb_ctx_get_operand_type(const jcb_ctx* ctx);
  *                    (likewise out_proj for 'o' adapters).  The ranks of q, k, v of one layer must sum to <= 64 (r <= 64
  *                    for 'o').  This schedule keeps the LayerNorms as stand-alone passes (the folded epilogues would
  *                    need the low-rank term pre-divided by the row's 1 / sigma), so it is the slower of the two; it
- *                    exists for callers that swap adapters per request.
+ *                    exists for callers that swap adapters per request.  It is also the mode that serves several
+ *                    adapter sets from one image tower, chosen per image (LoRA slots, jcb_vit_set_lora_slot).
  * A tower keeps the mode it was finalized with (jcb_vit_lora_mode / jcb_text_lora_mode). */
 #define JCB_LORA_MERGED 0
 #define JCB_LORA_APPLIED 1
@@ -178,6 +179,24 @@ int jcb_vit_set_param(jcb_vit* vit, const char* name, const float* data, int64_t
 /* Attach one LoRA adapter (reference LinearLoRA, test.py:340-398): A [r, width], B [width, r] host fp32,
  * scaling = alpha / sqrt(r) (test.py:288-289).  Replaces any adapter already on (layer, proj). */
 int jcb_vit_set_lora(jcb_vit* vit, int layer, int proj, const float* A, const float* B, int r, float scaling);
+/* LoRA slots: a tower holds adapter sets 0 .. G-1 (G <= JCB_MAX_LORA_SLOTS) and a call picks one per view
+ * (jcb_encode_image_slots) or per image (jcb_pipeline_slots): view v is encoded exactly -- bit for bit -- as if the tower
+ * carried only slot s[v], in applied mode.  Slot 0 is what jcb_vit_set_lora sets (jcb_vit_set_lora_slot with slot 0 is
+ * the same call); G = 1 + the highest slot given an adapter (or declared, jcb_vit_set_lora_slot_count) since the last
+ * jcb_vit_clear_lora, which clears all slots.
+ * More than one slot needs JCB_LORA_APPLIED: jcb_vit_finalize returns JCB_E_INVALID in merged mode, and also when a
+ * slot's q, k, v ranks of one layer sum to more than 64 or its 'o' rank exceeds 64.  A slot without an adapter on some
+ * (layer, projection) runs the plain projection there.  Per layer and projection the device holds one 64-row down block
+ * and one 64-column up block per slot; a 256-row GEMM tile multiplies the up blocks of the slots its rows use (measured
+ * on a B200 with one slot per image of 65 views: +2 to +3 % per step for G = 2 to 8; DESIGN.md section 4). */
+#define JCB_MAX_LORA_SLOTS 8
+int jcb_vit_set_lora_slot(jcb_vit* vit, int slot, int layer, int proj, const float* A, const float* B, int r, float scaling);
+/* Declare slots 0 .. n_slots-1 even if the highest of them has no adapter (an adapter set that is empty, e.g. the
+ * plain tower next to adapted ones): G = max(G, n_slots).  1 <= n_slots <= JCB_MAX_LORA_SLOTS; cleared by
+ * jcb_vit_clear_lora like the adapters. */
+int jcb_vit_set_lora_slot_count(jcb_vit* vit, int n_slots);
+/* G: the number of slots the next jcb_vit_finalize packs (1 without jcb_vit_set_lora_slot / _slot_count). */
+int jcb_vit_lora_slots(const jcb_vit* vit);
 int jcb_vit_clear_lora(jcb_vit* vit);
 /* Pack the weights for the device: W' = W + scaling * B A in fp32, then bf16 (GEMM operands); LayerNorm /
  * bias / embedding / final projection parameters stay fp32.  Must be called after the last set_param /
@@ -195,6 +214,11 @@ int jcb_vit_lora_mode(const jcb_vit* vit);
  *   out_dev      [n_views, embed_dim] float32 */
 int jcb_encode_image(jcb_vit* vit, const void* images_dev, int img_dtype, int64_t n_views, int apply_clip_norm,
                      int normalize, float* out_dev);
+/* jcb_encode_image with a LoRA slot per view: slot_of_view_host [n_views] int32 host array, each in [0, G).  It is
+ * validated before anything is launched (JCB_E_INVALID for a NULL array or a slot outside the tower's G, out_dev
+ * untouched) and copied to the device once per call.  A tower with one slot runs jcb_encode_image. */
+int jcb_encode_image_slots(jcb_vit* vit, const void* images_dev, int img_dtype, int64_t n_views,
+                           const int32_t* slot_of_view_host, int apply_clip_norm, int normalize, float* out_dev);
 /* Same with host buffers: host->device copies of the image chunks (overlapped with compute on a second
  * stream) and the device->host copy of the embeddings happen inside the call; it returns when out_host
  * is valid.  This is the call the end-to-end measurement times. */
@@ -364,6 +388,11 @@ typedef struct jcb_pipeline_args {
  * MTA solves.  `vit_zs` may be NULL (single tower) or a second tower for the zero-shot branch
  * (test.py:1711-1713). */
 int jcb_pipeline(jcb_vit* vit, jcb_vit* vit_zs, const jcb_pipeline_args* args);
+/* jcb_pipeline with a LoRA slot per image: slot_of_image_host [n_images] int32 host array, each in [0, G) of `vit`; every
+ * view of image i runs slot slot_of_image_host[i] of `vit` (jcb_vit_set_lora_slot), while `vit_zs` runs its own slot 0.
+ * Validated before anything is launched, like jcb_encode_image_slots.  These calls are never captured into or served
+ * from the CUDA graphs of jcb_ctx_set_graphs. */
+int jcb_pipeline_slots(jcb_vit* vit, jcb_vit* vit_zs, const jcb_pipeline_args* args, const int32_t* slot_of_image_host);
 
 /* Small calls (n_images * n_views <= max_views, default 1024; device work only; no out_feats / out_scores) are served
  * from CUDA graphs: the second jcb_pipeline call with the same towers, shapes and operand pointers is captured, later ones
@@ -382,6 +411,9 @@ int jcb_ctx_graph_stats(const jcb_ctx* ctx, int64_t* captured, int64_t* launched
  * JCB_MAX_INFLIGHT submissions may be un-waited (JCB_E_STATE otherwise). */
 #define JCB_MAX_INFLIGHT 4
 int jcb_pipeline_submit(jcb_vit* vit, jcb_vit* vit_zs, const jcb_pipeline_args* args, int64_t* ticket);
+/* jcb_pipeline_submit with per-image LoRA slots (jcb_pipeline_slots); the slot array is copied before the call returns. */
+int jcb_pipeline_submit_slots(jcb_vit* vit, jcb_vit* vit_zs, const jcb_pipeline_args* args, const int32_t* slot_of_image_host,
+                              int64_t* ticket);
 int jcb_pipeline_wait(jcb_ctx* ctx, int64_t ticket);
 
 /* ---------------------------------------------------------------- building blocks (tests) ---- */

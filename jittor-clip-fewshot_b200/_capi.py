@@ -17,6 +17,7 @@ JCB_OK = 0
 JCB_E_INVALID, JCB_E_CUDA, JCB_E_STATE, JCB_E_NO_DEVICE, JCB_E_KERNEL, JCB_E_NOMEM = -1, -2, -3, -4, -5, -6
 JCB_ABI_VERSION = 4
 MAX_INFLIGHT = 4   # JCB_MAX_INFLIGHT
+MAX_LORA_SLOTS = 8   # JCB_MAX_LORA_SLOTS
 IMG_F32, IMG_BF16, IMG_U8, IMG_PATCHES_BF16, IMG_PATCHES_F16 = 0, 1, 2, 3, 4
 PROJ_Q, PROJ_K, PROJ_V, PROJ_O = 0, 1, 2, 3
 SCORE_NAMES = ("logits", "cs", "cs1", "cs2", "cs3", "cs4", "cs5")
@@ -116,9 +117,13 @@ PROTOTYPES = {
     "jcb_vit_destroy": (c_int, [c_void_p]),
     "jcb_vit_set_param": (c_int, [c_void_p, c_char_p, c_void_p, c_int64]),
     "jcb_vit_set_lora": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_float]),
+    "jcb_vit_set_lora_slot": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_float]),
+    "jcb_vit_set_lora_slot_count": (c_int, [c_void_p, c_int]),
+    "jcb_vit_lora_slots": (c_int, [c_void_p]),
     "jcb_vit_clear_lora": (c_int, [c_void_p]),
     "jcb_vit_finalize": (c_int, [c_void_p]),
     "jcb_encode_image": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int, c_int, c_void_p]),
+    "jcb_encode_image_slots": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_void_p, c_int, c_int, c_void_p]),
     "jcb_encode_image_host": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int, c_int, c_void_p]),
     "jcb_vit_debug_tokens": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int, c_void_p]),
     "jcb_text_create": (c_int, [c_void_p, POINTER(TextConfig), POINTER(c_void_p)]),
@@ -146,9 +151,11 @@ PROTOTYPES = {
     "jcb_channel_lp": (c_int, [c_void_p, c_void_p, c_int64, c_int32, c_int32, POINTER(HeadWeights), c_void_p]),
     "jcb_logit_normalize": (c_int, [c_void_p, c_void_p, c_int64, c_int32, c_void_p]),
     "jcb_pipeline": (c_int, [c_void_p, c_void_p, POINTER(PipelineArgs)]),
+    "jcb_pipeline_slots": (c_int, [c_void_p, c_void_p, POINTER(PipelineArgs), c_void_p]),
     "jcb_ctx_set_graphs": (c_int, [c_void_p, c_int, c_int64]),
     "jcb_ctx_graph_stats": (c_int, [c_void_p, POINTER(c_int64), POINTER(c_int64), POINTER(c_int64)]),
     "jcb_pipeline_submit": (c_int, [c_void_p, c_void_p, POINTER(PipelineArgs), POINTER(c_int64)]),
+    "jcb_pipeline_submit_slots": (c_int, [c_void_p, c_void_p, POINTER(PipelineArgs), c_void_p, POINTER(c_int64)]),
     "jcb_pipeline_wait": (c_int, [c_void_p, c_int64]),
     "jcb_gemm": (c_int, [c_void_p, POINTER(GemmArgs)]),
     "jcb_fold_ln": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p,

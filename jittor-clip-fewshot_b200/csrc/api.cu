@@ -85,6 +85,8 @@ struct jcb_ctx {
   int operand_f16 = 1;               // 16-bit operand type towers are packed with: 1 = fp16 (default), 0 = bf16
   int lora_applied = 0;              // how towers packed from now on carry their LoRA adapters: 0 = merged into the
                                      // weights (default), 1 = applied as low-rank GEMMs (jcb_ctx_set_lora_mode)
+  int32_t* slot_dev = nullptr;       // per-view LoRA slots of the current call (jcb_*_slots), grow-only
+  int64_t slot_cap = 0;
   char err[512] = {0};
   // CUDA graphs of whole small pipelines (see PipelineGraph below)
   int graphs_on = 1;
@@ -234,12 +236,17 @@ struct LayerDev {
   // LoRA applied (jcb_ctx_set_lora_mode): the adapters of the packed in_proj / of out_proj side by side,
   // down = [A_q; A_k; A_v; 0] as [LORA_U_COLS, W] and up = [s B_q | s B_k | s B_v | 0] in the rows of its projection as
   // [3W, LORA_K2] ([W, LORA_K2] for out_proj); nullptr when the layer has no adapter there
+  // LoRA slots (jcb_vit_set_lora_slot): the same layout once per slot -- slot g's down rows are rows [64 g, 64 g + 64)
+  // of the down matrix ([lora_u_cols(G), W]), its up matrix is column block g of the up matrix ([3W | W, 64 G]).
   __nv_bfloat16 *lin_dn = nullptr, *lin_up = nullptr, *lout_dn = nullptr, *lout_up = nullptr;
+  uint32_t lin_slots = 0, lout_slots = 0;   // slots with an adapter on in_proj / out_proj of this layer
 };
 // columns of the low-rank intermediate U = x [A_q; A_k; A_v]^T (the GEMM kernel's minimum N) and the k extent the
 // second operand pair of the projection GEMM reads of it (one 64-wide k-block: the ranks of q, k, v together <= 64)
 constexpr int LORA_U_COLS = 128;
 constexpr int LORA_K2 = 64;
+// U of a tower with G slots: one 64-column block per slot, rounded up to the GEMM's N granularity (G = 1: LORA_U_COLS)
+int lora_u_cols(int G) { return (LORA_K2 * G + 127) / 128 * 128; }
 
 // What the image tower and the text tower share: a stack of pre-LN transformer blocks with packed-QKV
 // attention (+ LoRA adapters merged at pack time), the fp32 staging of the reference state dict and the
@@ -253,7 +260,8 @@ struct TowerBase {
   std::string prefix;                                // state-dict prefix of the blocks
   std::map<std::string, std::vector<float>> host;   // fp32 staging by reference key name
   std::map<std::string, int64_t> expected;          // key -> numel
-  std::map<int, LoraAdapter> lora;                  // layer * 4 + proj
+  std::vector<std::map<int, LoraAdapter>> lora = std::vector<std::map<int, LoraAdapter>>(1);   // [slot][layer * 4 + proj]
+  int lora_slots = 1;                               // slots the weights were packed with (the last finalize)
   bool finalized = false;
   void* arena = nullptr;                            // device weights
   size_t arena_bytes = 0;
@@ -277,7 +285,7 @@ struct jcb_text : TowerBase {
 namespace {
 
 int tower_set_param(TowerBase* t, const char* name, const float* data, int64_t numel);
-int tower_set_lora(TowerBase* t, int layer, int proj, const float* A, const float* B, int r, float scaling);
+int tower_set_lora(TowerBase* t, int layer, int proj, const float* A, const float* B, int r, float scaling, int slot = 0);
 
 std::string blk(const TowerBase* t, int i, const char* tail) { return t->prefix + std::to_string(i) + "." + tail; }
 
@@ -329,29 +337,29 @@ struct TowerWs {
   float* stats[2];
   float* shift[2];
 };
-size_t tower_ws_bytes_dims(size_t W, size_t T, size_t GG, size_t KP, int64_t n) {
+size_t tower_ws_bytes_dims(size_t W, size_t T, size_t GG, size_t KP, int64_t n, size_t u_cols = LORA_U_COLS) {
   const size_t big = std::max(n * GG * KP, n * T * 4 * W) * 2;
   return align_up(big) + align_up(n * T * W * 4) + align_up(n * T * W * 2) + align_up(n * T * 3 * W * 2) +
-         align_up(n * T * W * 2) + align_up(n * T * LORA_U_COLS * 2) + 2 * align_up(n * T * ((W + 255) / 256) * 8) +
+         align_up(n * T * W * 2) + align_up(n * T * u_cols * 2) + 2 * align_up(n * T * ((W + 255) / 256) * 8) +
          2 * align_up(n * T * 4);
 }
 size_t tower_ws_bytes(const jcb_vit* v, int64_t n) {
-  return tower_ws_bytes_dims(v->W, v->tokens, static_cast<size_t>(v->grid) * v->grid, v->kpatch, n);
+  return tower_ws_bytes_dims(v->W, v->tokens, static_cast<size_t>(v->grid) * v->grid, v->kpatch, n, lora_u_cols(v->lora_slots));
 }
-TowerWs tower_ws_carve_dims(size_t W, size_t T, size_t GG, size_t KP, int64_t n, Bump& b) {
+TowerWs tower_ws_carve_dims(size_t W, size_t T, size_t GG, size_t KP, int64_t n, Bump& b, size_t u_cols = LORA_U_COLS) {
   TowerWs w;
   w.big = b.take<__nv_bfloat16>(std::max(n * GG * KP, n * T * 4 * W));
   w.tokens = b.take<float>(n * T * W);
   w.ln_out = b.take<__nv_bfloat16>(n * T * W);
   w.qkv = b.take<__nv_bfloat16>(n * T * 3 * W);
   w.attn = b.take<__nv_bfloat16>(n * T * W);
-  w.lora_u = b.take<__nv_bfloat16>(n * T * LORA_U_COLS);
+  w.lora_u = b.take<__nv_bfloat16>(n * T * u_cols);
   for (int i = 0; i < 2; ++i) w.stats[i] = b.take<float>(n * T * ((W + 255) / 256) * 2);
   for (int i = 0; i < 2; ++i) w.shift[i] = b.take<float>(n * T);
   return w;
 }
 TowerWs tower_ws_carve(const jcb_vit* v, int64_t n, Bump& b) {
-  return tower_ws_carve_dims(v->W, v->tokens, static_cast<size_t>(v->grid) * v->grid, v->kpatch, n, b);
+  return tower_ws_carve_dims(v->W, v->tokens, static_cast<size_t>(v->grid) * v->grid, v->kpatch, n, b, lora_u_cols(v->lora_slots));
 }
 
 // LayerNorm-fold plumbing of one GEMM launch: the consumer (EPI_LNFOLD_*) reads `stats` / `colsum`; the producer
@@ -371,6 +379,10 @@ struct LnArgs {
   const __nv_bfloat16* B2 = nullptr;
   int K2 = 0;
   int64_t lda2 = 0, ldb2 = 0;
+  // LoRA slots (GemmArgs::slot_of_view)
+  const int* slot_of_view = nullptr;
+  int slot_rows = 0;
+  uint32_t slot_live = 0;
 };
 
 int run_gemm(jcb_ctx* ctx, int cls, int f16, const __nv_bfloat16* A, const __nv_bfloat16* B, int M, int N, int K,
@@ -380,19 +392,24 @@ int run_gemm(jcb_ctx* ctx, int cls, int f16, const __nv_bfloat16* A, const __nv_
   g.stats_in = ln.stats_in; g.shift_in = ln.shift_in; g.shift_out = ln.shift_out; g.stats_in_row_stride = ln.in_stride;
   g.A = A; g.B = B; g.lda = K; g.ldb = K; g.M = M; g.N = N; g.K = K; g.f16 = f16;
   g.A2 = ln.A2; g.B2 = ln.B2; g.K2 = ln.K2; g.lda2 = ln.lda2; g.ldb2 = ln.ldb2;
+  g.slot_of_view = ln.slot_of_view; g.slot_rows = ln.slot_rows; g.slot_live = ln.slot_live;
   g.bias = bias; g.epilogue = epi; g.out = out; g.ldo = ldo;
   // algorithmic bytes: A + B read once, C written once (read-modify-write for the residual epilogue)
   const bool lnprep = epi == EPI_RESID_LNPREP_SHORT || epi == EPI_RESID_LNPREP_LONG;
   const double out_b = (epi == EPI_BIAS_BF16 || epi == EPI_BIAS_GELU_BF16 || epi == EPI_LNFOLD_BF16 || epi == EPI_LNFOLD_GELU_BF16)
                            ? 2.0 : (epi == EPI_BIAS_RESID_F32 ? 8.0 : (lnprep ? 10.0 : 4.0));
-  const double bytes = 2.0 * M * (K + ln.K2) + 2.0 * N * (K + ln.K2) + out_b * M * N;
-  LAUNCH_P(ctx, cls, 2.0 * M * N * (K + ln.K2), bytes, launch_gemm(g, ctx->dev_status, ctx->num_sms, ctx->stream));
+  // with LoRA slots a row needs one slot's k-block (projection) / column block (down-projection) of the K2 / N extent
+  const int K2a = ln.slot_of_view && ln.K2 > 0 ? LORA_K2 : ln.K2;
+  const int Na = ln.slot_of_view && ln.K2 == 0 ? LORA_K2 : N;
+  const double bytes = 2.0 * M * (K + K2a) + 2.0 * N * (K + ln.K2) + out_b * M * N;
+  LAUNCH_P(ctx, cls, 2.0 * M * Na * (K + K2a), bytes, launch_gemm(g, ctx->dev_status, ctx->num_sms, ctx->stream));
   return JCB_OK;
 }
 
 // L pre-LN blocks on `n` sequences of t->tokens tokens: w.ln_out holds ln_1 of block 0 on entry, w.tokens the
 // fp32 residual stream; on exit w.tokens is the output of the last block (reference jclip/model.py:59-62).
-int tower_blocks(TowerBase* t, int64_t n, const TowerWs& w, int causal, bool cls_row0 = false) {
+// slot_dev (LoRA applied, towers with several slots): the slot of each of the n sequences, on the device; nullptr = slot 0.
+int tower_blocks(TowerBase* t, int64_t n, const TowerWs& w, int causal, bool cls_row0 = false, const int* slot_dev = nullptr) {
   jcb_ctx* ctx = t->ctx;
   cudaStream_t s = ctx->stream;
   const int W = t->W, T = t->tokens, f16 = t->f16;
@@ -476,25 +493,40 @@ int tower_blocks(TowerBase* t, int64_t n, const TowerWs& w, int causal, bool cls
   // LoRA applied (jcb_ctx_set_lora_mode; the form the reference evaluates, test.py:388-398: W x + b + s B (A x)):
   // U = x [A_q; A_k; A_v]^T as one narrow GEMM, then the projection GEMM accumulates U (s B)^T into the same TMEM
   // tile through its second operand pair -- the base weights stay un-merged, an adapter swap re-packs 2 x r rows.
-  auto lora_pair = [&](const __nv_bfloat16* x, const __nv_bfloat16* dn, const __nv_bfloat16* up, LnArgs* a) -> int {
-    if (!dn) return JCB_OK;
-    int rc2 = run_gemm(ctx, JCB_KC_GEMM_LORA, f16, x, dn, M, LORA_U_COLS, W, nullptr, EPI_BIAS_BF16, w.lora_u, LORA_U_COLS);
+  // Several slots, chosen per sequence (slot_dev): U holds one 64-column block per slot, zero outside the row's own
+  // slot, and the projection GEMM multiplies, per 256-row tile, the k-blocks of the slots present in it (gemm.cu SLOTS).
+  // Without slot_dev a multi-slot tower runs slot 0 alone: its 64 columns of U and k-block 0 of the up matrix.
+  const int G = t->lora_slots;
+  const int u_cols = lora_u_cols(G);
+  auto lora_pair = [&](const __nv_bfloat16* x, const __nv_bfloat16* dn, const __nv_bfloat16* up, uint32_t live, LnArgs* a) -> int {
+    if (!slot_dev) {
+      if (!(live & 1u)) return JCB_OK;
+      int rc2 = run_gemm(ctx, JCB_KC_GEMM_LORA, f16, x, dn, M, LORA_U_COLS, W, nullptr, EPI_BIAS_BF16, w.lora_u, LORA_U_COLS);
+      if (rc2) return rc2;
+      a->A2 = w.lora_u; a->B2 = up; a->K2 = LORA_K2; a->lda2 = LORA_U_COLS; a->ldb2 = static_cast<int64_t>(LORA_K2) * G;
+      return JCB_OK;
+    }
+    if (!live) return JCB_OK;
+    LnArgs d;
+    d.slot_of_view = slot_dev; d.slot_rows = T; d.slot_live = live;
+    int rc2 = run_gemm(ctx, JCB_KC_GEMM_LORA, f16, x, dn, M, u_cols, W, nullptr, EPI_BIAS_BF16, w.lora_u, u_cols, d);
     if (rc2) return rc2;
-    a->A2 = w.lora_u; a->B2 = up; a->K2 = LORA_K2; a->lda2 = LORA_U_COLS; a->ldb2 = LORA_K2;
+    a->A2 = w.lora_u; a->B2 = up; a->K2 = LORA_K2 * G; a->lda2 = u_cols; a->ldb2 = LORA_K2 * G;
+    a->slot_of_view = slot_dev; a->slot_rows = T; a->slot_live = live;
     return JCB_OK;
   };
   for (int l = 0; l < t->L; ++l) {
     const LayerDev& L = t->layers[l];
     {
       LnArgs a;
-      if ((rc = lora_pair(w.ln_out, L.lin_dn, L.lin_up, &a))) return rc;
+      if ((rc = lora_pair(w.ln_out, L.lin_dn, L.lin_up, L.lin_slots, &a))) return rc;
       if ((rc = run_gemm(ctx, JCB_KC_GEMM_QKV, f16, w.ln_out, L.in_w, M, 3 * W, W, L.in_b, EPI_BIAS_BF16, w.qkv, 3 * W, a))) return rc;
     }
     LAUNCH_P(ctx, JCB_KC_ATTENTION, 4.0 * n * t->heads * T * T * 64, MW * (6 + 2),
              launch_attention(w.qkv, n, T, t->heads, w.attn, s, causal, ctx->dev_status, ctx->num_sms, f16));
     {
       LnArgs a;
-      if ((rc = lora_pair(w.attn, L.lout_dn, L.lout_up, &a))) return rc;
+      if ((rc = lora_pair(w.attn, L.lout_dn, L.lout_up, L.lout_slots, &a))) return rc;
       if ((rc = run_gemm(ctx, JCB_KC_GEMM_OUT, f16, w.attn, L.out_w, M, W, W, L.out_b, EPI_BIAS_RESID_F32, w.tokens, W, a))) return rc;
     }
     LAUNCH_P(ctx, JCB_KC_LAYERNORM, 0, MW * (4 + 2), launch_layernorm(w.tokens, M, W, L.ln2_g, L.ln2_b, w.ln_out, s, f16));
@@ -510,7 +542,8 @@ int tower_blocks(TowerBase* t, int64_t n, const TowerWs& w, int causal, bool cls
 
 // The image tower on `n` views resident on the device.  Schedule = VisionTransformer.execute
 // (reference jclip/model.py:104-126) with every elementwise op fused into a neighbouring kernel.
-int tower_forward(jcb_vit* v, const void* images, int dt, int64_t n, int apply_norm, const TowerWs& w) {
+int tower_forward(jcb_vit* v, const void* images, int dt, int64_t n, int apply_norm, const TowerWs& w,
+                  const int* slot_dev = nullptr) {
   jcb_ctx* ctx = v->ctx;
   cudaStream_t s = ctx->stream;
   const int W = v->cfg.width, T = v->tokens, GG = v->grid * v->grid, KP = v->kpatch;
@@ -533,7 +566,7 @@ int tower_forward(jcb_vit* v, const void* images, int dt, int64_t n, int apply_n
   LAUNCH_P(ctx, JCB_KC_EMBED_LN, 0, MW * (4 + 4 + 2), launch_embed_ln(w.tokens, n, T, W, v->cls, v->pos, v->vpt, v->cfg.vpt_tokens, v->ln_pre_g, v->ln_pre_b, v->layers[0].ln1_g,
                               v->layers[0].ln1_b, w.ln_out, s, v->layers[0].in_wf ? w.stats[0] : nullptr, (W + 255) / 256,
                               patch_out, w.shift[0], v->f16));
-  return tower_blocks(v, n, w, 0, /*cls_row0=*/true);   // the tail reads token row 0 only
+  return tower_blocks(v, n, w, 0, /*cls_row0=*/true, slot_dev);   // the tail reads token row 0 only
 }
 
 // Views per pass through the tower.  Host input of a blocking call is cut into small passes so that the upload of
@@ -561,9 +594,9 @@ int check_vit(jcb_vit* v) {
 }
 
 // encode `n` views (device-resident when !on_host) into out_dev [n, E]; ws_extra bytes at the start of
-// the workspace are reserved for the caller.
+// the workspace are reserved for the caller.  slot_dev: the LoRA slot of each view on the device (slots_prepare), or nullptr.
 int encode_views(jcb_vit* v, const void* images, int dt, bool on_host, int64_t n, int apply_norm, int normalize,
-                 float* out_dev, size_t ws_extra) {
+                 float* out_dev, size_t ws_extra, const int* slot_dev = nullptr) {
   jcb_ctx* ctx = v->ctx;
   if (dt < 0 || dt > JCB_IMG_PATCHES_F16) return fail(ctx, JCB_E_INVALID, "unknown image dtype %d", dt);
   if (is_patches(dt)) {
@@ -604,7 +637,7 @@ int encode_views(jcb_vit* v, const void* images, int dt, bool on_host, int64_t n
       CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream, ctx->copy_done[buf], 0));
       src = ctx->stage[buf];
     }
-    if ((rc = tower_forward(v, src, dt, m, apply_norm, w))) return rc;
+    if ((rc = tower_forward(v, src, dt, m, apply_norm, w, slot_dev ? slot_dev + off : nullptr))) return rc;
     LAUNCH_P(ctx, JCB_KC_TAIL, 2.0 * m * v->cfg.width * v->cfg.embed_dim,
              static_cast<double>(m) * (v->cfg.width + v->cfg.embed_dim) * 4, launch_tail(w.tokens, m, v->tokens, v->cfg.width, v->ln_post_g, v->ln_post_b, v->proj,
                             v->cfg.embed_dim, normalize, out_dev + off * v->cfg.embed_dim, ctx->stream));
@@ -626,6 +659,41 @@ int sync_and_check(jcb_ctx* ctx) {
     cudaMemcpy(ctx->dev_status, &zero, sizeof(int), cudaMemcpyHostToDevice);
     return fail(ctx, JCB_E_KERNEL, "device-side kernel status %d (101 producer / 102 mma / 103 epilogue pipeline timeout)", st);
   }
+  return JCB_OK;
+}
+
+// LoRA slots of one call: `host` holds n_entries slots, each repeated for `repeat` consecutive views (1 per view, or V
+// per image).  Validated on the host before anything is launched, then copied to the device once, on the context's
+// stream (a pageable copy: the caller's array may be reused as soon as the call returns).  *dev = nullptr when the tower
+// has one slot: every entry is 0 and the call runs the single-slot schedule.
+int slots_prepare(jcb_vit* v, const int32_t* host, int64_t n_entries, int64_t repeat, const int32_t** dev) {
+  jcb_ctx* ctx = v->ctx;
+  *dev = nullptr;
+  if (!host) return fail(ctx, JCB_E_INVALID, "null LoRA slot array");
+  const int G = v->lora_slots;
+  for (int64_t i = 0; i < n_entries; ++i)
+    if (host[i] < 0 || host[i] >= G)
+      return fail(ctx, JCB_E_INVALID, "LoRA slot %d of entry %lld out of range: the tower carries %d slot(s)", host[i],
+                  static_cast<long long>(i), G);
+  if (G == 1 || n_entries <= 0) return JCB_OK;
+  const int64_t n = n_entries * repeat;
+  if (n > ctx->slot_cap) {   // growth: a queued submission may still read the old array
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    if (ctx->slot_dev) cudaFree(ctx->slot_dev);
+    ctx->slot_dev = nullptr;
+    ctx->slot_cap = 0;
+    cudaError_t e = cudaMalloc(&ctx->slot_dev, static_cast<size_t>(n) * sizeof(int32_t));
+    if (e != cudaSuccess) return fail(ctx, JCB_E_NOMEM, "cudaMalloc for the LoRA slot array failed: %s", cudaGetErrorString(e));
+    ctx->slot_cap = n;
+  }
+  std::vector<int32_t> per_view;
+  if (repeat > 1) {
+    per_view.resize(static_cast<size_t>(n));
+    for (int64_t i = 0; i < n; ++i) per_view[i] = host[i / repeat];
+    host = per_view.data();
+  }
+  CUDA_TRY(ctx, cudaMemcpyAsync(ctx->slot_dev, host, static_cast<size_t>(n) * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+  *dev = ctx->slot_dev;
   return JCB_OK;
 }
 
@@ -697,6 +765,7 @@ int jcb_ctx_destroy(jcb_ctx* ctx) {
     if (ctx->compute_done[i]) cudaEventDestroy(ctx->compute_done[i]);
   }
   if (ctx->dev_status) cudaFree(ctx->dev_status);
+  if (ctx->slot_dev) cudaFree(ctx->slot_dev);
   for (int i = 0; i < JCB_MAX_INFLIGHT; ++i)
     if (ctx->ticket_done[i]) cudaEventDestroy(ctx->ticket_done[i]);
   if (ctx->ticket_status) cudaFreeHost(ctx->ticket_status);
@@ -790,6 +859,9 @@ int jcb_ctx_trim(jcb_ctx* ctx) {
   }
   ctx->stage_bytes = 0;
   ctx->stage_recorded[0] = ctx->stage_recorded[1] = false;
+  if (ctx->slot_dev) cudaFree(ctx->slot_dev);
+  ctx->slot_dev = nullptr;
+  ctx->slot_cap = 0;
   return JCB_OK;
 }
 
@@ -910,9 +982,26 @@ int jcb_vit_set_lora(jcb_vit* v, int layer, int proj, const float* A, const floa
   return tower_set_lora(v, layer, proj, A, B, r, scaling);
 }
 
+int jcb_vit_set_lora_slot(jcb_vit* v, int slot, int layer, int proj, const float* A, const float* B, int r, float scaling) {
+  return tower_set_lora(v, layer, proj, A, B, r, scaling, slot);
+}
+
+int jcb_vit_set_lora_slot_count(jcb_vit* v, int n_slots) {
+  if (!v) return JCB_E_INVALID;
+  if (n_slots < 1 || n_slots > JCB_MAX_LORA_SLOTS)
+    return fail(v->ctx, JCB_E_INVALID, "set_lora_slot_count: %d slots out of range (1 .. %d)", n_slots, JCB_MAX_LORA_SLOTS);
+  if (static_cast<size_t>(n_slots) > v->lora.size()) {   // the new slots carry no adapter: plain projections
+    v->lora.resize(n_slots);
+    v->finalized = false;
+  }
+  return JCB_OK;
+}
+
+int jcb_vit_lora_slots(const jcb_vit* v) { return v ? static_cast<int>(v->lora.size()) : JCB_E_INVALID; }
+
 int jcb_vit_clear_lora(jcb_vit* v) {
   if (!v) return JCB_E_INVALID;
-  v->lora.clear();
+  v->lora.assign(1, {});
   v->finalized = false;
   return JCB_OK;
 }
@@ -1003,27 +1092,36 @@ struct Packer {
     CUDA_TRY(ctx, cudaStreamSynchronize(s));
     return JCB_OK;
   }
-  // LoRA applied: the adapters of one projection GEMM side by side (see LayerDev).  `adapters` = (row offset of the
-  // projection inside the packed weight, adapter); rows = rows of the packed weight.  s is folded into the up matrix.
-  int up_lora_applied(const std::vector<std::pair<size_t, const LoraAdapter*>>& adapters, size_t rows,
-                      __nv_bfloat16** dn, __nv_bfloat16** up) {
+  // LoRA applied: the adapters of one projection GEMM side by side (see LayerDev), once per slot.  `slots[g]` =
+  // (row offset of the projection inside the packed weight, adapter) of slot g; rows = rows of the packed weight.  s is
+  // folded into the up matrix.  *live = the slots with an adapter here.
+  int up_lora_applied(const std::vector<std::vector<std::pair<size_t, const LoraAdapter*>>>& slots, size_t rows,
+                      __nv_bfloat16** dn, __nv_bfloat16** up, uint32_t* live) {
     *dn = *up = nullptr;
-    if (adapters.empty()) return JCB_OK;
+    *live = 0;
+    const int G = static_cast<int>(slots.size());
+    for (int g = 0; g < G; ++g)
+      if (!slots[g].empty()) *live |= 1u << g;
+    if (!*live) return JCB_OK;
     cudaStream_t s = ctx->stream;
-    const size_t W = t->W;
-    int r_total = 0;
-    for (auto& ad : adapters) r_total += ad.second->r;
-    if (r_total > LORA_K2)
-      return fail(ctx, JCB_E_INVALID, "LoRA applied: the ranks of one projection GEMM sum to %d (max %d); use JCB_LORA_MERGED",
-                  r_total, LORA_K2);
-    std::vector<float> hd(static_cast<size_t>(LORA_U_COLS) * W, 0.f), hu(rows * LORA_K2, 0.f);
-    int j0 = 0;
-    for (auto& ad : adapters) {
-      const LoraAdapter* a = ad.second;
-      for (int j = 0; j < a->r; ++j) std::copy(a->A.begin() + j * W, a->A.begin() + (j + 1) * W, hd.begin() + (j0 + j) * W);
-      for (size_t n = 0; n < W; ++n)
-        for (int j = 0; j < a->r; ++j) hu[(ad.first + n) * LORA_K2 + j0 + j] = a->scaling * a->B[n * a->r + j];
-      j0 += a->r;
+    const size_t W = t->W, u_cols = lora_u_cols(G), k2 = static_cast<size_t>(LORA_K2) * G;
+    std::vector<float> hd(u_cols * W, 0.f), hu(rows * k2, 0.f);
+    for (int g = 0; g < G; ++g) {
+      int r_total = 0;
+      for (auto& ad : slots[g]) r_total += ad.second->r;
+      if (r_total > LORA_K2 && G == 1)
+        return fail(ctx, JCB_E_INVALID, "LoRA applied: the ranks of one projection GEMM sum to %d (max %d); use JCB_LORA_MERGED",
+                    r_total, LORA_K2);
+      if (r_total > LORA_K2)
+        return fail(ctx, JCB_E_INVALID, "LoRA slot %d: the ranks of one projection GEMM sum to %d (max %d)", g, r_total, LORA_K2);
+      size_t j0 = static_cast<size_t>(LORA_K2) * g;   // slot g: rows [64 g, 64 g + 64) of down, columns of up
+      for (auto& ad : slots[g]) {
+        const LoraAdapter* a = ad.second;
+        for (int j = 0; j < a->r; ++j) std::copy(a->A.begin() + j * W, a->A.begin() + (j + 1) * W, hd.begin() + (j0 + j) * W);
+        for (size_t n = 0; n < W; ++n)
+          for (int j = 0; j < a->r; ++j) hu[(ad.first + n) * k2 + j0 + j] = a->scaling * a->B[n * a->r + j];
+        j0 += a->r;
+      }
     }
     *dn = b.take<__nv_bfloat16>(hd.size());
     *up = b.take<__nv_bfloat16>(hu.size());
@@ -1040,21 +1138,25 @@ struct Packer {
     t->layers.assign(t->L, LayerDev());
     const bool applied = t->lora_applied != 0;
     const std::vector<std::pair<size_t, const LoraAdapter*>> none;
+    const size_t G = t->lora.size();
     int rc;
     for (int li = 0; li < t->L; ++li) {
       LayerDev& Ld = t->layers[li];
-      std::vector<std::pair<size_t, const LoraAdapter*>> in_ad, out_ad;
-      for (int p = 0; p < 3; ++p) {  // packed in_proj rows: q 0:W, k W:2W, v 2W:3W  (test.py:491-501)
-        auto it = t->lora.find(li * 4 + p);
-        if (it != t->lora.end()) in_ad.push_back({p * W, &it->second});
+      std::vector<std::vector<std::pair<size_t, const LoraAdapter*>>> in_ad(G), out_ad(G);   // per slot
+      for (size_t g = 0; g < G; ++g) {
+        for (int p = 0; p < 3; ++p) {  // packed in_proj rows: q 0:W, k W:2W, v 2W:3W  (test.py:491-501)
+          auto it = t->lora[g].find(li * 4 + p);
+          if (it != t->lora[g].end()) in_ad[g].push_back({p * W, &it->second});
+        }
+        auto ito = t->lora[g].find(li * 4 + JCB_PROJ_O);
+        if (ito != t->lora[g].end()) out_ad[g].push_back({0, &ito->second});
       }
-      auto ito = t->lora.find(li * 4 + JCB_PROJ_O);
-      if (ito != t->lora.end()) out_ad.push_back({0, &ito->second});
-      if ((rc = up_bf16(blk(t, li, "attn.in_proj_weight"), 3 * W, W, &Ld.in_w, applied ? none : in_ad))) return rc;
-      if ((rc = up_bf16(blk(t, li, "attn.out_proj.weight"), W, W, &Ld.out_w, applied ? none : out_ad))) return rc;
+      // merged mode has one slot (jcb_vit_finalize)
+      if ((rc = up_bf16(blk(t, li, "attn.in_proj_weight"), 3 * W, W, &Ld.in_w, applied ? none : in_ad[0]))) return rc;
+      if ((rc = up_bf16(blk(t, li, "attn.out_proj.weight"), W, W, &Ld.out_w, applied ? none : out_ad[0]))) return rc;
       if (applied) {
-        if ((rc = up_lora_applied(in_ad, 3 * W, &Ld.lin_dn, &Ld.lin_up))) return rc;
-        if ((rc = up_lora_applied(out_ad, W, &Ld.lout_dn, &Ld.lout_up))) return rc;
+        if ((rc = up_lora_applied(in_ad, 3 * W, &Ld.lin_dn, &Ld.lin_up, &Ld.lin_slots))) return rc;
+        if ((rc = up_lora_applied(out_ad, W, &Ld.lout_dn, &Ld.lout_up, &Ld.lout_slots))) return rc;
       }
       if ((rc = up_bf16(blk(t, li, "mlp.c_fc.weight"), 4 * W, W, &Ld.fc_w, {}))) return rc;
       if ((rc = up_bf16(blk(t, li, "mlp.c_proj.weight"), W, 4 * W, &Ld.proj_w, {}))) return rc;
@@ -1067,7 +1169,7 @@ struct Packer {
       if ((rc = up_f32(blk(t, li, "ln_2.weight"), &Ld.ln2_g))) return rc;
       if ((rc = up_f32(blk(t, li, "ln_2.bias"), &Ld.ln2_b))) return rc;
       if (!applied) {   // LoRA applied runs the stand-alone LayerNorm schedule (tower_blocks)
-        if ((rc = up_folded(blk(t, li, "attn.in_proj_weight"), 3 * W, W, in_ad, Ld.ln1_g, Ld.ln1_b, Ld.in_b, &Ld.in_wf,
+        if ((rc = up_folded(blk(t, li, "attn.in_proj_weight"), 3 * W, W, in_ad[0], Ld.ln1_g, Ld.ln1_b, Ld.in_b, &Ld.in_wf,
                             &Ld.in_S, &Ld.in_c))) return rc;
         if ((rc = up_folded(blk(t, li, "mlp.c_fc.weight"), 4 * W, W, {}, Ld.ln2_g, Ld.ln2_b, Ld.fc_b, &Ld.fc_wf, &Ld.fc_S,
                             &Ld.fc_c))) return rc;
@@ -1078,17 +1180,19 @@ struct Packer {
   int end() {
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     if (b.off > t->arena_bytes) return fail(ctx, JCB_E_STATE, "internal: weight arena overflow (%zu > %zu)", b.off, t->arena_bytes);
+    t->lora_slots = static_cast<int>(t->lora.size());
     t->finalized = true;
     return JCB_OK;
   }
 };
 
-size_t blocks_arena_bytes(size_t W, size_t L) {
+size_t blocks_arena_bytes(size_t W, size_t L, size_t G = 1) {
   // packed weights + biases / LayerNorm vectors, plus the LayerNorm-folded copies of in_proj / c_fc (Wf, S, c)
-  // (LoRA applied: the down / up matrices of in_proj and out_proj; the folded copies are not packed then)
+  // (LoRA applied: the down / up matrices of in_proj and out_proj for G slots; the folded copies are not packed then)
   return L * (align_up(3 * W * W * 2) + align_up(W * W * 2) + 2 * align_up(4 * W * W * 2) + 8 * align_up(4 * W * 4) +
               align_up(3 * W * W * 2) + align_up(4 * W * W * 2) + 4 * align_up(4 * W * 4) +
-              2 * align_up(LORA_U_COLS * W * 2) + align_up(3 * W * LORA_K2 * 2) + align_up(W * LORA_K2 * 2));
+              2 * align_up(lora_u_cols(static_cast<int>(G)) * W * 2) + align_up(3 * W * LORA_K2 * G * 2) +
+              align_up(W * LORA_K2 * G * 2));
 }
 
 int tower_set_param(TowerBase* t, const char* name, const float* data, int64_t numel) {
@@ -1103,11 +1207,14 @@ int tower_set_param(TowerBase* t, const char* name, const float* data, int64_t n
   return JCB_OK;
 }
 
-int tower_set_lora(TowerBase* t, int layer, int proj, const float* A, const float* B, int r, float scaling) {
+int tower_set_lora(TowerBase* t, int layer, int proj, const float* A, const float* B, int r, float scaling, int slot) {
   if (!t || !A || !B) return JCB_E_INVALID;
   if (layer < 0 || layer >= t->L || proj < 0 || proj > 3 || r < 1 || r > 256)
     return fail(t->ctx, JCB_E_INVALID, "set_lora: layer=%d proj=%d r=%d out of range", layer, proj, r);
-  LoraAdapter& a = t->lora[layer * 4 + proj];
+  if (slot < 0 || slot >= JCB_MAX_LORA_SLOTS)
+    return fail(t->ctx, JCB_E_INVALID, "set_lora_slot: slot %d out of range (0 .. %d)", slot, JCB_MAX_LORA_SLOTS - 1);
+  if (static_cast<size_t>(slot) >= t->lora.size()) t->lora.resize(slot + 1);
+  LoraAdapter& a = t->lora[slot][layer * 4 + proj];
   const int64_t W = t->W;
   a.A.assign(A, A + r * W);
   a.B.assign(B, B + W * r);
@@ -1133,9 +1240,27 @@ int jcb_vit_finalize(jcb_vit* v) {
   DeviceGuard g(ctx->device);
   int rc = tower_missing(v);
   if (rc) return rc;
+  const size_t G = v->lora.size();
+  if (G > 1) {   // several slots: every slot's rank limits are checked before anything is packed
+    if (!ctx->lora_applied)
+      return fail(ctx, JCB_E_INVALID, "%zu LoRA slots need JCB_LORA_APPLIED (applied mode); merged mode packs one adapter set", G);
+    for (size_t s = 0; s < G; ++s)
+      for (int li = 0; li < v->L; ++li) {
+        int r_qkv = 0;
+        for (int p = 0; p < 3; ++p) {
+          auto it = v->lora[s].find(li * 4 + p);
+          if (it != v->lora[s].end()) r_qkv += it->second.r;
+        }
+        auto ito = v->lora[s].find(li * 4 + JCB_PROJ_O);
+        const int r_o = ito != v->lora[s].end() ? ito->second.r : 0;
+        if (r_qkv > LORA_K2 || r_o > LORA_K2)
+          return fail(ctx, JCB_E_INVALID, "LoRA slot %zu, layer %d: the ranks of q, k, v sum to %d and r(o) = %d (max %d each)", s,
+                      li, r_qkv, r_o, LORA_K2);
+      }
+  }
   const size_t W = v->cfg.width, E = v->cfg.embed_dim, T = v->tokens, KP = v->kpatch, L = v->cfg.layers;
   // arena: bf16 GEMM operands, then fp32 vectors
-  const size_t bytes = align_up(W * KP * 2) + blocks_arena_bytes(W, L) + 9 * align_up(std::max(W * E, T * W) * 4);
+  const size_t bytes = align_up(W * KP * 2) + blocks_arena_bytes(W, L, G) + 9 * align_up(std::max(W * E, T * W) * 4);
   Packer pk(v);
   if ((rc = pk.begin(bytes, std::max(4 * W * W, W * KP)))) return rc;
   if ((rc = pk.up_bf16("visual.conv1.weight", W, KP, &v->conv_w, {}))) return rc;
@@ -1200,7 +1325,7 @@ int jcb_text_set_lora(jcb_text* t, int layer, int proj, const float* A, const fl
 
 int jcb_text_clear_lora(jcb_text* t) {
   if (!t) return JCB_E_INVALID;
-  t->lora.clear();
+  t->lora.assign(1, {});
   t->finalized = false;
   return JCB_OK;
 }
@@ -1264,6 +1389,16 @@ int jcb_encode_image(jcb_vit* v, const void* images_dev, int img_dtype, int64_t 
   if (rc) return rc;
   DeviceGuard g(v->ctx->device);
   return encode_views(v, images_dev, img_dtype, false, n_views, apply_clip_norm, normalize, out_dev, 0);
+}
+
+int jcb_encode_image_slots(jcb_vit* v, const void* images_dev, int img_dtype, int64_t n_views,
+                           const int32_t* slot_of_view_host, int apply_clip_norm, int normalize, float* out_dev) {
+  int rc = check_vit(v);
+  if (rc) return rc;
+  DeviceGuard g(v->ctx->device);
+  const int32_t* slot_dev = nullptr;
+  if ((rc = slots_prepare(v, slot_of_view_host, n_views, 1, &slot_dev))) return rc;
+  return encode_views(v, images_dev, img_dtype, false, n_views, apply_clip_norm, normalize, out_dev, 0, slot_dev);
 }
 
 int jcb_encode_image_host(jcb_vit* v, const void* images_host, int img_dtype, int64_t n_views, int apply_clip_norm,
@@ -1531,7 +1666,9 @@ int jcb_logit_normalize(jcb_ctx* ctx, const float* in, int64_t n, int32_t n_clas
 // ------------------------------------------------------------------------------------------------
 namespace {
 // Everything jcb_pipeline does, enqueued on the context's streams without waiting for any of it.
-int pipeline_enqueue(jcb_vit* vit, jcb_vit* vit_zs, const jcb_pipeline_args* a) {
+// with_slots: a jcb_pipeline_slots call, slot_of_image = its per-image LoRA slots of `vit` (host)
+int pipeline_enqueue(jcb_vit* vit, jcb_vit* vit_zs, const jcb_pipeline_args* a, bool with_slots = false,
+                     const int32_t* slot_of_image = nullptr) {
   int rc = check_vit(vit);
   if (rc) return rc;
   jcb_ctx* ctx = vit->ctx;
@@ -1540,8 +1677,11 @@ int pipeline_enqueue(jcb_vit* vit, jcb_vit* vit_zs, const jcb_pipeline_args* a) 
       !a->text_pt_t_dev || !a->text_hand_t_dev || !a->text_zs_t_dev)
     return fail(ctx, JCB_E_INVALID, "jcb_pipeline: null argument");
   if (a->n_images < 0 || a->n_views < 1 || a->k < 1 || a->k > 8) return fail(ctx, JCB_E_INVALID, "jcb_pipeline: bad sizes");
+  if (with_slots && !slot_of_image) return fail(ctx, JCB_E_INVALID, "jcb_pipeline_slots: null LoRA slot array");
   if (a->n_images == 0) return JCB_OK;
   DeviceGuard g(ctx->device);
+  const int32_t* slot_dev = nullptr;   // per view; vit_zs runs its own slot 0
+  if (with_slots && (rc = slots_prepare(vit, slot_of_image, a->n_images, a->n_views, &slot_dev))) return rc;
   const int E = vit->cfg.embed_dim, C = a->n_classes, V = a->n_views;
   const int64_t I = a->n_images, NV = I * V;
   // persistent part of the workspace: [feats] [feats_zs] [modes x3] [topk] [mta scratch]
@@ -1573,7 +1713,8 @@ int pipeline_enqueue(jcb_vit* vit, jcb_vit* vit_zs, const jcb_pipeline_args* a) 
   if (b.off > head_bytes) return fail(ctx, JCB_E_STATE, "internal: pipeline workspace overflow");
 
   // encode_image + L2 normalise over every view                      test.py:1705-1706 (:1711-1712)
-  if ((rc = encode_views(vit, a->images, a->img_dtype, a->images_on_host != 0, NV, a->apply_clip_norm, 1, feats, head_bytes))) return rc;
+  if ((rc = encode_views(vit, a->images, a->img_dtype, a->images_on_host != 0, NV, a->apply_clip_norm, 1, feats, head_bytes,
+                         slot_dev))) return rc;
   if (vit_zs && (rc = encode_views(vit_zs, a->images, a->img_dtype, a->images_on_host != 0, NV, a->apply_clip_norm, 1, feats_zs, head_bytes))) return rc;
   if (ctx->ws != ws_at_carve) return fail(ctx, JCB_E_STATE, "internal: the workspace moved while the pipeline held pointers into it");
   // solve_mta x3 in one launch                                        test.py:1708-1709, :1713
@@ -1750,6 +1891,13 @@ int jcb_pipeline(jcb_vit* vit, jcb_vit* vit_zs, const jcb_pipeline_args* a) {
   return JCB_OK;
 }
 
+int jcb_pipeline_slots(jcb_vit* vit, jcb_vit* vit_zs, const jcb_pipeline_args* a, const int32_t* slot_of_image_host) {
+  int rc = pipeline_enqueue(vit, vit_zs, a, true, slot_of_image_host);   // never served from a captured graph
+  if (rc) return rc;
+  if (a->n_images > 0 && a->topk_on_host) return sync_and_check(vit->ctx);
+  return JCB_OK;
+}
+
 }  // extern "C"
 void graphs_clear_fwd(jcb_ctx* ctx) { graphs_clear(ctx); }
 extern "C" {
@@ -1772,7 +1920,10 @@ int jcb_ctx_graph_stats(const jcb_ctx* ctx, int64_t* captured, int64_t* launched
   return JCB_OK;
 }
 
-int jcb_pipeline_submit(jcb_vit* vit, jcb_vit* vit_zs, const jcb_pipeline_args* a, int64_t* ticket) {
+}  // extern "C"
+namespace {
+int pipeline_submit(jcb_vit* vit, jcb_vit* vit_zs, const jcb_pipeline_args* a, bool with_slots, const int32_t* slot_of_image,
+                    int64_t* ticket) {
   int rc = check_vit(vit);
   if (rc) return rc;
   jcb_ctx* ctx = vit->ctx;
@@ -1781,7 +1932,7 @@ int jcb_pipeline_submit(jcb_vit* vit, jcb_vit* vit_zs, const jcb_pipeline_args* 
     return fail(ctx, JCB_E_STATE, "jcb_pipeline_submit: %d submissions already in flight; call jcb_pipeline_wait first",
                 JCB_MAX_INFLIGHT);
   ctx->overlapped = ctx->next_ticket > ctx->waited_ticket;
-  rc = pipeline_enqueue(vit, vit_zs, a);
+  rc = pipeline_enqueue(vit, vit_zs, a, with_slots, slot_of_image);
   ctx->overlapped = false;
   if (rc) return rc;
   DeviceGuard g(ctx->device);
@@ -1792,6 +1943,17 @@ int jcb_pipeline_submit(jcb_vit* vit, jcb_vit* vit_zs, const jcb_pipeline_args* 
   CUDA_TRY(ctx, cudaEventRecord(ctx->ticket_done[slot], ctx->stream));
   *ticket = ctx->next_ticket++;
   return JCB_OK;
+}
+}  // namespace
+extern "C" {
+
+int jcb_pipeline_submit(jcb_vit* vit, jcb_vit* vit_zs, const jcb_pipeline_args* a, int64_t* ticket) {
+  return pipeline_submit(vit, vit_zs, a, false, nullptr, ticket);
+}
+
+int jcb_pipeline_submit_slots(jcb_vit* vit, jcb_vit* vit_zs, const jcb_pipeline_args* a, const int32_t* slot_of_image_host,
+                              int64_t* ticket) {
+  return pipeline_submit(vit, vit_zs, a, true, slot_of_image_host, ticket);
 }
 
 int jcb_pipeline_wait(jcb_ctx* ctx, int64_t ticket) {

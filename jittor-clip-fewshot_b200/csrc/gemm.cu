@@ -122,11 +122,29 @@ struct GemmDev {
   float* shift_out;          // [M] new shift (written by the n_blk == 0 tiles)
   long long stats_in_stride; // row r of this GEMM = row r * stride of stats_in / shift_in (class-token-only last block)
   uint32_t idesc;            // tcgen05 instruction descriptor (operand formats, M, N)
+  // LoRA slots (SLOTS instantiations only; see GemmArgs::slot_of_view)
+  const int* slot_of_view;   // slot of view v = rows [v * slot_rows, (v + 1) * slot_rows)
+  int slot_rows;
+  uint32_t slot_live;        // slots that have an adapter in this GEMM
 };
+
+// Slots present among the rows of the CTA pair's 256-row tile m_blk, restricted to p.slot_live.  The producer, the MMA
+// issuer and the epilogue derive the same mask from the same inputs, so they agree on the k-blocks / tiles of a tile.
+__device__ __forceinline__ uint32_t tile_slot_mask(const GemmDev& p, int m_blk, int tile_m) {
+  const int r0 = m_blk * tile_m;
+  const int r1 = min(r0 + tile_m, p.M) - 1;
+  uint32_t mask = 0;
+  for (int v = r0 / p.slot_rows; v <= r1 / p.slot_rows; ++v) mask |= 1u << __ldg(p.slot_of_view + v);
+  return mask & p.slot_live;
+}
 
 // F16 selects the element type of 16-bit OUTPUTS (the conversion instruction of the epilogue); the operand formats
 // the tensor core assumes travel in p.idesc, so the fp32-output epilogues need no second instantiation.
-template <int BN, int EPI, bool F16>
+// SLOTS: several LoRA adapter sets, chosen per view (GemmArgs::slot_of_view).  With K2 > 0 (projection GEMM) second-pair
+// k-block g is slot g's up-projection and a tile loads / multiplies only the k-blocks of the slots its rows use; with
+// K2 == 0 (the down-projection GEMM) output column block [64 g, 64 g + 64) is slot g's: rows of other slots get exact
+// zeros there, and N tiles that hold no slot of the tile's rows are skipped (the projection GEMM never reads them).
+template <int BN, int EPI, bool F16, bool SLOTS>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(64 + 32 * epi_warps_of(EPI), 1)
 gemm_tcgen05_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                          const __grid_constant__ CUtensorMap tmOut, const __grid_constant__ CUtensorMap tmOut2,
@@ -170,6 +188,12 @@ gemm_tcgen05_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
   // the first pair's through the same ring into the same TMEM accumulator
   const int num_kb1 = p.K / BLOCK_K;
   const int num_kb = num_kb1 + p.K2 / BLOCK_K;
+  // SLOTS: the second-pair k-blocks of tile m_blk (projection), or whether tile (m_blk, n_blk) is computed at all (down)
+  constexpr uint32_t N_BLOCKS_MASK = (1u << (BN / 64)) - 1u;
+  auto slot_kb_mask = [&](int m_blk) -> uint32_t { return (SLOTS && p.K2 > 0) ? tile_slot_mask(p, m_blk, TILE_M) : 0u; };
+  auto slot_skip = [&](int m_blk, int n_blk) -> bool {
+    return SLOTS && p.K2 == 0 && ((tile_slot_mask(p, m_blk, TILE_M) >> (n_blk * (BN / 64))) & N_BLOCKS_MASK) == 0;
+  };
 
   if (threadIdx.x == 0) {
     tma_prefetch_desc(&tmA);
@@ -214,16 +238,23 @@ gemm_tcgen05_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
       bool ok = true;
       for (int tile = unit; tile < num_tiles && ok; tile += num_units) {
         const int m_blk = tile / n_tiles, n_blk = tile % n_tiles;
+        if (slot_skip(m_blk, n_blk)) continue;
         const int m0 = m_blk * TILE_M + static_cast<int>(cta_rank) * BLOCK_M;
         const int n0 = n_blk * BN + static_cast<int>(cta_rank) * Cfg::B_ROWS;
-        for (int kb = 0; kb < num_kb; ++kb) {
+        uint32_t kb2_rest = slot_kb_mask(m_blk);   // SLOTS: second-pair k-blocks still to load, lowest first
+        const int tile_kb = SLOTS && p.K2 > 0 ? num_kb1 + __popc(kb2_rest) : num_kb;
+        for (int kb = 0; kb < tile_kb; ++kb) {
           if (!mbar_wait(&empty_bar[stage], phase ^ 1u, p.status, JCB_DEV_TIMEOUT_PRODUCER)) { ok = false; break; }
           uint8_t* sa = ring + stage * Cfg::STAGE_BYTES;
           uint8_t* sb = sa + Cfg::A_BYTES;
           const bool second = kb >= num_kb1;
           const CUtensorMap* ta = second ? &tmA2 : &tmA;
           const CUtensorMap* tb = second ? &tmB2 : &tmB;
-          const int k0 = (second ? kb - num_kb1 : kb) * BLOCK_K;
+          int k0 = (second ? kb - num_kb1 : kb) * BLOCK_K;
+          if (SLOTS && second) {
+            k0 = (__ffs(static_cast<int>(kb2_rest)) - 1) * BLOCK_K;
+            kb2_rest &= kb2_rest - 1u;
+          }
           // the leader's barrier collects the bytes of BOTH CTAs; a complete_tx that lands before the
           // leader's expect_tx just drives the transaction count negative for a moment
           if (leader) mbar_arrive_expect_tx(&full_bar[stage], 2 * Cfg::STAGE_BYTES);
@@ -242,12 +273,16 @@ gemm_tcgen05_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
       int it = 0;
       bool ok = true;
       for (int tile = unit; tile < num_tiles && ok; tile += num_units, ++it) {
+        // `it` counts the tiles that use an accumulator stage: the stage and the barrier parities below are per use, so
+        // a skipped tile must not advance it (the `++it` of the loop header is undone)
+        if (slot_skip(tile / n_tiles, tile % n_tiles)) { --it; continue; }
         const int as = it & 1;
         const uint32_t aphase = (it >> 1) & 1;
         if (!mbar_wait(&tmem_empty_bar[as], aphase ^ 1u, p.status, JCB_DEV_TIMEOUT_MMA)) { ok = false; break; }
         tc_fence_after();
         const uint32_t tmem_d = tmem_base + static_cast<uint32_t>(as * BN);
-        for (int kb = 0; kb < num_kb; ++kb) {
+        const int tile_kb = SLOTS && p.K2 > 0 ? num_kb1 + __popc(slot_kb_mask(tile / n_tiles)) : num_kb;
+        for (int kb = 0; kb < tile_kb; ++kb) {
           if (!mbar_wait(&full_bar[stage], phase, p.status, JCB_DEV_TIMEOUT_MMA)) { ok = false; break; }
           tc_fence_after();
           const uint32_t sa = smem_u32(ring + stage * Cfg::STAGE_BYTES);
@@ -282,6 +317,7 @@ gemm_tcgen05_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
     bool ok = true;
     for (int tile = unit; tile < num_tiles && ok; tile += num_units, ++it) {
       const int m_blk = tile / n_tiles, n_blk = tile % n_tiles;
+      if (slot_skip(m_blk, n_blk)) { --it; continue; }   // as in the MMA issuer: `it` counts processed tiles only
       const int as = it & 1;
       const uint32_t aphase = (it >> 1) & 1;
       __syncwarp();
@@ -427,6 +463,11 @@ gemm_tcgen05_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
           ln_r = 1.0f / sqrtf(var + 1e-5f);
           ln_nmr = -mean * ln_r;
         }
+        // SLOTS down-projection: this thread's row keeps only the 64-column block of its own view's slot
+        int row_slot = -1;
+        if (SLOTS && p.K2 == 0 && row0 + lane < p.M) row_slot = __ldg(p.slot_of_view + (row0 + lane) / p.slot_rows);
+        const int blk0 = (n_blk * BN + col0) / 64;
+        (void)row_slot; (void)blk0;
         const uint64_t r2 = f2_pack(ln_r, ln_r), nmr2 = f2_pack(ln_nmr, ln_nmr);
         const uint64_t k05 = f2_pack(0.5f, 0.5f), k851 = f2_pack(0.851f, 0.851f);
         (void)r2; (void)nmr2; (void)k05; (void)k851;
@@ -501,6 +542,7 @@ gemm_tcgen05_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
               }
               o.x = pack_h2<F16>(f[0], f[1]); o.y = pack_h2<F16>(f[2], f[3]);
               o.z = pack_h2<F16>(f[4], f[5]); o.w = pack_h2<F16>(f[6], f[7]);
+              if (SLOTS && p.K2 == 0 && row_slot != blk0 + c) o = make_uint4(0u, 0u, 0u, 0u);   // CHUNK_COLS = 64
             } else {
               float f0, f1, f2, f3;
               f2_unpack(f2_add(f2_pack(__uint_as_float(cur[4 * j + 0]), __uint_as_float(cur[4 * j + 1])), bb2[2 * j]), f0, f1);
@@ -593,7 +635,7 @@ bool make_tmap_2d(CUtensorMap* tm, int dtype, const void* base, uint64_t rows, u
   return true;
 }
 
-template <int BN, int EPI, bool F16>
+template <int BN, int EPI, bool F16, bool SLOTS = false>
 cudaError_t launch_cfg(const GemmArgs& a, int* dev_status, int num_sms, cudaStream_t stream) {
   using Cfg = TileCfg<BN, EPI>;
   const int op_dt = a.f16 ? TM_F16 : TM_BF16;
@@ -615,7 +657,7 @@ cudaError_t launch_cfg(const GemmArgs& a, int* dev_status, int num_sms, cudaStre
     if (!make_tmap_2d(&tmA2, op_dt, a.A2, a.M, a.K2, a.lda2, BLOCK_M, BLOCK_K)) return cudaErrorInvalidValue;
     if (!make_tmap_2d(&tmB2, op_dt, a.B2, a.N, a.K2, a.ldb2, Cfg::B_ROWS, BLOCK_K)) return cudaErrorInvalidValue;
   }
-  auto kern = gemm_tcgen05_2cta_kernel<BN, EPI, F16>;
+  auto kern = gemm_tcgen05_2cta_kernel<BN, EPI, F16, SLOTS>;
   {
     cudaError_t e = ensure_dynamic_smem(kern, Cfg::SMEM_BYTES);
     if (e != cudaSuccess) return e;
@@ -627,6 +669,7 @@ cudaError_t launch_cfg(const GemmArgs& a, int* dev_status, int num_sms, cudaStre
   p.stats_in = a.stats_in; p.shift_in = a.shift_in; p.shift_out = a.shift_out;
   p.stats_in_stride = a.stats_in_row_stride > 0 ? a.stats_in_row_stride : 1;
   p.idesc = umma_idesc_f32acc(a.f16 != 0, BLOCK_M * CTAS, BN);
+  p.slot_of_view = a.slot_of_view; p.slot_rows = a.slot_rows; p.slot_live = a.slot_live;
   const int tile_m = BLOCK_M * CTAS;
   const int tiles = ((a.M + tile_m - 1) / tile_m) * (a.N / BN);
   const int units = num_sms / CTAS;                       // CTA pairs that fit the chip
@@ -641,6 +684,12 @@ cudaError_t launch_cfg(const GemmArgs& a, int* dev_status, int num_sms, cudaStre
 
 template <int BN>
 cudaError_t launch_bn(const GemmArgs& a, int* st, int sms, cudaStream_t s) {
+  if (a.slot_of_view) {   // LoRA slots: the QKV projection / down-projection (16-bit out) and out_proj (residual) only
+    if (a.epilogue == EPI_BIAS_BF16)
+      return a.f16 ? launch_cfg<BN, EPI_BIAS_BF16, true, true>(a, st, sms, s) : launch_cfg<BN, EPI_BIAS_BF16, false, true>(a, st, sms, s);
+    if (a.epilogue == EPI_BIAS_RESID_F32 && a.K2 > 0) return launch_cfg<BN, EPI_BIAS_RESID_F32, false, true>(a, st, sms, s);
+    return cudaErrorInvalidValue;
+  }
 #define JCB_CASE16(E) \
   case E: return a.f16 ? launch_cfg<BN, E, true>(a, st, sms, s) : launch_cfg<BN, E, false>(a, st, sms, s)
   switch (a.epilogue) {
@@ -691,8 +740,14 @@ cudaError_t launch_gemm(const GemmArgs& a, int* dev_status, int num_sms, cudaStr
   if (a.K2 > 0 && (!a.A2 || !a.B2 || (reinterpret_cast<uintptr_t>(a.A2) & 15) || (reinterpret_cast<uintptr_t>(a.B2) & 15) ||
                    (a.lda2 % 8) || (a.ldb2 % 8) || a.lda2 < a.K2 || a.ldb2 < a.K2))
     return cudaErrorInvalidValue;
-  // BN = 256 whenever N allows it; 128 otherwise (only used by generic/test shapes).
-  if (a.N % 256 == 0) return launch_bn<256>(a, dev_status, num_sms, stream);
+  if (a.slot_of_view && (a.slot_rows < 1 || a.slot_live == 0 || a.slot_live >= (1u << LORA_MAX_SLOTS) ||
+                         (a.K2 > 0 && 64 * (32 - __builtin_clz(a.slot_live)) > a.K2) ||
+                         (a.K2 == 0 && 64 * (32 - __builtin_clz(a.slot_live)) > a.N)))
+    return cudaErrorInvalidValue;
+  // BN = 256 whenever N allows it; 128 otherwise (only used by generic/test shapes).  The LoRA-slot down-projection
+  // always runs BN = 128: an N tile then covers two slots' 64-column blocks, so a tile whose rows use one slot computes
+  // (and skips) in steps of two slots instead of four.
+  if (a.N % 256 == 0 && !(a.slot_of_view && a.K2 == 0)) return launch_bn<256>(a, dev_status, num_sms, stream);
   return launch_bn<128>(a, dev_status, num_sms, stream);
 }
 

@@ -59,7 +59,17 @@ struct GemmArgs {
   const float* shift_in = nullptr;   // [M * stats_in_row_stride]
   float* shift_out = nullptr;        // [M]
   int64_t stats_in_row_stride = 1;
+  // LoRA slots (several adapter sets, chosen per view): slot_of_view[v] is the slot of rows [v * slot_rows,
+  // (v + 1) * slot_rows) and slot_live the slots that have an adapter in this GEMM.  With K2 > 0, second-pair k-block g
+  // belongs to slot g: a 256-row tile multiplies only the k-blocks of slots its rows use.  With K2 == 0 (EPI_BIAS_BF16,
+  // the down-projection U = x A^T), output columns [64 g, 64 g + 64) belong to slot g: a row gets exact zeros in the
+  // blocks of other slots, and tiles whose column blocks hold no slot of the tile's rows are not computed (nor written).
+  // nullptr: none (the kernels without the per-tile slot logic).
+  const int* slot_of_view = nullptr;
+  int slot_rows = 0;
+  uint32_t slot_live = 0;
 };
+constexpr int LORA_MAX_SLOTS = 8;   // JCB_MAX_LORA_SLOTS
 
 // Persistent TMA + tcgen05 GEMM.  Requires N % 128 == 0 and K % 64 == 0 (every GEMM of the ViT-B/32
 // tower satisfies it); any M.  Returns cudaErrorInvalidValue otherwise.

@@ -215,9 +215,29 @@ class VisionTransformer(Module):
         self._dirty = True
         self._vit = None        # jcb_vit*
         self._ctx = None
+        self._lora_slots = []   # LoRA slots 1 .. G-1: {layer: {proj code: (A, B, r, scaling)}} (set_lora_slots)
 
     def mark_dirty(self):
         self._dirty = True
+
+    def set_lora_slots(self, slots, alpha=1.0):
+        """Register LoRA slots 1 .. len(slots) of the image tower; slot 0 stays what `apply_lora` / `load_lora` put on the
+        model.  Each entry is the path of a reference-layout LoRA pickle (`save_lora`) or a dict {layer: {proj: (A, B)}}
+        (proj in "q", "k", "v", "o"; A [r, width], B [width, r]; scaling alpha / sqrt(r), or pass (A, B, scaling)).
+        A call then picks a slot per view (`visual(x, slot_of_view=...)`) or per image (HotPath `slot_of_image`), and
+        each view comes out bit-identical to a tower that carries only its slot.  Slots need the applied LoRA mode
+        (`Context.set_lora_mode("applied")`).  `set_lora_slots([])` drops them."""
+        from ..lora import slot_adapters
+        slots = list(slots)
+        if len(slots) + 1 > _capi.MAX_LORA_SLOTS:
+            raise ValueError(f"{len(slots) + 1} LoRA slots (slot 0 + {len(slots)}); at most {_capi.MAX_LORA_SLOTS}")
+        self._lora_slots = [slot_adapters(s, self.layers, self.width, alpha) for s in slots]
+        self._dirty = True
+
+    @property
+    def lora_slots(self):
+        """G: slot 0 plus the slots registered with set_lora_slots."""
+        return 1 + len(self._lora_slots)
 
     # ---- native engine ------------------------------------------------------------------------
     def _engine(self, device=None):
@@ -254,6 +274,13 @@ class VisionTransformer(Module):
                     B = np.ascontiguousarray(lin.w_lora_B.data, dtype=np.float32)
                     check(lib.jcb_vit_set_lora(self._vit, i, code, A.ctypes.data_as(c_void_p),
                                                B.ctypes.data_as(c_void_p), lin.r, float(lin.scaling)), ctx.handle)
+            if self._lora_slots:   # every registered slot counts, also one that carries no adapter
+                check(lib.jcb_vit_set_lora_slot_count(self._vit, 1 + len(self._lora_slots)), ctx.handle)
+            for g, slot in enumerate(self._lora_slots, 1):
+                for i, projs in sorted(slot.items()):
+                    for code, (A, B, r, scaling) in sorted(projs.items()):
+                        check(lib.jcb_vit_set_lora_slot(self._vit, g, i, code, A.ctypes.data_as(c_void_p),
+                                                        B.ctypes.data_as(c_void_p), r, scaling), ctx.handle)
             check(lib.jcb_vit_finalize(self._vit), ctx.handle)
             self._dirty = False
         return ctx, self._vit
@@ -274,9 +301,10 @@ class VisionTransformer(Module):
         except Exception:
             pass
 
-    def execute(self, x, apply_clip_norm=False, normalize=False):
+    def execute(self, x, apply_clip_norm=False, normalize=False, slot_of_view=None):
         """[B,3,R,R] -> [B,output_dim] float32.  Device tensors (torch, or anything exporting DLPack
-        such as a jittor.Var) are used in place; host arrays go through the *_host entry point."""
+        such as a jittor.Var) are used in place; host arrays go through the *_host entry point.
+        slot_of_view: None, or B LoRA slot indices (set_lora_slots): view b is encoded with slot slot_of_view[b] only."""
         was_numpy = isinstance(x, np.ndarray)
         t = as_torch(x)
         R = self.input_resolution
@@ -287,6 +315,21 @@ class VisionTransformer(Module):
         code = img_dtype_code(t)
         t = t.contiguous()
         n = t.shape[0]
+        if slot_of_view is not None:
+            # host images are copied to the device first (the slot entry point takes device input)
+            slots = slot_array(slot_of_view, n, "slot_of_view")
+            on_device = t.is_cuda
+            dev = t.device if on_device else torch.device("cuda", get_context(None).device)
+            with torch.cuda.device(dev):
+                t = t.to(dev)
+                ctx, vit = self._engine(dev)
+                ctx.bind_current_stream()
+                out = torch.empty((n, self.output_dim), dtype=torch.float32, device=dev)
+                check(ctx.lib.jcb_encode_image_slots(vit, ptr(t), code, n, slots.ctypes.data_as(c_void_p),
+                                                     int(apply_clip_norm), int(normalize), ptr(out)), ctx.handle)
+            if on_device:
+                return out
+            return out.cpu().numpy() if was_numpy else out.cpu()
         if t.is_cuda:
             with torch.cuda.device(t.device):
                 ctx, vit = self._engine(t.device)
@@ -324,6 +367,15 @@ class VisionTransformer(Module):
             check(ctx.lib.jcb_vit_debug_tokens(vit, ptr(t), img_dtype_code(t), t.shape[0], int(apply_clip_norm), ptr(out)),
                   ctx.handle)
         return out
+
+
+def slot_array(slots, n, name):
+    """A host int32 array of n LoRA slot indices (the library validates their range)."""
+    a = np.ascontiguousarray(as_torch(slots).cpu().numpy() if isinstance(slots, torch.Tensor) else np.asarray(slots),
+                             dtype=np.int32)
+    if a.shape != (n,):
+        raise ValueError(f"{name} must hold {n} slot indices, got shape {a.shape}")
+    return a
 
 
 class Embedding(Module):

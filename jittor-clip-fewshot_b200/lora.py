@@ -228,3 +228,54 @@ def load_lora_swa(args, list_lora_layers, swa_weights_folder):
             for k in pw:
                 pw[k] /= count
     _assign(args, list_lora_layers, acc)
+
+
+_PROJ_CODE = {'q': 0, 'k': 1, 'v': 2, 'o': 3}
+_NAME_PROJ = {name: p for p, name in _KEYS}
+
+
+def _vision_blocks(metadata, layers):
+    """Image-tower block index of each `layer_i` entry of a pickle written by save_lora: apply_lora's order, text blocks
+    first for encoder 'both' (test.py:608-640)."""
+    enc, pos = metadata['encoder'], metadata['position']
+    if enc not in ('vision', 'both'):
+        raise ValueError(f"the pickle holds {enc!r} adapters; LoRA slots are image-tower adapters")
+    table = INDEX_POSITIONS_VISION['ViT-L/14' if layers > 12 else 'ViT-B/16']
+    blocks = [i for i in table[pos] if i < layers]
+    skip = len(INDEX_POSITIONS_TEXT[pos]) if enc == 'both' else 0
+    return skip, blocks
+
+
+def slot_adapters(entry, layers, width, alpha=1.0):
+    """One LoRA slot as {block: {proj code: (A [r, width], B [width, r], r, scaling)}} float32, from a reference-layout
+    pickle path (scaling = metadata alpha / sqrt(r), test.py:288-289) or from a dict {block: {proj: (A, B)}} with proj in
+    'q', 'k', 'v', 'o' (scaling alpha / sqrt(r), or given as a third element)."""
+    out = {}
+
+    def put(block, proj, A, B, scaling):
+        A = np.ascontiguousarray(A, dtype=np.float32)
+        B = np.ascontiguousarray(B, dtype=np.float32)
+        r = A.shape[0]
+        if not 0 <= block < layers:
+            raise ValueError(f"LoRA slot: block {block} outside the tower's {layers} blocks")
+        if A.shape != (r, width) or B.shape != (width, r):
+            raise ValueError(f"LoRA slot, block {block} proj {proj}: A {A.shape} / B {B.shape}, expected [r, {width}] / [{width}, r]")
+        out.setdefault(block, {})[_PROJ_CODE[proj]] = (A, B, r, float(alpha / math.sqrt(r) if scaling is None else scaling))
+
+    if isinstance(entry, (str, os.PathLike)):
+        if not os.path.exists(entry):
+            raise FileNotFoundError(f'File {entry} does not exist.')
+        with open(entry, 'rb') as f:
+            loaded = pickle.load(f)
+        md = loaded['metadata']
+        skip, blocks = _vision_blocks(md, layers)
+        for i, block in enumerate(blocks):
+            for name, w in loaded['weights'].get(f'layer_{skip + i}', {}).items():
+                put(block, _NAME_PROJ[name], w['w_lora_A'], w['w_lora_B'], md['alpha'] / math.sqrt(md['r']))
+        return out
+    for block, projs in entry.items():
+        for proj, ab in projs.items():
+            if proj not in _PROJ_CODE:
+                raise ValueError(f"LoRA slot: unknown projection {proj!r} (q, k, v, o)")
+            put(int(block), proj, ab[0], ab[1], ab[2] if len(ab) > 2 else None)
+    return out

@@ -15,6 +15,7 @@ import torch
 
 from . import _capi
 from ._capi import check
+from .jclip.model import slot_array
 from .methods import Channel_LP, cosine_topk, solve_mta_batched
 from .runtime import as_torch, dev_f32, get_context, img_dtype_code, ptr
 
@@ -83,12 +84,15 @@ class HotPath:
         a.out_scores_dev = out_scores.data_ptr() if out_scores is not None else None
         return a
 
-    def evaluate_base(self, images, return_feats=False, return_scores=False, topk_to_host=None):
+    def evaluate_base(self, images, return_feats=False, return_scores=False, topk_to_host=None, slot_of_image=None):
         """images [I, V, 3, R, R] (V = N+1 views, view 0 un-augmented; reference test.py:1700), float32 /
         bfloat16 / uint8, on the device or in (pinned) host memory.  Returns int32 top-k [I, k] -- on the
-        host when the images were on the host (the end-to-end call), else on the device."""
+        host when the images were on the host (the end-to-end call), else on the device.
+        slot_of_image: None, or I LoRA slot indices of the image tower (VisionTransformer.set_lora_slots): every view of
+        image i runs slot slot_of_image[i]; the zero-shot tower runs its own slot 0."""
         t = self._check_input(images)
         I, V = t.shape[0], t.shape[1]
+        slots = slot_array(slot_of_image, I, "slot_of_image") if slot_of_image is not None else None
         on_host = not t.is_cuda
         device = self.text.device
         if topk_to_host is None:
@@ -102,7 +106,11 @@ class HotPath:
             feats = torch.empty((I * V, self.text.dim), dtype=torch.float32, device=device) if return_feats else None
             scores = torch.empty((I, self.text.num_classes), dtype=torch.float32, device=device) if return_scores else None
             a = self._args(t, I, V, on_host, topk, feats, scores, device)
-            check(ctx.lib.jcb_pipeline(vit, vit_zs, _capi.byref(a)), ctx.handle)
+            if slots is None:
+                check(ctx.lib.jcb_pipeline(vit, vit_zs, _capi.byref(a)), ctx.handle)
+            else:
+                check(ctx.lib.jcb_pipeline_slots(vit, vit_zs, _capi.byref(a), slots.ctypes.data_as(_capi.c_void_p)),
+                      ctx.handle)
         out = [topk]
         if return_feats:
             out.append(feats.view(I, V, -1))
@@ -112,12 +120,13 @@ class HotPath:
 
     # ---- streams of batches: the reference's `for images in loader:` loop with the next batch's uploads
     #      overlapping this batch's compute (jcb_pipeline_submit / jcb_pipeline_wait)
-    def submit(self, images):
-        """Enqueue evaluate_base(images) without waiting and return a ticket for `collect`.  `images` as in
-        evaluate_base; host images must be page-locked (pin_memory) for the copies to overlap compute and
+    def submit(self, images, slot_of_image=None):
+        """Enqueue evaluate_base(images, slot_of_image=...) without waiting and return a ticket for `collect`.  `images`
+        as in evaluate_base; host images must be page-locked (pin_memory) for the copies to overlap compute and
         must not be modified until `collect` returns."""
         t = self._check_input(images)
         I, V = t.shape[0], t.shape[1]
+        slots = slot_array(slot_of_image, I, "slot_of_image") if slot_of_image is not None else None
         device = self.text.device
         with torch.cuda.device(device):
             ctx, vit = self.model.visual._engine(device)
@@ -126,7 +135,11 @@ class HotPath:
             topk = torch.empty((I, self.k), dtype=torch.int32, device="cpu", pin_memory=True)
             a = self._args(t, I, V, not t.is_cuda, topk, None, None, device)
             ticket = _capi.c_int64()
-            check(ctx.lib.jcb_pipeline_submit(vit, vit_zs, _capi.byref(a), _capi.byref(ticket)), ctx.handle)
+            if slots is None:
+                check(ctx.lib.jcb_pipeline_submit(vit, vit_zs, _capi.byref(a), _capi.byref(ticket)), ctx.handle)
+            else:
+                check(ctx.lib.jcb_pipeline_submit_slots(vit, vit_zs, _capi.byref(a), slots.ctypes.data_as(_capi.c_void_p),
+                                                        _capi.byref(ticket)), ctx.handle)
         return _Ticket(ctx, ticket.value, topk, (t, a))
 
     def collect(self, ticket):
@@ -137,12 +150,14 @@ class HotPath:
 
     def evaluate_stream(self, batches, depth=2):
         """Generator over an iterable of image batches: yields the host top-k of each batch in order while up to
-        `depth` batches are in flight (depth 2 = the uploads of batch k+1 overlap the compute of batch k)."""
+        `depth` batches are in flight (depth 2 = the uploads of batch k+1 overlap the compute of batch k).  An item of
+        `batches` is an image batch, or an (images, slot_of_image) pair to run LoRA slots per image (see submit)."""
         if not 1 <= depth <= _capi.MAX_INFLIGHT:
             raise ValueError(f"depth must be in 1..{_capi.MAX_INFLIGHT}")
         pending = []
-        for images in batches:
-            pending.append(self.submit(images))
+        for item in batches:
+            images, slots = item if isinstance(item, tuple) else (item, None)
+            pending.append(self.submit(images, slot_of_image=slots))
             if len(pending) >= depth:
                 yield self.collect(pending.pop(0))
         while pending:
