@@ -152,7 +152,11 @@ int64_t jcb_ctx_launch_count(const jcb_ctx* ctx);
 #define JCB_KC_OTHER 12
 #define JCB_KC_TTA 13
 #define JCB_KC_GEMM_LORA 14   /* LoRA applied: the narrow down-projection GEMMs */
-#define JCB_KC_COUNT 15
+#define JCB_KC_BWD_GEMM 15    /* LoRA training backward: input-gradient GEMMs, the c_fc recompute and the LoRA GEMMs */
+#define JCB_KC_BWD_ATTENTION 16   /* LoRA training backward: attention */
+#define JCB_KC_BWD_ROWWISE 17 /* LoRA training: LayerNorm / QuickGELU / dropout / tail backward, casts, tape copies */
+#define JCB_KC_LORA_GRAD 18   /* LoRA training backward: the dA / dB reductions */
+#define JCB_KC_COUNT 19
 int jcb_ctx_profile(jcb_ctx* ctx, int enable);
 int jcb_ctx_profile_read(const jcb_ctx* ctx, int kernel_class, double* total_ms, int64_t* launches,
                          int64_t* timed_launches, double* flops, double* bytes);
@@ -415,6 +419,44 @@ int jcb_pipeline_submit(jcb_vit* vit, jcb_vit* vit_zs, const jcb_pipeline_args* 
 int jcb_pipeline_submit_slots(jcb_vit* vit, jcb_vit* vit_zs, const jcb_pipeline_args* args, const int32_t* slot_of_image_host,
                               int64_t* ticket);
 int jcb_pipeline_wait(jcb_ctx* ctx, int64_t ticket);
+
+/* ---------------------------------------------------------------- LoRA training -------------- */
+/* Gradients of a scalar loss with respect to the image tower's LoRA adapters A and B (slot 0), for the reference's
+ * training step (lora_train_vlp.py:921-1024): a training forward that keeps a tape, then a backward that takes
+ * dL/dfeatures.  Every other parameter is frozen.  Supported: towers of at most 64 tokens (ViT-B/32, plain or IVLP),
+ * packed in JCB_LORA_APPLIED mode with one slot and at least one adapter (q, k, v, o on any blocks; per block the
+ * ranks of q, k, v sum to at most 64 and r(o) <= 64).  Anything else returns JCB_E_INVALID before any launch, outputs
+ * untouched (also for a tower that is not finalized).
+ *
+ * Training dropout on the LoRA branch input (reference LoRALayer, test.py:291-297): inverted dropout with an
+ * independent mask per (layer, projection), generated on the device from Philox4x32-10 of (seed, step, layer,
+ * projection, row, column); row = view index within the call * tokens + token.  jcb_lora_dropout_mask writes one. */
+typedef struct jcb_tape jcb_tape;
+/* Re-pack the adapter values from device fp32 arrays without touching the base weights (after an optimiser step).
+ * A_dev / B_dev: host arrays of layers * 4 device pointers, index layer * 4 + JCB_PROJ_*; A [r, width], B [width, r]
+ * (the layout of jcb_vit_set_lora).  The set of adapters, their ranks and scalings are the ones of the last
+ * jcb_vit_finalize: a pointer must be non-NULL exactly where the tower carries an adapter.  Must be called at least once
+ * after each finalize before jcb_vit_train_forward; jcb_encode_image then also runs the new values.  JCB_E_STATE while a
+ * tape is alive (its backward would mix old and new adapters). */
+int jcb_vit_train_set_lora(jcb_vit* vit, const float* const* A_dev, const float* const* B_dev);
+/* jcb_encode_image (applied-mode schedule) that also records what the backward needs in a new tape *tape.  dropout_rate
+ * in [0, 1); 0 runs the LoRA branch on its undropped input.  out_dev [n_views, embed_dim] fp32.  The tape is sized for
+ * this call (about 0.64 MB per view per block for ViT-B/32, computed from shapes) and owned by the caller until
+ * jcb_tape_release. */
+int jcb_vit_train_forward(jcb_vit* vit, const void* images_dev, int img_dtype, int64_t n_views, int apply_clip_norm,
+                          int normalize, float dropout_rate, uint64_t seed, int64_t step, float* out_dev, jcb_tape** tape);
+/* The same with DLPack tensors (borrowed, as jcb_encode_image_dlpack). */
+int jcb_vit_train_forward_dlpack(jcb_vit* vit, void* images_dlmanaged, void* out_dlmanaged, int apply_clip_norm, int normalize,
+                                 float dropout_rate, uint64_t seed, int64_t step, jcb_tape** tape);
+/* dfeat_dev [n_views, embed_dim] fp32 = dL/d(out_dev of the forward).  Writes (overwrites) dA [r, width] and dB [width, r]
+ * fp32 for every adapter, through host arrays of layers * 4 device pointers laid out like jcb_vit_train_set_lora's.
+ * The sums over rows run in a fixed order given the view count: the same inputs give the same bits.  May be called
+ * more than once on a tape. */
+int jcb_vit_train_backward(jcb_tape* tape, const float* dfeat_dev, float* const* dA_dev, float* const* dB_dev);
+int jcb_tape_release(jcb_tape* tape);
+/* out_dev [rows, cols] uint8: 1 where the training dropout keeps element (row, col) of projection `proj` of `layer`. */
+int jcb_lora_dropout_mask(jcb_ctx* ctx, uint64_t seed, int64_t step, int layer, int proj, int64_t rows, int32_t cols, float rate,
+                          uint8_t* out_dev);
 
 /* ---------------------------------------------------------------- building blocks (tests) ---- */
 /* GEMM epilogues fused into the tcgen05 kernel (csrc/kernels.h GemmEpilogue) */

@@ -9,13 +9,14 @@ behind the reference's own Python API: `jclip.load`, `model.encode_image`, `appl
 
 The directory name has hyphens, so import it through the repo-root shim:  `import jclip_b200`.
 """
-from . import _capi, blocks, dist, jclip, lora, methods, pipeline, runtime, synth, tta  # noqa: F401
+from . import _capi, blocks, dist, jclip, lora, methods, pipeline, runtime, synth, train, tta  # noqa: F401
 from ._capi import JcbError, load_library  # noqa: F401
 from .jclip import clip  # noqa: F401
 from .lora import apply_lora, load_lora, load_lora_swa, save_lora  # noqa: F401
 from .methods import Channel_LP, clip_classifier, cls_acc, cosine_topk, logit_normalize, solve_mta, solve_mta_batched, solve_mta_logits  # noqa: F401
 from .pipeline import HotPath, TextBank, clean_results, evaluate_new_batch, merge_results, split_ood_batch  # noqa: F401
 from .runtime import get_context  # noqa: F401
+from .train import LoraTrainer  # noqa: F401
 from .tta import TTAViews  # noqa: F401
 
 __version__ = "0.1.0"

@@ -22,7 +22,7 @@ IMG_F32, IMG_BF16, IMG_U8, IMG_PATCHES_BF16, IMG_PATCHES_F16 = 0, 1, 2, 3, 4
 PROJ_Q, PROJ_K, PROJ_V, PROJ_O = 0, 1, 2, 3
 SCORE_NAMES = ("logits", "cs", "cs1", "cs2", "cs3", "cs4", "cs5")
 SCORE_INDEX = {n: i for i, n in enumerate(SCORE_NAMES)}
-KC_COUNT = 15
+KC_COUNT = 19
 FILTER_BILINEAR, FILTER_BICUBIC = 0, 1
 # JCB_EPI_* (epilogue 3, the conv1 scatter, no longer exists)
 EPI_BIAS_16, EPI_BIAS_GELU_16, EPI_BIAS_RESID_F32, EPI_F32 = 0, 1, 2, 4
@@ -165,6 +165,14 @@ PROTOTYPES = {
     "jcb_im2col": (c_int, [c_void_p, c_void_p, c_int32, c_int64, c_int32, c_int32, c_int32, c_int32, c_void_p]),
     "jcb_tensor_map_cache_stats": (None, [POINTER(ctypes.c_uint64), POINTER(ctypes.c_uint64)]),
     "jcb_encode_image_dlpack": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int]),
+    "jcb_vit_train_set_lora": (c_int, [c_void_p, c_void_p, c_void_p]),
+    "jcb_vit_train_forward": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int, c_int, c_float, ctypes.c_uint64, c_int64,
+                                      c_void_p, POINTER(c_void_p)]),
+    "jcb_vit_train_forward_dlpack": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_float, ctypes.c_uint64, c_int64,
+                                             POINTER(c_void_p)]),
+    "jcb_vit_train_backward": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
+    "jcb_tape_release": (c_int, [c_void_p]),
+    "jcb_lora_dropout_mask": (c_int, [c_void_p, ctypes.c_uint64, c_int64, c_int, c_int, c_int64, c_int32, c_float, c_void_p]),
 }
 
 

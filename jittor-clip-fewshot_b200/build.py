@@ -18,7 +18,7 @@ PKG_DIR = Path(__file__).resolve().parent
 CSRC = PKG_DIR / "csrc"
 OBJ_DIR = CSRC / "build"
 LIB_PATH = PKG_DIR / "libjclip_b200.so"
-SOURCES = ["api.cu", "gemm.cu", "attention.cu", "attention_tc.cu", "rowwise.cu", "mta.cu", "head.cu", "tta.cu"]
+SOURCES = ["api.cu", "gemm.cu", "attention.cu", "attention_tc.cu", "rowwise.cu", "mta.cu", "head.cu", "tta.cu", "train.cu"]
 HEADERS = [CSRC / "kernels.h", CSRC / "ptx.cuh", PKG_DIR.parent / "include" / "jclip_b200.h"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

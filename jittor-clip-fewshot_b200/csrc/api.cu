@@ -268,8 +268,12 @@ struct TowerBase {
   std::vector<LayerDev> layers;
 };
 
+struct TrainState;
+void train_state_free(TrainState* ts);   // LoRA training section below
 struct jcb_vit : TowerBase {
   jcb_vit_config cfg{};
+  TrainState* train = nullptr;   // LoRA training: Wt copies and training adapter packing (jcb_vit_train_set_lora)
+  int live_tapes = 0;            // tapes of jcb_vit_train_forward not yet released
   int grid = 0, kpatch = 0;
   __nv_bfloat16* conv_w = nullptr;
   float *vpt = nullptr;
@@ -542,8 +546,9 @@ int tower_blocks(TowerBase* t, int64_t n, const TowerWs& w, int causal, bool cls
 
 // The image tower on `n` views resident on the device.  Schedule = VisionTransformer.execute
 // (reference jclip/model.py:104-126) with every elementwise op fused into a neighbouring kernel.
-int tower_forward(jcb_vit* v, const void* images, int dt, int64_t n, int apply_norm, const TowerWs& w,
-                  const int* slot_dev = nullptr) {
+// conv1 (im2col + GEMM), class token, positional embedding, ln_pre and layer 0's ln_1: w.tokens holds the residual
+// stream and w.ln_out the input of block 0's QKV projection on exit
+int tower_front(jcb_vit* v, const void* images, int dt, int64_t n, int apply_norm, const TowerWs& w) {
   jcb_ctx* ctx = v->ctx;
   cudaStream_t s = ctx->stream;
   const int W = v->cfg.width, T = v->tokens, GG = v->grid * v->grid, KP = v->kpatch;
@@ -566,6 +571,13 @@ int tower_forward(jcb_vit* v, const void* images, int dt, int64_t n, int apply_n
   LAUNCH_P(ctx, JCB_KC_EMBED_LN, 0, MW * (4 + 4 + 2), launch_embed_ln(w.tokens, n, T, W, v->cls, v->pos, v->vpt, v->cfg.vpt_tokens, v->ln_pre_g, v->ln_pre_b, v->layers[0].ln1_g,
                               v->layers[0].ln1_b, w.ln_out, s, v->layers[0].in_wf ? w.stats[0] : nullptr, (W + 255) / 256,
                               patch_out, w.shift[0], v->f16));
+  return JCB_OK;
+}
+
+int tower_forward(jcb_vit* v, const void* images, int dt, int64_t n, int apply_norm, const TowerWs& w,
+                  const int* slot_dev = nullptr) {
+  int rc = tower_front(v, images, dt, n, apply_norm, w);
+  if (rc) return rc;
   return tower_blocks(v, n, w, 0, /*cls_row0=*/true, slot_dev);   // the tail reads token row 0 only
 }
 
@@ -930,7 +942,7 @@ int jcb_ctx_profile_read(const jcb_ctx* ctx, int kernel_class, double* total_ms,
 const char* jcb_kernel_class_name(int kernel_class) {
   static const char* names[JCB_KC_COUNT] = {"im2col", "gemm_patch", "embed_ln", "gemm_qkv", "attention", "gemm_out",
                                             "layernorm", "gemm_fc1", "gemm_fc2", "tail", "mta", "head", "other", "tta_views",
-                                            "gemm_lora"};
+                                            "gemm_lora", "bwd_gemm", "bwd_attention", "bwd_rowwise", "lora_grad"};
   return kernel_class >= 0 && kernel_class < JCB_KC_COUNT ? names[kernel_class] : "?";
 }
 
@@ -970,6 +982,7 @@ int jcb_vit_destroy(jcb_vit* v) {
   cudaStreamSynchronize(v->ctx->stream);
   graphs_clear_fwd(v->ctx);      // captured pipelines point into this tower's weights
   if (v->arena) cudaFree(v->arena);
+  train_state_free(v->train);
   delete v;
   return JCB_OK;
 }
@@ -2046,6 +2059,7 @@ struct DLTensor {
 };
 struct DLManagedTensor { DLTensor dl_tensor; void* manager_ctx; void (*deleter)(DLManagedTensor*); };
 constexpr int kDLCUDA = 2, kDLUInt = 1, kDLFloat = 2, kDLBfloat = 4;
+int dl_unpack(jcb_vit* v, void* images_dlmanaged, void* out_dlmanaged, const void** images, int* dt_out, int64_t* n, float** out_ptr);
 bool dl_contiguous(const DLTensor& t) {
   if (!t.strides) return true;
   int64_t expect = 1;
@@ -2057,9 +2071,22 @@ bool dl_contiguous(const DLTensor& t) {
 }
 }  // namespace
 
+
 int jcb_encode_image_dlpack(jcb_vit* v, void* images_dlmanaged, void* out_dlmanaged, int apply_clip_norm, int normalize) {
   int rc = check_vit(v);
   if (rc) return rc;
+  const void* images;
+  int dt;
+  int64_t n;
+  float* out;
+  if ((rc = dl_unpack(v, images_dlmanaged, out_dlmanaged, &images, &dt, &n, &out))) return rc;
+  DeviceGuard g(v->ctx->device);
+  return encode_views(v, images, dt, false, n, apply_clip_norm, normalize, out, 0);
+}
+
+namespace {
+// the image batch and the embedding output of a DLPack call, validated
+int dl_unpack(jcb_vit* v, void* images_dlmanaged, void* out_dlmanaged, const void** images, int* dt_out, int64_t* n, float** out_ptr) {
   jcb_ctx* ctx = v->ctx;
   if (!images_dlmanaged || !out_dlmanaged) return fail(ctx, JCB_E_INVALID, "null DLManagedTensor");
   const DLTensor& in = static_cast<DLManagedTensor*>(images_dlmanaged)->dl_tensor;
@@ -2082,9 +2109,523 @@ int jcb_encode_image_dlpack(jcb_vit* v, void* images_dlmanaged, void* out_dlmana
   if (out.ndim != 2 || out.shape[0] != in.shape[0] || out.shape[1] != v->cfg.embed_dim || out.dtype.code != kDLFloat ||
       out.dtype.bits != 32 || !dl_contiguous(out))
     return fail(ctx, JCB_E_INVALID, "out must be contiguous float32 [n, %d]", v->cfg.embed_dim);
+  *images = static_cast<const uint8_t*>(in.data) + in.byte_offset;
+  *dt_out = dt;
+  *n = in.shape[0];
+  *out_ptr = reinterpret_cast<float*>(static_cast<uint8_t*>(out.data) + out.byte_offset);
+  return JCB_OK;
+}
+}  // namespace
+
+}  // extern "C"
+
+// ================================================================================================ LoRA training
+// Gradients of a scalar loss with respect to the image tower's LoRA adapters (include/jclip_b200.h "LoRA training").
+// Forward: the applied-mode schedule of tower_blocks (stand-alone LayerNorms, W x + b + s B (A dropout(x))) with the
+// tape written on the way.  Backward, per pass of views and per block in reverse: a 32-bit residual-gradient stream g;
+// the input-gradient GEMMs dX = dY W on the tcgen05 GEMM with bf16 Wt copies; the c_fc pre-activation recomputed from
+// the taped ln_2 input (one forward-sized GEMM instead of 8 bytes per hidden element on the tape); the LoRA parameter
+// gradients as deterministic split-row reductions.  The LoRA term of the input gradients cannot ride the GEMM's second
+// operand pair: q, k and v see different dropout masks, applied after the product (dropout_bwd_add).
+struct TrainLayer {
+  __nv_bfloat16 *in_wt = nullptr, *out_wt = nullptr, *fc_wt = nullptr, *proj_wt = nullptr;   // bf16 Wt [in, out]
+  __nv_bfloat16 *in_blk = nullptr;     // [128, 3W] forward type: U = [drop_q x | drop_k x | drop_v x] in_blk^T
+  __nv_bfloat16 *in_blk_t = nullptr;   // [3W, 64] bf16
+  __nv_bfloat16 *in_up_t = nullptr;    // [128, 3W] bf16: V = dY up_t^T = s dY B
+  __nv_bfloat16 *out_blk_t = nullptr;  // [W, 64] bf16
+  __nv_bfloat16 *out_up_t = nullptr;   // [128, W] bf16
+  LoraGroup gin, gout;                 // ranks / offsets / scalings of the adapters (pointers: last set_lora)
+};
+struct TrainState {
+  uint64_t gen = 0;          // the finalize generation the Wt copies were made for
+  bool lora_set = false;     // jcb_vit_train_set_lora ran since that finalize
+  void* arena = nullptr;
+  std::vector<TrainLayer> layers;
+  void* bws = nullptr;       // grow-only backward workspace
+  size_t bws_bytes = 0;
+};
+void train_state_free(TrainState* ts) {
+  if (!ts) return;
+  if (ts->arena) cudaFree(ts->arena);
+  if (ts->bws) cudaFree(ts->bws);
+  delete ts;
+}
+
+struct jcb_tape {
+  jcb_vit* vit = nullptr;
+  uint64_t gen = 0;
+  int64_t n = 0;             // views
+  int normalize = 0;
+  DropoutArgs drop;          // layer field unused
+  void* mem = nullptr;
+  // per block: [n T, W] fp32 residual at ln_1 / ln_2, q|k|v, attention output, U of in_proj / out_proj
+  std::vector<float*> res1, res2;
+  std::vector<__nv_bfloat16*> qkv, attn, u_in, u_out;
+  float* x0 = nullptr;       // [n, W] class-token rows of the last block's output
+};
+
+namespace {
+
+constexpr int64_t TRAIN_PASS_VIEWS = 1024;   // views per backward pass (workspace ~2.5 MB per ViT-B/32 view)
+
+int train_gemm(jcb_ctx* ctx, int cls, int f16, const __nv_bfloat16* A, int64_t lda, const __nv_bfloat16* B, int M, int N, int K,
+               const float* bias, int epi, void* out, int64_t ldo, const __nv_bfloat16* A2 = nullptr,
+               const __nv_bfloat16* B2 = nullptr) {
+  GemmArgs g;
+  g.A = A; g.B = B; g.lda = lda; g.ldb = K; g.M = M; g.N = N; g.K = K; g.f16 = f16;
+  g.bias = bias; g.epilogue = epi; g.out = out; g.ldo = ldo;
+  if (A2) { g.A2 = A2; g.B2 = B2; g.K2 = LORA_K2; g.lda2 = LORA_U_COLS; g.ldb2 = LORA_K2; }
+  const double bytes = 2.0 * M * K + 2.0 * N * K + (epi == EPI_F32 ? 4.0 : epi == EPI_BIAS_RESID_F32 ? 8.0 : 2.0) * M * N;
+  LAUNCH_P(ctx, cls, 2.0 * M * N * (K + (A2 ? LORA_K2 : 0)), bytes, launch_gemm(g, ctx->dev_status, ctx->num_sms, ctx->stream));
+  return JCB_OK;
+}
+
+// what every training entry point checks before it launches anything
+int train_check(jcb_vit* v) {
+  if (!v) return JCB_E_INVALID;
+  jcb_ctx* ctx = v->ctx;
+  if (!v->finalized) return fail(ctx, JCB_E_INVALID, "LoRA training: the tower is not finalized (jcb_vit_finalize)");
+  if (v->tokens > 64)
+    return fail(ctx, JCB_E_INVALID, "LoRA training supports towers of at most 64 tokens (this one has %d)", v->tokens);
+  if (!v->lora_applied) return fail(ctx, JCB_E_INVALID, "LoRA training needs a tower packed in JCB_LORA_APPLIED mode");
+  if (v->lora_slots != 1) return fail(ctx, JCB_E_INVALID, "LoRA training supports one adapter slot (the tower has %d)", v->lora_slots);
+  if (v->lora[0].empty()) return fail(ctx, JCB_E_INVALID, "LoRA training: the tower carries no adapter");
+  for (int li = 0; li < v->L; ++li) {   // finalize checked it in applied mode; restated for clarity of the contract
+    int r_qkv = 0, r_o = 0;
+    for (int p = 0; p < 4; ++p) {
+      auto it = v->lora[0].find(li * 4 + p);
+      if (it != v->lora[0].end()) (p < 3 ? r_qkv : r_o) += it->second.r;
+    }
+    if (r_qkv > LORA_K2 || r_o > LORA_K2)
+      return fail(ctx, JCB_E_INVALID, "LoRA training, layer %d: ranks of q, k, v sum to %d, r(o) = %d (max %d each)", li, r_qkv, r_o, LORA_K2);
+  }
+  return JCB_OK;
+}
+
+// the Wt copies (once per finalize) and the adapter layout of the training packing
+int train_prepare(jcb_vit* v) {
+  jcb_ctx* ctx = v->ctx;
+  if (v->train && v->train->gen == v->gen) return JCB_OK;
+  if (v->live_tapes) return fail(ctx, JCB_E_STATE, "LoRA training: re-finalized while a tape is alive");
+  CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+  train_state_free(v->train);
+  v->train = new TrainState();
+  TrainState* ts = v->train;
+  const size_t W = v->W, L = v->L;
+  const size_t per_layer = align_up(3 * W * W * 2) + align_up(W * W * 2) + 2 * align_up(4 * W * W * 2) + align_up(128 * 3 * W * 2) +
+                           align_up(3 * W * 64 * 2) + align_up(128 * 3 * W * 2) + align_up(W * 64 * 2) + align_up(128 * W * 2);
+  cudaError_t e = cudaMalloc(&ts->arena, per_layer * L);
+  if (e != cudaSuccess) return fail(ctx, JCB_E_NOMEM, "cudaMalloc(%zu) for the training weights failed: %s", per_layer * L, cudaGetErrorString(e));
+  float* tmp = nullptr;
+  e = cudaMalloc(&tmp, 4 * W * W * 4);
+  if (e != cudaSuccess) return fail(ctx, JCB_E_NOMEM, "cudaMalloc for packing failed: %s", cudaGetErrorString(e));
+  struct Free { float* p; ~Free() { cudaFree(p); } } free_tmp{tmp};
+  Bump b(ts->arena);
+  ts->layers.assign(L, TrainLayer());
+  auto wt = [&](int li, const char* key, int rows, int cols, __nv_bfloat16** dst) -> int {
+    const std::vector<float>& h = v->host[blk(v, li, key)];
+    *dst = b.take<__nv_bfloat16>(h.size());
+    CUDA_TRY(ctx, cudaMemcpyAsync(tmp, h.data(), h.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
+    LAUNCH(ctx, launch_transpose_cast(tmp, rows, cols, 0, *dst, ctx->stream));
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));   // tmp is reused
+    return JCB_OK;
+  };
+  int rc;
+  for (size_t li = 0; li < L; ++li) {
+    TrainLayer& T = ts->layers[li];
+    if ((rc = wt(li, "attn.in_proj_weight", 3 * W, W, &T.in_wt))) return rc;
+    if ((rc = wt(li, "attn.out_proj.weight", W, W, &T.out_wt))) return rc;
+    if ((rc = wt(li, "mlp.c_fc.weight", 4 * W, W, &T.fc_wt))) return rc;
+    if ((rc = wt(li, "mlp.c_proj.weight", W, 4 * W, &T.proj_wt))) return rc;
+    T.in_blk = b.take<__nv_bfloat16>(128 * 3 * W);
+    T.in_blk_t = b.take<__nv_bfloat16>(3 * W * 64);
+    T.in_up_t = b.take<__nv_bfloat16>(128 * 3 * W);
+    T.out_blk_t = b.take<__nv_bfloat16>(W * 64);
+    T.out_up_t = b.take<__nv_bfloat16>(128 * W);
+    T.gin.npj = 3;
+    T.gout.npj = 1;
+    int j0 = 0;
+    for (int p = 0; p < 4; ++p) {
+      auto it = v->lora[0].find(static_cast<int>(li) * 4 + p);
+      if (it == v->lora[0].end()) continue;
+      LoraGroup& G = p < 3 ? T.gin : T.gout;
+      const int q = p < 3 ? p : 0;
+      G.r[q] = it->second.r;
+      G.s[q] = it->second.scaling;
+      G.j0[q] = p < 3 ? j0 : 0;
+      G.n0[q] = static_cast<int>(q * W);
+      if (p < 3) j0 += it->second.r;   // the order up_lora_applied packs them in
+    }
+  }
+  ts->gen = v->gen;
+  return JCB_OK;
+}
+
+struct TapeLayer {
+  float *res1, *res2;
+  __nv_bfloat16 *qkv, *attn, *u_in, *u_out;
+};
+TapeLayer tape_layer(const jcb_tape* tp, int l, int64_t v0) {
+  const jcb_vit* v = tp->vit;
+  const int64_t r0 = v0 * v->tokens, W = v->W;
+  return {tp->res1[l] + r0 * W, tp->res2[l] + r0 * W, tp->qkv[l] + r0 * 3 * W, tp->attn[l] + r0 * W,
+          tp->u_in[l] + r0 * LORA_U_COLS, tp->u_out[l] + r0 * LORA_U_COLS};
+}
+
+// the blocks of views [v0, v0 + n) with the tape: tower_blocks' applied-mode loop plus dropout and the tape writes
+int train_blocks(jcb_vit* v, int64_t n, int64_t v0, const TowerWs& w, jcb_tape* tp) {
+  jcb_ctx* ctx = v->ctx;
+  cudaStream_t s = ctx->stream;
+  const int W = v->W, T = v->tokens, f16 = v->f16;
+  const int M = static_cast<int>(n * T);
+  const double MW = static_cast<double>(M) * W;
+  const int64_t row0 = v0 * T;
+  int rc;
+  for (int l = 0; l < v->L; ++l) {
+    const LayerDev& L = v->layers[l];
+    const TrainLayer& TL = v->train->layers[l];
+    const TapeLayer tl = tape_layer(tp, l, v0);
+    DropoutArgs d = tp->drop;
+    d.layer = l;
+    CUDA_TRY(ctx, cudaMemcpyAsync(tl.res1, w.tokens, MW * 4, cudaMemcpyDeviceToDevice, s));
+    const __nv_bfloat16* A2 = nullptr;
+    if (L.lin_slots) {
+      LAUNCH_P(ctx, JCB_KC_BWD_ROWWISE, 0, MW * 8, launch_dropout_fwd(w.ln_out, M, W, 3, JCB_PROJ_Q, d, row0, f16, w.big, s));
+      if ((rc = train_gemm(ctx, JCB_KC_GEMM_LORA, f16, w.big, 3 * W, TL.in_blk, M, LORA_U_COLS, 3 * W, nullptr, EPI_BIAS_BF16, tl.u_in,
+                           LORA_U_COLS))) return rc;
+      A2 = tl.u_in;
+    }
+    if ((rc = train_gemm(ctx, JCB_KC_GEMM_QKV, f16, w.ln_out, W, L.in_w, M, 3 * W, W, L.in_b, EPI_BIAS_BF16, tl.qkv, 3 * W, A2, L.lin_up)))
+      return rc;
+    LAUNCH_P(ctx, JCB_KC_ATTENTION, 4.0 * n * v->heads * T * T * 64, MW * (6 + 2),
+             launch_attention(tl.qkv, n, T, v->heads, tl.attn, s, 0, ctx->dev_status, ctx->num_sms, f16));
+    A2 = nullptr;
+    if (L.lout_slots) {
+      LAUNCH_P(ctx, JCB_KC_BWD_ROWWISE, 0, MW * 4, launch_dropout_fwd(tl.attn, M, W, 1, JCB_PROJ_O, d, row0, f16, w.big, s));
+      if ((rc = train_gemm(ctx, JCB_KC_GEMM_LORA, f16, w.big, W, L.lout_dn, M, LORA_U_COLS, W, nullptr, EPI_BIAS_BF16, tl.u_out,
+                           LORA_U_COLS))) return rc;
+      A2 = tl.u_out;
+    }
+    if ((rc = train_gemm(ctx, JCB_KC_GEMM_OUT, f16, tl.attn, W, L.out_w, M, W, W, L.out_b, EPI_BIAS_RESID_F32, w.tokens, W, A2, L.lout_up)))
+      return rc;
+    CUDA_TRY(ctx, cudaMemcpyAsync(tl.res2, w.tokens, MW * 4, cudaMemcpyDeviceToDevice, s));
+    LAUNCH_P(ctx, JCB_KC_LAYERNORM, 0, MW * (4 + 2), launch_layernorm(w.tokens, M, W, L.ln2_g, L.ln2_b, w.ln_out, s, f16));
+    if ((rc = train_gemm(ctx, JCB_KC_GEMM_FC1, f16, w.ln_out, W, L.fc_w, M, 4 * W, W, L.fc_b, EPI_BIAS_GELU_BF16, w.big, 4 * W))) return rc;
+    if ((rc = train_gemm(ctx, JCB_KC_GEMM_FC2, f16, w.big, 4 * W, L.proj_w, M, W, 4 * W, L.proj_b, EPI_BIAS_RESID_F32, w.tokens, W))) return rc;
+    if (l + 1 < v->L) {
+      const LayerDev& Nx = v->layers[l + 1];
+      LAUNCH_P(ctx, JCB_KC_LAYERNORM, 0, MW * (4 + 2), launch_layernorm(w.tokens, M, W, Nx.ln1_g, Nx.ln1_b, w.ln_out, s, f16));
+    }
+  }
+  return JCB_OK;
+}
+
+// the passes of a training forward, as encode_views runs them for device-resident input
+int train_forward_passes(jcb_vit* v, const void* images, int dt, int64_t n, int apply_norm, int normalize, float* out, jcb_tape* tp) {
+  jcb_ctx* ctx = v->ctx;
+  const int64_t T = v->tokens, W = v->W;
+  const int64_t chunk = balanced_chunk(n, views_bound(ctx, false, v->tokens));
+  int rc;
+  if ((rc = ws_reserve(ctx, tower_ws_bytes(v, chunk)))) return rc;
+  Bump wb(ctx->ws);
+  TowerWs w = tower_ws_carve(v, chunk, wb);
+  const size_t view_bytes = static_cast<size_t>(3) * v->cfg.resolution * v->cfg.resolution * img_elem_bytes(dt);
+  for (int64_t off = 0; off < n; off += chunk) {
+    const int64_t m = std::min(chunk, n - off);
+    if ((rc = tower_front(v, static_cast<const uint8_t*>(images) + off * view_bytes, dt, m, apply_norm, w))) return rc;
+    if ((rc = train_blocks(v, m, off, w, tp))) return rc;
+    CUDA_TRY(ctx, cudaMemcpy2DAsync(tp->x0 + off * W, W * 4, w.tokens, T * W * 4, W * 4, m, cudaMemcpyDeviceToDevice, ctx->stream));
+    LAUNCH_P(ctx, JCB_KC_TAIL, 2.0 * m * W * v->cfg.embed_dim, static_cast<double>(m) * (W + v->cfg.embed_dim) * 4,
+             launch_tail(w.tokens, m, v->tokens, v->cfg.width, v->ln_post_g, v->ln_post_b, v->proj, v->cfg.embed_dim, normalize,
+                         out + off * v->cfg.embed_dim, ctx->stream));
+  }
+  return JCB_OK;
+}
+
+int train_forward(jcb_vit* v, const void* images, int dt, int64_t n, int apply_norm, int normalize, float rate, uint64_t seed,
+                  int64_t step, float* out, jcb_tape** tape) {
+  int rc = train_check(v);
+  if (rc) return rc;
+  jcb_ctx* ctx = v->ctx;
+  if (!tape) return fail(ctx, JCB_E_INVALID, "null tape pointer");
+  *tape = nullptr;
+  if (!(rate >= 0.f && rate < 1.f)) return fail(ctx, JCB_E_INVALID, "dropout_rate %g outside [0, 1)", static_cast<double>(rate));
+  if (n < 1) return fail(ctx, JCB_E_INVALID, "LoRA training forward: n_views must be >= 1");
+  if (!images || !out) return fail(ctx, JCB_E_INVALID, "null image / output pointer");
+  if (dt < 0 || dt > JCB_IMG_PATCHES_F16) return fail(ctx, JCB_E_INVALID, "unknown image dtype %d", dt);
+  if (is_patches(dt) && (dt == JCB_IMG_PATCHES_F16) != (v->f16 != 0))
+    return fail(ctx, JCB_E_INVALID, "patch matrix type differs from the tower's operand type");
+  if (!v->train || v->train->gen != v->gen || !v->train->lora_set)
+    return fail(ctx, JCB_E_STATE, "LoRA training: call jcb_vit_train_set_lora after jcb_vit_finalize");
   DeviceGuard g(ctx->device);
-  return encode_views(v, static_cast<const uint8_t*>(in.data) + in.byte_offset, dt, false, in.shape[0], apply_clip_norm,
-                      normalize, reinterpret_cast<float*>(static_cast<uint8_t*>(out.data) + out.byte_offset), 0);
+  const int64_t T = v->tokens, W = v->W, L = v->L;
+  // tape: per block 2 fp32 residuals, q|k|v, attention output and two U (16-bit), plus the class-token rows
+  const size_t rows = static_cast<size_t>(n * T);
+  const size_t per_block = 2 * align_up(rows * W * 4) + align_up(rows * 3 * W * 2) + align_up(rows * W * 2) + 2 * align_up(rows * LORA_U_COLS * 2);
+  const size_t bytes = per_block * L + align_up(static_cast<size_t>(n) * W * 4);
+  jcb_tape* tp = new jcb_tape();
+  cudaError_t e = cudaMalloc(&tp->mem, bytes);
+  if (e != cudaSuccess) {
+    delete tp;
+    return fail(ctx, JCB_E_NOMEM, "cudaMalloc(%zu) for the LoRA training tape failed: %s", bytes, cudaGetErrorString(e));
+  }
+  tp->vit = v;
+  tp->gen = v->gen;
+  tp->n = n;
+  tp->normalize = normalize;
+  tp->drop.seed = seed;
+  tp->drop.step = step;
+  tp->drop.thr24 = static_cast<unsigned>(static_cast<double>(rate) * 16777216.0);
+  tp->drop.inv = 1.f / (1.f - rate);
+  Bump b(tp->mem);
+  for (int64_t l = 0; l < L; ++l) {
+    tp->res1.push_back(b.take<float>(rows * W));
+    tp->res2.push_back(b.take<float>(rows * W));
+    tp->qkv.push_back(b.take<__nv_bfloat16>(rows * 3 * W));
+    tp->attn.push_back(b.take<__nv_bfloat16>(rows * W));
+    tp->u_in.push_back(b.take<__nv_bfloat16>(rows * LORA_U_COLS));
+    tp->u_out.push_back(b.take<__nv_bfloat16>(rows * LORA_U_COLS));
+  }
+  tp->x0 = b.take<float>(static_cast<size_t>(n) * W);
+  ++v->live_tapes;
+  if ((rc = train_forward_passes(v, images, dt, n, apply_norm, normalize, out, tp))) {
+    jcb_tape_release(tp);   // a failed forward leaves no tape behind
+    return rc;
+  }
+  *tape = tp;
+  return JCB_OK;
+}
+
+// backward workspace of one pass of m views
+struct BwdWs {
+  float *g, *dxn, *do32, *big32;                       // big32: dH [M, 4W] / dXd [M, 3W]
+  __nv_bfloat16 *g16, *h16, *xn16, *dqkv16, *v16, *xd16;
+  float *partial;                                      // 128 chunks x the largest reduction (3W x 64)
+  float *acc;                                          // per layer: dB_in [3W, 64], dA_in [64, 3W], dB_o [W, 64], dA_o [64, W]
+};
+size_t acc_floats_per_layer(size_t W) { return 2 * 3 * W * 64 + 2 * W * 64; }
+size_t bwd_ws_bytes(size_t W, size_t T, int64_t m, size_t L) {
+  const size_t M = static_cast<size_t>(m) * T;
+  return 3 * align_up(M * W * 4) + align_up(M * 4 * W * 4) + align_up(M * W * 2) + align_up(M * 4 * W * 2) + align_up(M * W * 2) +
+         2 * align_up(M * 3 * W * 2) + align_up(M * LORA_U_COLS * 2) + align_up(128 * 3 * W * 64 * 4) +
+         align_up(L * acc_floats_per_layer(W) * 4);
+}
+
+int train_backward(jcb_tape* tp, const float* dfeat, float* const* dA, float* const* dB) {
+  if (!tp) return JCB_E_INVALID;
+  jcb_vit* v = tp->vit;
+  jcb_ctx* ctx = v->ctx;
+  int rc;
+  if (!dfeat || !dA || !dB) return fail(ctx, JCB_E_INVALID, "null dL/dfeatures or gradient array");
+  if (tp->gen != v->gen || !v->finalized) return fail(ctx, JCB_E_STATE, "the tower was re-packed after this tape's forward");
+  for (int li = 0; li < v->L; ++li)
+    for (int p = 0; p < 4; ++p) {
+      const bool has = v->lora[0].count(li * 4 + p) != 0;
+      if (has != (dA[li * 4 + p] != nullptr) || has != (dB[li * 4 + p] != nullptr))
+        return fail(ctx, JCB_E_INVALID, "gradient pointers of layer %d, projection %d: %s expected", li, p, has ? "non-NULL" : "NULL");
+    }
+  DeviceGuard dg(ctx->device);
+  cudaStream_t s = ctx->stream;
+  TrainState* ts = v->train;
+  const int W = v->W, T = v->tokens, f16 = v->f16, E = v->cfg.embed_dim, L = v->L;
+  const int64_t n = tp->n;
+  const int64_t chunk = balanced_chunk(n, std::min<int64_t>(TRAIN_PASS_VIEWS, ctx->chunk_views));
+  const size_t need = bwd_ws_bytes(W, T, chunk, L);
+  if (need > ts->bws_bytes) {
+    CUDA_TRY(ctx, cudaStreamSynchronize(s));
+    if (ts->bws) cudaFree(ts->bws);
+    ts->bws = nullptr;
+    ts->bws_bytes = 0;
+    cudaError_t e = cudaMalloc(&ts->bws, need);
+    if (e != cudaSuccess) return fail(ctx, JCB_E_NOMEM, "cudaMalloc(%zu) for the LoRA backward failed: %s", need, cudaGetErrorString(e));
+    ts->bws_bytes = need;
+  }
+  const size_t Mc = static_cast<size_t>(chunk) * T;
+  Bump b(ts->bws);
+  BwdWs w;
+  w.g = b.take<float>(Mc * W);
+  w.dxn = b.take<float>(Mc * W);
+  w.do32 = b.take<float>(Mc * W);
+  w.big32 = b.take<float>(Mc * 4 * W);
+  w.g16 = b.take<__nv_bfloat16>(Mc * W);
+  w.h16 = b.take<__nv_bfloat16>(Mc * 4 * W);
+  w.xn16 = b.take<__nv_bfloat16>(Mc * W);
+  w.dqkv16 = b.take<__nv_bfloat16>(Mc * 3 * W);
+  w.xd16 = b.take<__nv_bfloat16>(Mc * 3 * W);
+  w.v16 = b.take<__nv_bfloat16>(Mc * LORA_U_COLS);
+  w.partial = b.take<float>(128 * 3 * static_cast<size_t>(W) * 64);
+  w.acc = b.take<float>(L * acc_floats_per_layer(W));
+  const size_t accL = acc_floats_per_layer(W);
+  CUDA_TRY(ctx, cudaMemsetAsync(w.acc, 0, L * accL * 4, s));
+  const int ft = f16 ? TR_F16 : TR_BF16;
+  for (int64_t off = 0; off < n; off += chunk) {
+    const int64_t m = std::min(chunk, n - off);
+    const int M = static_cast<int>(m * T);
+    const double MW = static_cast<double>(M) * W;
+    const int64_t row0 = off * T;
+    CUDA_TRY(ctx, cudaMemsetAsync(w.g, 0, MW * 4, s));
+    LAUNCH_P(ctx, JCB_KC_BWD_ROWWISE, 4.0 * m * W * E, static_cast<double>(m) * (W + E) * 8,
+             launch_tail_bwd(tp->x0 + off * W, dfeat + off * E, m, W, E, v->ln_post_g, v->ln_post_b, v->proj, tp->normalize, T, w.g, s));
+    for (int l = L - 1; l >= 0; --l) {
+      const LayerDev& Ld = v->layers[l];
+      const TrainLayer& TL = ts->layers[l];
+      const TapeLayer tl = tape_layer(tp, l, off);
+      DropoutArgs d = tp->drop;
+      d.layer = l;
+      float* accBi = w.acc + l * accL;
+      float* accAi = accBi + 3 * W * 64;
+      float* accBo = accAi + 3 * W * 64;
+      float* accAo = accBo + W * 64;
+      // MLP: g -> dH = g c_proj -> QuickGELU' (pre-activation recomputed) -> dxn = dh c_fc -> ln_2 backward
+      LAUNCH_P(ctx, JCB_KC_BWD_ROWWISE, 0, MW * 6, launch_cast_bf16(w.g, w.g16, static_cast<int64_t>(MW), s, 0));
+      LAUNCH_P(ctx, JCB_KC_BWD_ROWWISE, 0, MW * 6, launch_layernorm(tl.res2, M, W, Ld.ln2_g, Ld.ln2_b, w.xn16, s, f16));
+      if ((rc = train_gemm(ctx, JCB_KC_BWD_GEMM, f16, w.xn16, W, Ld.fc_w, M, 4 * W, W, Ld.fc_b, EPI_BIAS_BF16, w.h16, 4 * W))) return rc;
+      if ((rc = train_gemm(ctx, JCB_KC_BWD_GEMM, 0, w.g16, W, TL.proj_wt, M, 4 * W, W, nullptr, EPI_F32, w.big32, 4 * W))) return rc;
+      LAUNCH_P(ctx, JCB_KC_BWD_ROWWISE, 0, MW * 4 * 8, launch_gelu_bwd(w.big32, w.h16, static_cast<int64_t>(MW) * 4, f16, w.h16, s));
+      if ((rc = train_gemm(ctx, JCB_KC_BWD_GEMM, 0, w.h16, 4 * W, TL.fc_wt, M, W, 4 * W, nullptr, EPI_F32, w.dxn, W))) return rc;
+      LAUNCH_P(ctx, JCB_KC_BWD_ROWWISE, 0, MW * 16, launch_ln_bwd(tl.res2, w.dxn, M, W, Ld.ln2_g, w.g, s));
+      // attention: dO = g out_proj (+ dropout_o(s (g B_o) A_o)), attention backward, dxn = dqkv in_proj (+ LoRA), ln_1 backward
+      LAUNCH_P(ctx, JCB_KC_BWD_ROWWISE, 0, MW * 6, launch_cast_bf16(w.g, w.g16, static_cast<int64_t>(MW), s, 0));
+      if ((rc = train_gemm(ctx, JCB_KC_BWD_GEMM, 0, w.g16, W, TL.out_wt, M, W, W, nullptr, EPI_F32, w.do32, W))) return rc;
+      if (Ld.lout_slots) {
+        if ((rc = train_gemm(ctx, JCB_KC_BWD_GEMM, 0, w.g16, W, TL.out_up_t, M, LORA_U_COLS, W, nullptr, EPI_BIAS_BF16, w.v16, LORA_U_COLS)))
+          return rc;
+        LAUNCH_P(ctx, JCB_KC_LORA_GRAD, 2.0 * M * W * 64, MW * 4, launch_xty_accumulate(w.g, TR_F32, W, tl.u_out, ft, LORA_U_COLS, M, W, 64, w.partial, accBo, s));
+        LAUNCH_P(ctx, JCB_KC_BWD_ROWWISE, 0, MW * 4, launch_dropout_fwd(tl.attn, M, W, 1, JCB_PROJ_O, d, row0, f16, w.xd16, s));
+        LAUNCH_P(ctx, JCB_KC_LORA_GRAD, 2.0 * M * W * 64, MW * 2, launch_xty_accumulate(w.v16, TR_BF16, LORA_U_COLS, w.xd16, ft, W, M, 64, W, w.partial, accAo, s));
+        if ((rc = train_gemm(ctx, JCB_KC_BWD_GEMM, 0, w.v16, LORA_U_COLS, TL.out_blk_t, M, W, LORA_K2, nullptr, EPI_F32, w.big32, W))) return rc;
+        LAUNCH_P(ctx, JCB_KC_BWD_ROWWISE, 0, MW * 12, launch_dropout_bwd_add(w.big32, M, W, 1, JCB_PROJ_O, d, row0, w.do32, s));
+      }
+      LAUNCH_P(ctx, JCB_KC_BWD_ATTENTION, 10.0 * m * v->heads * T * T * 64, MW * 12,
+               launch_attention_bwd(tl.qkv, w.do32, m, T, v->heads, f16, w.dqkv16, s));
+      if ((rc = train_gemm(ctx, JCB_KC_BWD_GEMM, 0, w.dqkv16, 3 * W, TL.in_wt, M, W, 3 * W, nullptr, EPI_F32, w.dxn, W))) return rc;
+      if (Ld.lin_slots) {
+        if ((rc = train_gemm(ctx, JCB_KC_BWD_GEMM, 0, w.dqkv16, 3 * W, TL.in_up_t, M, LORA_U_COLS, 3 * W, nullptr, EPI_BIAS_BF16, w.v16,
+                             LORA_U_COLS))) return rc;
+        LAUNCH_P(ctx, JCB_KC_LORA_GRAD, 2.0 * M * 3 * W * 64, MW * 6,
+                 launch_xty_accumulate(w.dqkv16, TR_BF16, 3 * W, tl.u_in, ft, LORA_U_COLS, M, 3 * W, 64, w.partial, accBi, s));
+        LAUNCH_P(ctx, JCB_KC_BWD_ROWWISE, 0, MW * 6, launch_layernorm(tl.res1, M, W, Ld.ln1_g, Ld.ln1_b, w.xn16, s, f16));
+        LAUNCH_P(ctx, JCB_KC_BWD_ROWWISE, 0, MW * 8, launch_dropout_fwd(w.xn16, M, W, 3, JCB_PROJ_Q, d, row0, f16, w.xd16, s));
+        LAUNCH_P(ctx, JCB_KC_LORA_GRAD, 2.0 * M * 3 * W * 64, MW * 6,
+                 launch_xty_accumulate(w.v16, TR_BF16, LORA_U_COLS, w.xd16, ft, 3 * W, M, 64, 3 * W, w.partial, accAi, s));
+        if ((rc = train_gemm(ctx, JCB_KC_BWD_GEMM, 0, w.v16, LORA_U_COLS, TL.in_blk_t, M, 3 * W, LORA_K2, nullptr, EPI_F32, w.big32, 3 * W)))
+          return rc;
+        LAUNCH_P(ctx, JCB_KC_BWD_ROWWISE, 0, MW * 20, launch_dropout_bwd_add(w.big32, M, W, 3, JCB_PROJ_Q, d, row0, w.dxn, s));
+      }
+      LAUNCH_P(ctx, JCB_KC_BWD_ROWWISE, 0, MW * 16, launch_ln_bwd(tl.res1, w.dxn, M, W, Ld.ln1_g, w.g, s));
+    }
+  }
+  // dB = s dY^T U, dA = (s dY B)^T dropout(x): the diagonal blocks of the accumulated products
+  for (int l = 0; l < L; ++l) {
+    const TrainLayer& TL = ts->layers[l];
+    const float* accBi = w.acc + l * accL;
+    const float* accAi = accBi + 3 * W * 64;
+    const float* accBo = accAi + 3 * W * 64;
+    const float* accAo = accBo + W * 64;
+    for (int p = 0; p < 4; ++p) {
+      if (!dA[l * 4 + p]) continue;
+      const LoraGroup& G = p < 3 ? TL.gin : TL.gout;
+      const int q = p < 3 ? p : 0;
+      LAUNCH_P(ctx, JCB_KC_LORA_GRAD, 0, 0, launch_extract(p < 3 ? accBi : accBo, 64, q * W, G.j0[q], W, G.r[q], G.s[q], dB[l * 4 + p], s));
+      LAUNCH_P(ctx, JCB_KC_LORA_GRAD, 0, 0, launch_extract(p < 3 ? accAi : accAo, p < 3 ? 3 * W : W, G.j0[q], q * W, G.r[q], W, 1.f,
+                                                           dA[l * 4 + p], s));
+    }
+  }
+  return JCB_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int jcb_vit_train_set_lora(jcb_vit* v, const float* const* A_dev, const float* const* B_dev) {
+  int rc = train_check(v);
+  if (rc) return rc;
+  jcb_ctx* ctx = v->ctx;
+  if (!A_dev || !B_dev) return fail(ctx, JCB_E_INVALID, "null adapter pointer array");
+  for (int li = 0; li < v->L; ++li)
+    for (int p = 0; p < 4; ++p) {
+      const bool has = v->lora[0].count(li * 4 + p) != 0;
+      if (has != (A_dev[li * 4 + p] != nullptr) || has != (B_dev[li * 4 + p] != nullptr))
+        return fail(ctx, JCB_E_INVALID, "adapter pointers of layer %d, projection %d: %s expected", li, p, has ? "non-NULL" : "NULL");
+    }
+  if (v->live_tapes) return fail(ctx, JCB_E_STATE, "jcb_vit_train_set_lora while a tape is alive (release it first)");
+  DeviceGuard g(ctx->device);
+  if ((rc = train_prepare(v))) return rc;
+  const int W = v->W;
+  cudaStream_t s = ctx->stream;
+  for (int li = 0; li < v->L; ++li) {
+    TrainLayer& TL = v->train->layers[li];
+    const LayerDev& Ld = v->layers[li];
+    for (int p = 0; p < 4; ++p) {
+      LoraGroup& G = p < 3 ? TL.gin : TL.gout;
+      const int q = p < 3 ? p : 0;
+      G.A[q] = A_dev[li * 4 + p];
+      G.B[q] = B_dev[li * 4 + p];
+    }
+    if (Ld.lin_slots) {
+      LAUNCH(ctx, launch_lora_pack(TL.gin, LP_DN, W, 3 * W, v->f16, Ld.lin_dn, s));
+      LAUNCH(ctx, launch_lora_pack(TL.gin, LP_UP, W, 3 * W, v->f16, Ld.lin_up, s));
+      LAUNCH(ctx, launch_lora_pack(TL.gin, LP_DN_BLK, W, 3 * W, v->f16, TL.in_blk, s));
+      LAUNCH(ctx, launch_lora_pack(TL.gin, LP_DN_T, W, 3 * W, v->f16, TL.in_blk_t, s));
+      LAUNCH(ctx, launch_lora_pack(TL.gin, LP_UP_T, W, 3 * W, v->f16, TL.in_up_t, s));
+    }
+    if (Ld.lout_slots) {
+      LAUNCH(ctx, launch_lora_pack(TL.gout, LP_DN, W, W, v->f16, Ld.lout_dn, s));
+      LAUNCH(ctx, launch_lora_pack(TL.gout, LP_UP, W, W, v->f16, Ld.lout_up, s));
+      LAUNCH(ctx, launch_lora_pack(TL.gout, LP_DN_T, W, W, v->f16, TL.out_blk_t, s));
+      LAUNCH(ctx, launch_lora_pack(TL.gout, LP_UP_T, W, W, v->f16, TL.out_up_t, s));
+    }
+  }
+  v->train->lora_set = true;
+  return JCB_OK;
+}
+
+int jcb_vit_train_forward(jcb_vit* v, const void* images_dev, int img_dtype, int64_t n_views, int apply_clip_norm, int normalize,
+                          float dropout_rate, uint64_t seed, int64_t step, float* out_dev, jcb_tape** tape) {
+  return train_forward(v, images_dev, img_dtype, n_views, apply_clip_norm, normalize, dropout_rate, seed, step, out_dev, tape);
+}
+
+int jcb_vit_train_forward_dlpack(jcb_vit* v, void* images_dlmanaged, void* out_dlmanaged, int apply_clip_norm, int normalize,
+                                 float dropout_rate, uint64_t seed, int64_t step, jcb_tape** tape) {
+  int rc = train_check(v);
+  if (rc) return rc;
+  const void* images;
+  int dt;
+  int64_t n;
+  float* out;
+  if ((rc = dl_unpack(v, images_dlmanaged, out_dlmanaged, &images, &dt, &n, &out))) return rc;
+  return train_forward(v, images, dt, n, apply_clip_norm, normalize, dropout_rate, seed, step, out, tape);
+}
+
+int jcb_vit_train_backward(jcb_tape* tape, const float* dfeat_dev, float* const* dA_dev, float* const* dB_dev) {
+  return train_backward(tape, dfeat_dev, dA_dev, dB_dev);
+}
+
+int jcb_tape_release(jcb_tape* tape) {
+  if (!tape) return JCB_OK;
+  jcb_ctx* ctx = tape->vit->ctx;
+  DeviceGuard g(ctx->device);
+  cudaStreamSynchronize(ctx->stream);   // the backward may still read it
+  if (tape->mem) cudaFree(tape->mem);
+  --tape->vit->live_tapes;
+  delete tape;
+  return JCB_OK;
+}
+
+int jcb_lora_dropout_mask(jcb_ctx* ctx, uint64_t seed, int64_t step, int layer, int proj, int64_t rows, int32_t cols, float rate,
+                          uint8_t* out_dev) {
+  if (!ctx) return JCB_E_INVALID;
+  if (!out_dev || rows < 0 || cols < 0 || proj < 0 || proj > 3 || layer < 0 || !(rate >= 0.f && rate < 1.f))
+    return fail(ctx, JCB_E_INVALID, "jcb_lora_dropout_mask: bad arguments");
+  DeviceGuard g(ctx->device);
+  DropoutArgs d;
+  d.seed = seed;
+  d.step = step;
+  d.layer = layer;
+  d.thr24 = static_cast<unsigned>(static_cast<double>(rate) * 16777216.0);
+  LAUNCH(ctx, launch_dropout_mask(d, proj, rows, cols, out_dev, ctx->stream));
+  return JCB_OK;
 }
 
 }  // extern "C"

@@ -134,6 +134,50 @@ cudaError_t launch_merge_lora_f32(float* W, const float* A, const float* B, int 
 cudaError_t launch_fold_ln(const float* W, const float* gamma, const float* beta, const float* bias, int N, int K,
                            __nv_bfloat16* Wf, float* S, float* c, cudaStream_t stream, int f16 = 0);
 
+// ---- LoRA training (train.cu): the backward pass of the image tower with respect to the adapters --------------
+// element types of launch_xty_accumulate's operands
+enum TrainElem : int { TR_BF16 = 0, TR_F16 = 1, TR_F32 = 2 };
+// training dropout of the LoRA branch input (one (layer, step) of a call; see dropout_keep in train.cu)
+struct DropoutArgs {
+  unsigned long long seed = 0;
+  long long step = 0;
+  int layer = 0;
+  unsigned thr24 = 0;   // floor(rate * 2^24): an element is kept iff the top 24 bits of its Philox word are >= thr24
+  float inv = 1.f;      // 1 / (1 - rate)
+};
+// the adapters of one projection group: npj = 3 (in_proj: q, k, v) or 1 (out_proj: o); A[p] == nullptr: no adapter
+struct LoraGroup {
+  int npj = 0;
+  const float* A[3] = {nullptr, nullptr, nullptr};   // [r, W] fp32, device
+  const float* B[3] = {nullptr, nullptr, nullptr};   // [W, r] fp32, device
+  int r[3] = {0, 0, 0};
+  int j0[3] = {0, 0, 0};    // first rank column of projection p in the packed intermediate U
+  int n0[3] = {0, 0, 0};    // first output row of projection p in the packed weight
+  float s[3] = {0.f, 0.f, 0.f};
+};
+enum LoraPackKind : int { LP_DN = 0, LP_UP = 1, LP_DN_BLK = 2, LP_DN_T = 3, LP_UP_T = 4 };
+cudaError_t launch_lora_pack(const LoraGroup& g, int kind, int W, int n_out, int f16, __nv_bfloat16* out, cudaStream_t s);
+cudaError_t launch_dropout_fwd(const __nv_bfloat16* x, int64_t M, int W, int npj, int proj0, const DropoutArgs& d, int64_t row0,
+                               int f16, __nv_bfloat16* xd, cudaStream_t s);
+cudaError_t launch_dropout_bwd_add(const float* dxd, int64_t M, int W, int npj, int proj0, const DropoutArgs& d, int64_t row0,
+                                   float* dx, cudaStream_t s);
+cudaError_t launch_dropout_mask(const DropoutArgs& d, int proj, int64_t rows, int cols, uint8_t* out, cudaStream_t s);
+cudaError_t launch_gelu_bwd(const float* dy, const __nv_bfloat16* h, int64_t n, int h_f16, __nv_bfloat16* dh, cudaStream_t s);
+cudaError_t launch_ln_bwd(const float* x, const float* dy, int64_t rows, int W, const float* gamma, float* g, cudaStream_t s);
+// qkv [n_views * T, 3W] 16-bit (forward), dout [n_views * T, W] fp32 -> dqkv [n_views * T, 3W] bf16; T <= 64
+cudaError_t launch_attention_bwd(const __nv_bfloat16* qkv, const float* dout, int64_t n_views, int T, int heads, int f16,
+                                 __nv_bfloat16* dqkv, cudaStream_t s);
+// grad row 0 of every view (stride T rows) := d(loss)/d(last block output) through ln_post, proj and the normalisation
+cudaError_t launch_tail_bwd(const float* x0, const float* dfeat, int64_t n_views, int W, int E, const float* g, const float* b,
+                            const float* proj, int normalize, int T, float* grad, cudaStream_t s);
+// acc[I, J] += X[:, :I]^T Y[:, :J] over M rows, split in at most 128 fixed row chunks summed in order (deterministic);
+// partial needs 128 * I * J floats
+int64_t xty_chunk_rows(int64_t M);
+cudaError_t launch_xty_accumulate(const void* X, int xt, int64_t ldx, const void* Y, int yt, int64_t ldy, int64_t M, int I, int J,
+                                  float* partial, float* acc, cudaStream_t s);
+cudaError_t launch_extract(const float* src, int64_t lds, int r0, int c0, int rows, int cols, float scale, float* out, cudaStream_t s);
+cudaError_t launch_transpose_cast(const float* src, int rows, int cols, int f16, __nv_bfloat16* dst, cudaStream_t s);
+
 // ---- MTA + head --------------------------------------------------------------------------------
 struct MtaParams {
   float lambda_y = 0.2f, lambda_q = 4.0f, th = 1e-6f, temperature = 1.0f;
