@@ -423,9 +423,9 @@ int jcb_pipeline_wait(jcb_ctx* ctx, int64_t ticket);
 /* ---------------------------------------------------------------- LoRA training -------------- */
 /* Gradients of a scalar loss with respect to the image tower's LoRA adapters A and B (slot 0), for the reference's
  * training step (lora_train_vlp.py:921-1024): a training forward that keeps a tape, then a backward that takes
- * dL/dfeatures.  Every other parameter is frozen.  Supported: towers of at most 64 tokens (ViT-B/32, plain or IVLP),
- * packed in JCB_LORA_APPLIED mode with one slot and at least one adapter (q, k, v, o on any blocks; per block the
- * ranks of q, k, v sum to at most 64 and r(o) <= 64).  Anything else returns JCB_E_INVALID before any launch, outputs
+ * dL/dfeatures.  Every other parameter is frozen.  Supported: towers of at most 256 tokens (ViT-B/32 and ViT-B/16,
+ * plain or IVLP), packed in JCB_LORA_APPLIED mode with one slot and at least one adapter (q, k, v, o on any blocks; per
+ * block the ranks of q, k, v sum to at most 64 and r(o) <= 64).  Anything else returns JCB_E_INVALID before any launch, outputs
  * untouched (also for a tower that is not finalized).
  *
  * Training dropout on the LoRA branch input (reference LoRALayer, test.py:291-297): inverted dropout with an
@@ -441,8 +441,8 @@ typedef struct jcb_tape jcb_tape;
 int jcb_vit_train_set_lora(jcb_vit* vit, const float* const* A_dev, const float* const* B_dev);
 /* jcb_encode_image (applied-mode schedule) that also records what the backward needs in a new tape *tape.  dropout_rate
  * in [0, 1); 0 runs the LoRA branch on its undropped input.  out_dev [n_views, embed_dim] fp32.  The tape is sized for
- * this call (about 0.64 MB per view per block for ViT-B/32, computed from shapes) and owned by the caller until
- * jcb_tape_release. */
+ * this call (about 0.64 MB per view per block for ViT-B/32 and 2.5 MB for ViT-B/16, computed from shapes) and owned by
+ * the caller until jcb_tape_release. */
 int jcb_vit_train_forward(jcb_vit* vit, const void* images_dev, int img_dtype, int64_t n_views, int apply_clip_norm,
                           int normalize, float dropout_rate, uint64_t seed, int64_t step, float* out_dev, jcb_tape** tape);
 /* The same with DLPack tensors (borrowed, as jcb_encode_image_dlpack). */
@@ -510,6 +510,11 @@ int jcb_im2col(jcb_ctx* ctx, const void* images_dev, int32_t img_dtype, int64_t 
  * mask, tokens <= 128 with it (JCB_E_INVALID otherwise) */
 int jcb_attention(jcb_ctx* ctx, const void* qkv16_dev, int64_t n_views, int32_t tokens, int32_t heads, int32_t causal,
                   int32_t operand_type, void* out16_dev);
+/* The backward of jcb_attention without the mask, as the LoRA training backward runs it: from the forward's qkv16_dev
+ * [n_views * tokens, 3 * 64 * heads] (operand_type) and dout_dev = dL/d(out) [n_views * tokens, 64 * heads] fp32, writes
+ * dqkv_bf16_dev = dL/d(q | k | v) [n_views * tokens, 3 * 64 * heads] bf16; 1 <= tokens <= 256 (JCB_E_INVALID otherwise) */
+int jcb_attention_bwd(jcb_ctx* ctx, const void* qkv16_dev, const float* dout_dev, int64_t n_views, int32_t tokens,
+                      int32_t heads, int32_t operand_type, void* dqkv_bf16_dev);
 /* hits / misses of the process-wide cache of encoded TMA tensor maps (one entry per (pointer, shape) launched) */
 void jcb_tensor_map_cache_stats(uint64_t* hits, uint64_t* misses);
 

@@ -162,6 +162,7 @@ PROTOTYPES = {
                             c_void_p, c_void_p]),
     "jcb_layernorm": (c_int, [c_void_p, c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_int32, c_void_p]),
     "jcb_attention": (c_int, [c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32, c_int32, c_void_p]),
+    "jcb_attention_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32, c_void_p]),
     "jcb_im2col": (c_int, [c_void_p, c_void_p, c_int32, c_int64, c_int32, c_int32, c_int32, c_int32, c_void_p]),
     "jcb_tensor_map_cache_stats": (None, [POINTER(ctypes.c_uint64), POINTER(ctypes.c_uint64)]),
     "jcb_encode_image_dlpack": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int]),

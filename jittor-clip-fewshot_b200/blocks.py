@@ -85,6 +85,15 @@ def attention(qkv, n_views, tokens, heads, out, causal=False, sync=True):
         ctx.sync()
 
 
+def attention_bwd(qkv, dout, n_views, tokens, heads, dqkv, sync=True):
+    """dqkv [n_views * tokens, 3 * 64 * heads] bf16 = dL/d(q | k | v) of `attention` (no mask) for dout = dL/d(out) fp32."""
+    ctx = _ctx(qkv)
+    check(ctx.lib.jcb_attention_bwd(ctx.handle, ptr(qkv), ptr(dout), n_views, tokens, heads, operand_code(qkv.dtype),
+                                    ptr(dqkv)), ctx.handle)
+    if sync:
+        ctx.sync()
+
+
 def mta_debug(feats, text, params=None):
     """jcb_mta_debug on feats [I, V, D] fp32 and text [D, C] fp32 (CUDA): the modes [I, D] and logits [I, C] of jcb_mta
     with the solver's state -- bandwidths [I, V], final inlierness weights y [I, V], affinity [I, V, V].  `params`: dict

@@ -2047,6 +2047,19 @@ int jcb_attention(jcb_ctx* ctx, const void* qkv, int64_t n_views, int32_t tokens
   return JCB_OK;
 }
 
+int jcb_attention_bwd(jcb_ctx* ctx, const void* qkv, const float* dout, int64_t n_views, int32_t tokens, int32_t heads,
+                      int32_t operand_type, void* dqkv) {
+  if (!ctx) return JCB_E_INVALID;
+  if (!qkv || !dout || !dqkv) return fail(ctx, JCB_E_INVALID, "jcb_attention_bwd: null pointer");
+  if (n_views < 0 || tokens < 1 || tokens > 256 || heads < 1)
+    return fail(ctx, JCB_E_INVALID, "jcb_attention_bwd: %d tokens, %d heads (1..256 tokens)", tokens, heads);
+  DeviceGuard g(ctx->device);
+  LAUNCH(ctx, launch_attention_bwd(static_cast<const __nv_bfloat16*>(qkv), dout, n_views, tokens, heads,
+                                   operand_type == JCB_OPERAND_F16, static_cast<__nv_bfloat16*>(dqkv), ctx->stream,
+                                   ctx->dev_status));
+  return JCB_OK;
+}
+
 void jcb_tensor_map_cache_stats(uint64_t* hits, uint64_t* misses) { tmap_cache_stats(hits, misses); }
 
 // ------------------------------------------------------------------------------------------------
@@ -2166,7 +2179,9 @@ struct jcb_tape {
 
 namespace {
 
-constexpr int64_t TRAIN_PASS_VIEWS = 1024;   // views per backward pass (workspace ~2.5 MB per ViT-B/32 view)
+// views per backward pass for towers of up to 64 tokens (workspace ~2.5 MB per ViT-B/32 view); a longer tower runs
+// proportionally fewer (token_rows_bound), so a pass holds about the same number of token rows
+constexpr int64_t TRAIN_PASS_VIEWS = 1024;
 
 int train_gemm(jcb_ctx* ctx, int cls, int f16, const __nv_bfloat16* A, int64_t lda, const __nv_bfloat16* B, int M, int N, int K,
                const float* bias, int epi, void* out, int64_t ldo, const __nv_bfloat16* A2 = nullptr,
@@ -2185,8 +2200,8 @@ int train_check(jcb_vit* v) {
   if (!v) return JCB_E_INVALID;
   jcb_ctx* ctx = v->ctx;
   if (!v->finalized) return fail(ctx, JCB_E_INVALID, "LoRA training: the tower is not finalized (jcb_vit_finalize)");
-  if (v->tokens > 64)
-    return fail(ctx, JCB_E_INVALID, "LoRA training supports towers of at most 64 tokens (this one has %d)", v->tokens);
+  if (v->tokens > 256)
+    return fail(ctx, JCB_E_INVALID, "LoRA training supports towers of at most 256 tokens (this one has %d)", v->tokens);
   if (!v->lora_applied) return fail(ctx, JCB_E_INVALID, "LoRA training needs a tower packed in JCB_LORA_APPLIED mode");
   if (v->lora_slots != 1) return fail(ctx, JCB_E_INVALID, "LoRA training supports one adapter slot (the tower has %d)", v->lora_slots);
   if (v->lora[0].empty()) return fail(ctx, JCB_E_INVALID, "LoRA training: the tower carries no adapter");
@@ -2429,7 +2444,7 @@ int train_backward(jcb_tape* tp, const float* dfeat, float* const* dA, float* co
   TrainState* ts = v->train;
   const int W = v->W, T = v->tokens, f16 = v->f16, E = v->cfg.embed_dim, L = v->L;
   const int64_t n = tp->n;
-  const int64_t chunk = balanced_chunk(n, std::min<int64_t>(TRAIN_PASS_VIEWS, ctx->chunk_views));
+  const int64_t chunk = balanced_chunk(n, token_rows_bound(std::min<int64_t>(TRAIN_PASS_VIEWS, ctx->chunk_views), T));
   const size_t need = bwd_ws_bytes(W, T, chunk, L);
   if (need > ts->bws_bytes) {
     CUDA_TRY(ctx, cudaStreamSynchronize(s));
@@ -2497,7 +2512,7 @@ int train_backward(jcb_tape* tp, const float* dfeat, float* const* dA, float* co
         LAUNCH_P(ctx, JCB_KC_BWD_ROWWISE, 0, MW * 12, launch_dropout_bwd_add(w.big32, M, W, 1, JCB_PROJ_O, d, row0, w.do32, s));
       }
       LAUNCH_P(ctx, JCB_KC_BWD_ATTENTION, 10.0 * m * v->heads * T * T * 64, MW * 12,
-               launch_attention_bwd(tl.qkv, w.do32, m, T, v->heads, f16, w.dqkv16, s));
+               launch_attention_bwd(tl.qkv, w.do32, m, T, v->heads, f16, w.dqkv16, s, ctx->dev_status));
       if ((rc = train_gemm(ctx, JCB_KC_BWD_GEMM, 0, w.dqkv16, 3 * W, TL.in_wt, M, W, 3 * W, nullptr, EPI_F32, w.dxn, W))) return rc;
       if (Ld.lin_slots) {
         if ((rc = train_gemm(ctx, JCB_KC_BWD_GEMM, 0, w.dqkv16, 3 * W, TL.in_up_t, M, LORA_U_COLS, 3 * W, nullptr, EPI_BIAS_BF16, w.v16,

@@ -534,9 +534,6 @@ attention_tcgen05_long_kernel(const __grid_constant__ CUtensorMap tmQKV, const _
   }
 }
 
-// [n_seq, T, blocks, 64] 16-bit elements as a 4-D tensor (d, block, token, sequence); boxes of 64 x 1 x 64 x 1 = one
-// head's [64 tokens][64] tile.  The token dimension is T long, so the rows T.. of a box are out of bounds: zero on
-// load, dropped on store.  Encoded once per (pointer, shape) and cached (same reason as gemm.cu's cache).
 struct HeadsKey {
   const void* base; uint64_t n_seq, T, blocks; int f16;
   bool operator<(const HeadsKey& o) const {
@@ -550,6 +547,12 @@ struct HeadsKey {
 std::mutex g_heads_mu;
 std::map<HeadsKey, CUtensorMap> g_heads_cache;
 
+}  // namespace
+
+// [n_seq, T, blocks, 64] 16-bit elements as a 4-D tensor (d, block, token, sequence); boxes of 64 x 1 x 64 x 1 = one
+// head's [64 tokens][64] tile.  The token dimension is T long, so the rows T.. of a box are out of bounds: zero on
+// load, dropped on store.  Encoded once per (pointer, shape) and cached (same reason as gemm.cu's cache).  Also used by
+// the attention backward (train.cu).
 bool make_tmap_heads(CUtensorMap* tm, const void* base, uint64_t n_seq, uint64_t T, uint64_t blocks, int f16) {
   const HeadsKey key{base, n_seq, T, blocks, f16};
   {
@@ -574,6 +577,8 @@ bool make_tmap_heads(CUtensorMap* tm, const void* base, uint64_t n_seq, uint64_t
   g_heads_cache.emplace(key, *tm);
   return true;
 }
+
+namespace {
 
 template <int TCT, int MODE>
 cudaError_t launch_atc(const CUtensorMap& tmQKV, const CUtensorMap& tmOut, const AtcDev& p, int f16, int num_sms,

@@ -164,9 +164,10 @@ cudaError_t launch_dropout_bwd_add(const float* dxd, int64_t M, int W, int npj, 
 cudaError_t launch_dropout_mask(const DropoutArgs& d, int proj, int64_t rows, int cols, uint8_t* out, cudaStream_t s);
 cudaError_t launch_gelu_bwd(const float* dy, const __nv_bfloat16* h, int64_t n, int h_f16, __nv_bfloat16* dh, cudaStream_t s);
 cudaError_t launch_ln_bwd(const float* x, const float* dy, int64_t rows, int W, const float* gamma, float* g, cudaStream_t s);
-// qkv [n_views * T, 3W] 16-bit (forward), dout [n_views * T, W] fp32 -> dqkv [n_views * T, 3W] bf16; T <= 64
+// qkv [n_views * T, 3W] 16-bit (forward), dout [n_views * T, W] fp32 -> dqkv [n_views * T, 3W] bf16; T <= 64 on the
+// FFMA kernel, 65 <= T <= 256 on the tcgen05 kernel (which reports pipeline timeouts in dev_status)
 cudaError_t launch_attention_bwd(const __nv_bfloat16* qkv, const float* dout, int64_t n_views, int T, int heads, int f16,
-                                 __nv_bfloat16* dqkv, cudaStream_t s);
+                                 __nv_bfloat16* dqkv, cudaStream_t s, int* dev_status);
 // grad row 0 of every view (stride T rows) := d(loss)/d(last block output) through ln_post, proj and the normalisation
 cudaError_t launch_tail_bwd(const float* x0, const float* dfeat, int64_t n_views, int W, int E, const float* g, const float* b,
                             const float* proj, int normalize, int T, float* grad, cudaStream_t s);

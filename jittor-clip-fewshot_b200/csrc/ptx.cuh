@@ -180,8 +180,11 @@ __host__ __device__ constexpr uint32_t umma_idesc_bf16_f32(int m, int n) {
 }
 // The same with the 16-bit operand type chosen by the caller: kind::f16 multiplies fp16 (format 0) and bf16 (format 1)
 // operands at the same rate, so the operand type is a property of the data, not of the kernel.
-__host__ __device__ constexpr uint32_t umma_idesc_f32acc(bool f16, int m, int n, bool b_mn_major = false) {
-  return (1u << 4) | (f16 ? 0u : ((1u << 7) | (1u << 10))) | (b_mn_major ? (1u << 16) : 0u) |
+// a_mn_major (bit 15): A is MN-major, i.e. the product takes the transpose of a K-major-stored matrix.
+__host__ __device__ constexpr uint32_t umma_idesc_f32acc(bool f16, int m, int n, bool b_mn_major = false,
+                                                         bool a_mn_major = false) {
+  return (1u << 4) | (f16 ? 0u : ((1u << 7) | (1u << 10))) | (a_mn_major ? (1u << 15) : 0u) |
+         (b_mn_major ? (1u << 16) : 0u) |
          (static_cast<uint32_t>(n >> 3) << 17) | (static_cast<uint32_t>(m >> 4) << 24);
 }
 // D[tmem] (+)= A[smem] * B[smem]^T ; issued by ONE thread for the whole CTA.
@@ -224,12 +227,13 @@ __device__ __forceinline__ void tmem_st_32x32b_x32(uint32_t taddr, const uint32_
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 // Shared-memory matrix descriptor of an MN-major operand tile (the MN dimension is the contiguous one) written
 // by TMA with 128-byte swizzle: rows = K index, 128 B (64 bf16 of MN) per row, 8-row groups 1024 B apart (SBO).
-// One 64-element MN atom only, so the leading byte offset (stride between MN atoms) is never used.
+// The leading byte offset `lbo` is the stride between 64-element MN atoms; it matters only for an MN extent over 64
+// (the attention backward's M = 128 transposed operands).
 // Advancing K by 16 = two 8-row groups adds 2048 B to the start address.
-__device__ __forceinline__ uint64_t umma_desc_sw128_mn(uint32_t smem_addr) {
+__device__ __forceinline__ uint64_t umma_desc_sw128_mn(uint32_t smem_addr, uint32_t lbo = 1024) {
   uint64_t d = 0;
   d |= static_cast<uint64_t>((smem_addr & 0x3FFFFu) >> 4);
-  d |= static_cast<uint64_t>(1024 >> 4) << 16;
+  d |= static_cast<uint64_t>((lbo >> 4) & 0x3FFFu) << 16;
   d |= static_cast<uint64_t>(1024 >> 4) << 32;
   d |= static_cast<uint64_t>(1) << 46;
   d |= static_cast<uint64_t>(2) << 61;

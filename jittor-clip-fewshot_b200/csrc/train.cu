@@ -5,9 +5,16 @@
 #include <cuda_fp16.h>
 #include <curand_philox4x32_x.h>
 
+#include <cudaTypedefs.h>
+
 #include "kernels.h"
+#include "ptx.cuh"
 
 namespace jcb {
+
+void* gemm_encode_tiled_fn();   // gemm.cu
+bool make_tmap_heads(CUtensorMap* tm, const void* base, uint64_t n_seq, uint64_t T, uint64_t blocks, int f16);   // attention_tc.cu
+
 namespace {
 
 // 16-bit element of type t (TR_BF16 / TR_F16) or fp32 (TR_F32) at p[i]
@@ -199,6 +206,390 @@ __global__ void __launch_bounds__(AB_THREADS) attention_bwd_kernel(const uint16_
     }
     dqkv[(row0 + t) * 3 * W + h * 64 + d] = to16(aq, false);
     dqkv[(row0 + t) * 3 * W + W + h * 64 + d] = to16(ak, false);
+  }
+}
+
+// Attention backward of one (view, head) for 65 <= T <= 256, head dim 64, no mask, on the 5th-generation tensor cores:
+// the same contract as attention_bwd_kernel, every product a tcgen05.mma with fp32 accumulators in TMEM.
+//
+//   CTA = one (view, head), 128 threads; thread = query row = TMEM lane.  Thread 0 issues the TMA copies and the MMAs;
+//   the phases below are separated by mbarriers (TMA bytes, MMA commits) and __syncthreads.
+//   shared   K, V       resident, ceil(T / 64) swizzled [64 tokens][64] boxes each (the attention_tc.cu layout)   64 KB
+//            Q, dO      the current 128-row query tile (dO: bf16, converted from fp32 in shared memory)            32 KB
+//            P / dS     [128 queries][256 keys] 16-bit as four swizzled [128][64] sub-tiles; dS overwrites P   64 KB
+//            staging    the query tile's fp32 dO (two TMA boxes of [128 tokens][32]), then dQ's bf16 output       32 KB
+//   TMEM     dV, dK     [256 keys][64] each, accumulated over the query tiles                          columns 0..255
+//            S, dP, dQ  in turn in columns 256..511
+//   per query tile qt (one or two):  S = Q K^T -> exact two-pass softmax (row max, then sum) -> P in shared memory;
+//            dP = dO V^T, dV += P^T dO -> D = rowsum(P dP), dS = P (dP - D) / 8 in shared memory;
+//            dQ = dS K -> TMA store, dK += dS^T Q.  After the last tile dK and dV are stored from TMEM.
+//   K is centred (its mean over the T keys subtracted) once it lands: see the comment at that step.
+//   P^T and dS^T are the same shared tiles read as MN-major A operands (two 64-key atoms 16 KB apart).  Boxes wholly
+//   past T are neither loaded nor multiplied; rows of a tile past T get P = dS = 0 and their outputs are clipped.
+//
+// Operand types: kind::f16 multiplies operands of one type, and dO and dS are bf16 (as in the backward GEMMs), so an fp16
+// tower's Q, K and V tiles are converted to bf16 in shared memory after they land.  Their rounding is then bf16's,
+// the same as a bf16 tower's (within the gradient bounds of tests/test_gpu_lora_train_b16.py).
+constexpr int BT_TILE = 64 * 64 * 2;                 // one [64 tokens][64] 16-bit box: 8 KB
+constexpr int BT_K = 0, BT_V = 4 * BT_TILE, BT_Q = 8 * BT_TILE, BT_DO = 10 * BT_TILE, BT_P = 12 * BT_TILE;
+constexpr int BT_P_SUB = 2 * BT_TILE;                // one [128 queries][64 keys] sub-tile of P / dS: 16 KB
+constexpr int BT_ST = BT_P + 4 * BT_P_SUB;           // staging: 32 KB
+constexpr int BT_BARS = BT_ST + 4 * BT_TILE;
+constexpr int BT_KMEAN = BT_BARS + 64;               // [64] fp32 mean key
+constexpr int BT_SMEM = BT_KMEAN + 256;              // 196928 B: one CTA per SM
+constexpr int BT_THREADS = 128;
+constexpr uint32_t BT_DV_COL = 0, BT_DK_COL = 128, BT_S_COL = 256, BT_TMEM_COLS = 512;
+
+struct AbtDev {
+  int heads;
+  int T;
+  int f16;
+  int* status;
+};
+
+// 8 16-bit values of the tower's type (fp16) -> bf16, in place
+__device__ __forceinline__ void f16_to_bf16_x8(uint4* p) {
+  uint4 v = *p;
+  uint32_t* w = reinterpret_cast<uint32_t*>(&v);
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const float2 f = unpack_h2<true>(w[i]);
+    w[i] = pack_bf16x2(f.x, f.y);
+  }
+  *p = v;
+}
+
+__global__ void __launch_bounds__(BT_THREADS, 1)
+attention_bwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant__ CUtensorMap tmDO,
+                             const __grid_constant__ CUtensorMap tmOut, const AbtDev p) {
+  extern __shared__ __align__(1024) uint8_t bt_smem[];
+  uint64_t* bars = reinterpret_cast<uint64_t*>(bt_smem + BT_BARS);
+  uint64_t* kv_full = bars;       // K, V landed
+  uint64_t* q_full = bars + 1;    // Q, dO of the query tile landed
+  uint64_t* mma_done = bars + 2;  // every MMA issued so far completed
+  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 3);
+
+  const int tid = threadIdx.x;
+  const int warp = tid >> 5;
+  const int T = p.T;
+  const int h = static_cast<int>(blockIdx.x % p.heads);
+  const int seq = static_cast<int>(blockIdx.x / p.heads);
+  const int nkb = (T + 63) >> 6;   // 64-key boxes holding valid keys: 2..4
+  const int nqt = (T + 127) >> 7;  // 128-row query (and key) tiles: 1 or 2
+  const uint32_t sbase = smem_u32(bt_smem);
+
+  if (tid == 0) {
+    if ((sbase & 1023u) != 0u) atomicCAS(p.status, 0, JCB_DEV_SMEM_ALIGN);
+    tma_prefetch_desc(&tmQKV);
+    tma_prefetch_desc(&tmDO);
+    tma_prefetch_desc(&tmOut);
+    mbar_init(kv_full, 1);
+    mbar_init(q_full, 1);
+    mbar_init(mma_done, 1);
+    fence_mbar_init();
+    fence_proxy_async_smem();
+  }
+  if (warp == 0) {
+    tmem_alloc(tmem_ptr_smem, BT_TMEM_COLS);
+    tmem_relinquish();
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(tmem_ptr_smem);
+  const uint32_t lane_base = tmem_base + (static_cast<uint32_t>(warp * 32) << 16);
+
+  if (tid == 0) {
+    mbar_arrive_expect_tx(kv_full, static_cast<uint32_t>(2 * nkb * BT_TILE));
+    // coordinates: (d, 64-wide column block of the [T, 3W] row, token, sequence); blocks: q | k | v heads
+    for (int b = 0; b < nkb; ++b) {
+      tma_load_4d(bt_smem + BT_K + b * BT_TILE, &tmQKV, kv_full, 0, p.heads + h, 64 * b, seq);
+      tma_load_4d(bt_smem + BT_V + b * BT_TILE, &tmQKV, kv_full, 0, 2 * p.heads + h, 64 * b, seq);
+    }
+  }
+  // every thread waits; a timeout anywhere ends the work of the whole CTA
+  uint32_t mph = 0;
+  auto wait_all = [&](uint64_t* bar, uint32_t parity) {
+    const bool ok = mbar_wait(bar, parity, p.status, JCB_DEV_TIMEOUT_EPILOGUE);
+    return __syncthreads_and(ok) != 0;
+  };
+  auto commit_wait = [&]() {
+    if (tid == 0) umma_commit(mma_done);
+    const bool ok = wait_all(mma_done, mph);
+    mph ^= 1u;
+    tc_fence_after();
+    return ok;
+  };
+  // 16-byte chunk j (8 elements, columns 8j..8j+7) of row r of a swizzled [rows][64] 16-bit tile at `tile`
+  auto chunk = [](uint8_t* tile, int r, int j) {
+    return reinterpret_cast<uint4*>(tile + (r >> 6) * BT_TILE + (r & 63) * 128 + ((j ^ (r & 7)) << 4));
+  };
+  const float scale_log2 = 0.125f * 1.4426950408889634f;   // 1/sqrt(64) * log2(e)
+  const uint32_t idesc_s = umma_idesc_f32acc(false, 128, 64 * nkb);                           // S, dP
+  constexpr uint32_t idesc_q = umma_idesc_f32acc(false, 128, 64, /*b_mn_major=*/true);        // dQ
+  constexpr uint32_t idesc_t = umma_idesc_f32acc(false, 128, 64, true, /*a_mn_major=*/true);  // dV, dK
+  bool ok = true;
+
+  for (int qt = 0; qt < nqt && ok; ++qt) {
+    const int q0 = 128 * qt;
+    const int nq = q0 + 64 < T ? 2 : 1;   // Q boxes holding valid rows
+    const int r = q0 + tid;               // this thread's query token
+    if (tid == 0) {
+      bulk_wait_read<0>();   // the previous tile's dQ store has read the staging
+      mbar_arrive_expect_tx(q_full, static_cast<uint32_t>(nq * BT_TILE + 4 * BT_TILE));
+      for (int b = 0; b < nq; ++b) tma_load_4d(bt_smem + BT_Q + b * BT_TILE, &tmQKV, q_full, 0, h, q0 + 64 * b, seq);
+      tma_load_4d(bt_smem + BT_ST, &tmDO, q_full, 0, h, q0, seq);
+      tma_load_4d(bt_smem + BT_ST + 2 * BT_TILE, &tmDO, q_full, 32, h, q0, seq);
+    }
+    if (qt == 0 && !(ok = wait_all(kv_full, 0))) break;
+    if (!(ok = wait_all(q_full, static_cast<uint32_t>(qt) & 1u))) break;
+    // ---- operands to bf16: fp16 Q (and K, V once), fp32 dO -> the swizzled dO tile
+    if (p.f16) {
+      for (int i = tid; i < nq * BT_TILE / 16; i += BT_THREADS) f16_to_bf16_x8(reinterpret_cast<uint4*>(bt_smem + BT_Q) + i);
+      if (qt == 0)
+        for (int i = tid; i < nkb * BT_TILE / 16; i += BT_THREADS) {
+          f16_to_bf16_x8(reinterpret_cast<uint4*>(bt_smem + BT_K) + i);
+          f16_to_bf16_x8(reinterpret_cast<uint4*>(bt_smem + BT_V) + i);
+        }
+    }
+    if (qt == 0) {
+      // K minus its mean over the T keys.  Softmax ignores a vector added to every key (each score of a row moves by
+      // the same amount), so P, dP, dS and dK are unchanged; but dQ = dS K no longer carries the mean key times the
+      // rounding error of sum_j dS_j (exactly 0 before dS is rounded to bf16), which dominated dQ's error when the
+      // keys share a large common component, and S is computed from smaller operands.
+      float* kmean = reinterpret_cast<float*>(bt_smem + BT_KMEAN);
+      __syncthreads();   // K converted
+      if (tid < 64) {
+        float acc = 0.f;
+        for (int t = 0; t < T; ++t) {
+          const uint32_t w = reinterpret_cast<const uint32_t*>(chunk(bt_smem + BT_K, t, tid >> 3))[(tid & 7) >> 1];
+          const float2 f = unpack_h2<false>(w);
+          acc += (tid & 1) ? f.y : f.x;
+        }
+        kmean[tid] = acc / static_cast<float>(T);
+      }
+      __syncthreads();
+      for (int i = tid; i < T * 8; i += BT_THREADS) {
+        const int t = i >> 3, j = i & 7;
+        uint4* cp = chunk(bt_smem + BT_K, t, j);
+        const uint4 c = *cp;
+        uint32_t w[4] = {c.x, c.y, c.z, c.w};
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+          const float2 f = unpack_h2<false>(w[e]);
+          w[e] = pack_bf16x2(f.x - kmean[8 * j + 2 * e], f.y - kmean[8 * j + 2 * e + 1]);
+        }
+        *cp = make_uint4(w[0], w[1], w[2], w[3]);
+      }
+    }
+    for (int i = tid; i < 128 * 8; i += BT_THREADS) {
+      const int rr = i >> 3, j = i & 7;
+      const float4* src = reinterpret_cast<const float4*>(bt_smem + BT_ST + (j >> 2) * 2 * BT_TILE + rr * 128 + (j & 3) * 32);
+      const float4 a = src[0], b = src[1];
+      *chunk(bt_smem + BT_DO, rr, j) = make_uint4(pack_bf16x2(a.x, a.y), pack_bf16x2(a.z, a.w), pack_bf16x2(b.x, b.y),
+                                                  pack_bf16x2(b.z, b.w));
+    }
+    fence_proxy_async_smem();
+    __syncthreads();
+
+    // ---- S = Q K^T
+    if (tid == 0) {
+      tc_fence_after();
+      const uint64_t dq = umma_desc_sw128(sbase + BT_Q), dk = umma_desc_sw128(sbase + BT_K);
+#pragma unroll
+      for (int k = 0; k < 4; ++k)
+        umma_bf16(tmem_base + BT_S_COL, dq + 2 * k, dk + 2 * k, idesc_s, k != 0 ? 1u : 0u);
+    }
+    if (!(ok = commit_wait())) break;
+
+    // ---- exact softmax of this row: maximum, sum, then P = exp / sum as bf16 into the P sub-tiles (zeros past T)
+    {
+      const bool valid = r < T;
+      float m4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
+      for (int ch = 0; ch < 2 * nkb; ++ch) {
+        uint32_t sv[32];
+        tmem_ld_32x32b_x32(lane_base + BT_S_COL + static_cast<uint32_t>(ch * 32), sv);
+        tmem_ld_wait();
+#pragma unroll
+        for (int c = 0; c < 32; ++c)
+          if (ch * 32 + c < T) m4[c & 3] = fmaxf(m4[c & 3], __uint_as_float(sv[c]));
+      }
+      const float nmx = -fmaxf(fmaxf(m4[0], m4[1]), fmaxf(m4[2], m4[3])) * scale_log2;
+      float s4[4] = {0.f, 0.f, 0.f, 0.f};
+      for (int ch = 0; ch < 2 * nkb; ++ch) {
+        uint32_t sv[32];
+        tmem_ld_32x32b_x32(lane_base + BT_S_COL + static_cast<uint32_t>(ch * 32), sv);
+        tmem_ld_wait();
+#pragma unroll
+        for (int c = 0; c < 32; ++c)
+          if (ch * 32 + c < T) s4[c & 3] += ex2_approx(fmaf(__uint_as_float(sv[c]), scale_log2, nmx));
+      }
+      const float inv = 1.f / ((s4[0] + s4[1]) + (s4[2] + s4[3]));
+      for (int ch = 0; ch < 4 * nqt; ++ch) {   // 32 keys per chunk, over the key tiles the dV / dK products read
+        uint32_t sv[32] = {};
+        if (ch < 2 * nkb) {
+          tmem_ld_32x32b_x32(lane_base + BT_S_COL + static_cast<uint32_t>(ch * 32), sv);
+          tmem_ld_wait();
+        }
+        uint32_t pv[16];
+#pragma unroll
+        for (int c = 0; c < 16; ++c) {
+          const int k0 = ch * 32 + 2 * c;
+          const float p0 = valid && k0 < T ? ex2_approx(fmaf(__uint_as_float(sv[2 * c]), scale_log2, nmx)) * inv : 0.f;
+          const float p1 = valid && k0 + 1 < T ? ex2_approx(fmaf(__uint_as_float(sv[2 * c + 1]), scale_log2, nmx)) * inv : 0.f;
+          pv[c] = pack_bf16x2(p0, p1);
+        }
+        uint8_t* sub = bt_smem + BT_P + (ch >> 1) * BT_P_SUB;
+#pragma unroll
+        for (int j = 0; j < 4; ++j)
+          *chunk(sub, tid, (ch & 1) * 4 + j) = make_uint4(pv[4 * j], pv[4 * j + 1], pv[4 * j + 2], pv[4 * j + 3]);
+      }
+    }
+    fence_proxy_async_smem();
+    tc_fence_before();
+    __syncthreads();
+
+    // ---- dP = dO V^T (over S), dV += P^T dO
+    if (tid == 0) {
+      tc_fence_after();
+      const uint64_t ddo = umma_desc_sw128(sbase + BT_DO), dv = umma_desc_sw128(sbase + BT_V);
+#pragma unroll
+      for (int k = 0; k < 4; ++k)
+        umma_bf16(tmem_base + BT_S_COL, ddo + 2 * k, dv + 2 * k, idesc_s, k != 0 ? 1u : 0u);
+      const uint64_t bdo = umma_desc_sw128_mn(sbase + BT_DO);
+      for (int kt = 0; kt < nqt; ++kt) {
+        const uint64_t apt = umma_desc_sw128_mn(sbase + BT_P + 2 * kt * BT_P_SUB, BT_P_SUB);
+        for (int ks = 0; ks < 4 * nq; ++ks)   // 16 query rows per step
+          umma_bf16(tmem_base + BT_DV_COL + 64 * kt, apt + ks * (2048 >> 4), bdo + ks * (2048 >> 4), idesc_t,
+                    (qt > 0 || ks > 0) ? 1u : 0u);
+      }
+    }
+    if (!(ok = commit_wait())) break;
+
+    // ---- D = rowsum(P dP); dS = P (dP - D) / 8 over P.  D is taken over the stored (bf16) P divided by that P's sum,
+    // so that dP - D keeps its relative accuracy when one key holds almost all of a row's weight.
+    {
+      float d4[4] = {0.f, 0.f, 0.f, 0.f}, s4[4] = {0.f, 0.f, 0.f, 0.f};
+      for (int ch = 0; ch < 2 * nkb; ++ch) {
+        uint32_t dv[32];
+        tmem_ld_32x32b_x32(lane_base + BT_S_COL + static_cast<uint32_t>(ch * 32), dv);
+        tmem_ld_wait();
+        uint8_t* sub = bt_smem + BT_P + (ch >> 1) * BT_P_SUB;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          const uint4 pc = *chunk(sub, tid, (ch & 1) * 4 + j);
+          const uint32_t pw[4] = {pc.x, pc.y, pc.z, pc.w};
+#pragma unroll
+          for (int e = 0; e < 4; ++e) {
+            const float2 pf = unpack_h2<false>(pw[e]);
+            d4[e] = fmaf(pf.x, __uint_as_float(dv[8 * j + 2 * e]), d4[e]);
+            d4[e] = fmaf(pf.y, __uint_as_float(dv[8 * j + 2 * e + 1]), d4[e]);
+            s4[e] += pf.x + pf.y;
+          }
+        }
+      }
+      const float psum = (s4[0] + s4[1]) + (s4[2] + s4[3]);   // 0 on rows past T
+      const float D = psum > 0.f ? ((d4[0] + d4[1]) + (d4[2] + d4[3])) / psum : 0.f;
+      for (int ch = 0; ch < 2 * nkb; ++ch) {
+        uint32_t dv[32];
+        tmem_ld_32x32b_x32(lane_base + BT_S_COL + static_cast<uint32_t>(ch * 32), dv);
+        tmem_ld_wait();
+        uint8_t* sub = bt_smem + BT_P + (ch >> 1) * BT_P_SUB;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          uint4* cp = chunk(sub, tid, (ch & 1) * 4 + j);
+          const uint4 pc = *cp;
+          uint32_t pw[4] = {pc.x, pc.y, pc.z, pc.w};
+#pragma unroll
+          for (int e = 0; e < 4; ++e) {
+            const float2 pf = unpack_h2<false>(pw[e]);
+            pw[e] = pack_bf16x2(pf.x * (__uint_as_float(dv[8 * j + 2 * e]) - D) * 0.125f,
+                                pf.y * (__uint_as_float(dv[8 * j + 2 * e + 1]) - D) * 0.125f);
+          }
+          *cp = make_uint4(pw[0], pw[1], pw[2], pw[3]);
+        }
+      }
+    }
+    fence_proxy_async_smem();
+    tc_fence_before();
+    __syncthreads();
+
+    // ---- dQ = dS K (over dP), dK += dS^T Q
+    if (tid == 0) {
+      tc_fence_after();
+      const uint64_t bk = umma_desc_sw128_mn(sbase + BT_K);
+      for (int ks = 0; ks < 4 * nkb; ++ks)   // 16 keys per step: 32 B within a 64-key sub-tile, then the next sub-tile
+        umma_bf16(tmem_base + BT_S_COL, umma_desc_sw128(sbase + BT_P + (ks >> 2) * BT_P_SUB) + 2 * (ks & 3),
+                  bk + ks * (2048 >> 4), idesc_q, ks != 0 ? 1u : 0u);
+      const uint64_t bq = umma_desc_sw128_mn(sbase + BT_Q);
+      for (int kt = 0; kt < nqt; ++kt) {
+        const uint64_t ast = umma_desc_sw128_mn(sbase + BT_P + 2 * kt * BT_P_SUB, BT_P_SUB);
+        for (int ks = 0; ks < 4 * nq; ++ks)
+          umma_bf16(tmem_base + BT_DK_COL + 64 * kt, ast + ks * (2048 >> 4), bq + ks * (2048 >> 4), idesc_t,
+                    (qt > 0 || ks > 0) ? 1u : 0u);
+      }
+    }
+    if (!(ok = commit_wait())) break;
+
+    // ---- dQ -> bf16 -> staging -> TMA store (rows past T clipped)
+    {
+      uint32_t ov[64];
+      tmem_ld_32x32b_x32(lane_base + BT_S_COL, *reinterpret_cast<uint32_t(*)[32]>(&ov[0]));
+      tmem_ld_32x32b_x32(lane_base + BT_S_COL + 32, *reinterpret_cast<uint32_t(*)[32]>(&ov[32]));
+      tmem_ld_wait();
+#pragma unroll
+      for (int j = 0; j < 8; ++j)
+        *chunk(bt_smem + BT_ST, tid, j) =
+            make_uint4(pack_bf16x2(__uint_as_float(ov[8 * j]), __uint_as_float(ov[8 * j + 1])),
+                       pack_bf16x2(__uint_as_float(ov[8 * j + 2]), __uint_as_float(ov[8 * j + 3])),
+                       pack_bf16x2(__uint_as_float(ov[8 * j + 4]), __uint_as_float(ov[8 * j + 5])),
+                       pack_bf16x2(__uint_as_float(ov[8 * j + 6]), __uint_as_float(ov[8 * j + 7])));
+    }
+    fence_proxy_async_smem();
+    tc_fence_before();   // the next tile's scores overwrite these columns
+    __syncthreads();
+    if (tid == 0) {
+      for (int b = 0; b < nq; ++b) tma_store_4d(&tmOut, bt_smem + BT_ST + b * BT_TILE, 0, h, q0 + 64 * b, seq);
+      bulk_commit();
+    }
+  }
+
+  // ---- dK, dV of the key tiles -> bf16 -> staging over the (now free) P / dS tile -> TMA store
+  if (ok) {
+    for (int kt = 0; kt < nqt; ++kt)
+      for (int m = 0; m < 2; ++m) {   // m = 0: dK, 1: dV
+        uint32_t ov[64];
+        const uint32_t col = (m == 0 ? BT_DK_COL : BT_DV_COL) + 64 * kt;
+        tmem_ld_32x32b_x32(lane_base + col, *reinterpret_cast<uint32_t(*)[32]>(&ov[0]));
+        tmem_ld_32x32b_x32(lane_base + col + 32, *reinterpret_cast<uint32_t(*)[32]>(&ov[32]));
+        tmem_ld_wait();
+        uint8_t* st = bt_smem + BT_P + (2 * kt + m) * BT_P_SUB;
+#pragma unroll
+        for (int j = 0; j < 8; ++j)
+          *chunk(st, tid, j) = make_uint4(pack_bf16x2(__uint_as_float(ov[8 * j]), __uint_as_float(ov[8 * j + 1])),
+                                          pack_bf16x2(__uint_as_float(ov[8 * j + 2]), __uint_as_float(ov[8 * j + 3])),
+                                          pack_bf16x2(__uint_as_float(ov[8 * j + 4]), __uint_as_float(ov[8 * j + 5])),
+                                          pack_bf16x2(__uint_as_float(ov[8 * j + 6]), __uint_as_float(ov[8 * j + 7])));
+      }
+    fence_proxy_async_smem();
+    __syncthreads();
+    if (tid == 0) {
+      for (int kt = 0; kt < nqt; ++kt)
+        for (int m = 0; m < 2; ++m)
+          for (int b = 0; b < 2; ++b)
+            if (128 * kt + 64 * b < T)
+              tma_store_4d(&tmOut, bt_smem + BT_P + (2 * kt + m) * BT_P_SUB + b * BT_TILE, 0, (m + 1) * p.heads + h,
+                           128 * kt + 64 * b, seq);
+      bulk_commit();
+    }
+  }
+  if (tid == 0) bulk_wait<0>();
+
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 0) {
+    tc_fence_after();
+    tmem_dealloc(tmem_base, BT_TMEM_COLS);
   }
 }
 
@@ -415,10 +806,44 @@ cudaError_t launch_ln_bwd(const float* x, const float* dy, int64_t rows, int W, 
   ln_bwd_kernel<<<static_cast<unsigned>((rows + 7) / 8), 256, 0, s>>>(x, dy, rows, W, gamma, g);
   return cudaGetLastError();
 }
+// fp32 dO [n_seq, T, heads, 64] as a 4-D tensor (d, head, token, sequence), boxes of [128 tokens][32] (128-byte rows,
+// unswizzled); tokens past T are zero on load
+bool make_tmap_dout(CUtensorMap* tm, const float* base, uint64_t n_seq, uint64_t T, uint64_t heads) {
+  auto encode = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(gemm_encode_tiled_fn());
+  if (!encode) return false;
+  const uint64_t row_bytes = heads * 64 * 4;
+  cuuint64_t gdim[4] = {64, heads, T, n_seq};
+  cuuint64_t gstride[3] = {64 * 4, row_bytes, T * row_bytes};
+  cuuint32_t box[4] = {32, 1, 128, 1};
+  cuuint32_t estr[4] = {1, 1, 1, 1};
+  return encode(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(base), gdim, gstride, box, estr,
+                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+
 cudaError_t launch_attention_bwd(const __nv_bfloat16* qkv, const float* dout, int64_t n_views, int T, int heads, int f16,
-                                 __nv_bfloat16* dqkv, cudaStream_t s) {
-  if (T < 1 || T > AB_T) return cudaErrorInvalidValue;
+                                 __nv_bfloat16* dqkv, cudaStream_t s, int* dev_status) {
+  if (T < 1 || T > 256 || heads < 1) return cudaErrorInvalidValue;
   if (n_views <= 0) return cudaSuccess;
+  if (T > AB_T) {
+    if (dev_status == nullptr) return cudaErrorInvalidValue;
+    if ((reinterpret_cast<uintptr_t>(qkv) | reinterpret_cast<uintptr_t>(dout) | reinterpret_cast<uintptr_t>(dqkv)) & 15)
+      return cudaErrorInvalidValue;
+    CUtensorMap tmQKV, tmDO, tmOut;
+    if (!make_tmap_heads(&tmQKV, qkv, static_cast<uint64_t>(n_views), static_cast<uint64_t>(T), 3ull * heads, f16) ||
+        !make_tmap_dout(&tmDO, dout, static_cast<uint64_t>(n_views), static_cast<uint64_t>(T), static_cast<uint64_t>(heads)) ||
+        !make_tmap_heads(&tmOut, dqkv, static_cast<uint64_t>(n_views), static_cast<uint64_t>(T), 3ull * heads, 0))
+      return cudaErrorInvalidValue;
+    cudaError_t e = ensure_dynamic_smem(attention_bwd_tcgen05_kernel, BT_SMEM);
+    if (e != cudaSuccess) return e;
+    AbtDev p;
+    p.heads = heads;
+    p.T = T;
+    p.f16 = f16 != 0;
+    p.status = dev_status;
+    attention_bwd_tcgen05_kernel<<<static_cast<unsigned>(n_views * heads), BT_THREADS, BT_SMEM, s>>>(tmQKV, tmDO, tmOut, p);
+    return cudaGetLastError();
+  }
   const size_t smem = (6 * AB_T * AB_LD + AB_T) * sizeof(float);
   cudaError_t e = ensure_dynamic_smem(attention_bwd_kernel, smem);
   if (e != cudaSuccess) return e;

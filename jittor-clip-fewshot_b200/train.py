@@ -13,7 +13,7 @@ Everything else -- loss, optimiser, schedule -- stays in torch; it acts on a few
     loss = F.cross_entropy(100 * f @ text.T, labels); loss.backward(); opt.step()
     trainer.save(args, epoch)                            # the reference pickle, readable by load_lora
 
-Scope: towers of at most 64 tokens (ViT-B/32, plain or IVLP), one adapter set, q / k / v / o on any blocks with the
+Scope: towers of at most 256 tokens (ViT-B/32 and ViT-B/16, plain or IVLP), one adapter set, q / k / v / o on any blocks with the
 ranks of q, k, v of a block summing to at most 64.  Base weights, biases, LayerNorms, embeddings and `visual.VPT` are
 frozen.  The trainer switches the context to the applied LoRA mode (`Context.set_lora_mode("applied")`).
 """
